@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- reads/s through SAGE2's overlap-graph build (reference steps 1-3) on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg4]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload cfg4] [--dump-outputs DIR]
 
 A "step" is one complete pass of the hot path over one batch of synthetic reads: ingest (filter,
 canonicalise, 2-bit pack), sort + dedupe, prefix/suffix table, phase A search + extension state
@@ -42,6 +42,8 @@ import numpy as np
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+# the tree stays as the build left it (it may be read-only): no bytecode caches from this run
+sys.dont_write_bytecode = True
 
 METRIC = "reads/sec through exact-overlap graph build (SAGE2 steps 1-3)"
 UNIT = "reads/s"
@@ -183,14 +185,14 @@ def run_reference_arm(args):
     rank = int(os.environ.get("RANK", "0"))
     if rank != 0:
         return
-    tmp = tempfile.mkdtemp(prefix="sage2_ref_")
     per_step = max(4.0, 170.0 / max(1, args.steps + args.warmup))
-    reads, k, cfg = sample_workload(args.workload, min(25.0, per_step), tmp)
     times, last = [], None
-    for i in range(args.warmup + args.steps):
-        last = reference_run(reads, k, tmp)
-        if i >= args.warmup:
-            times.append(last["t_steps123"])
+    with tempfile.TemporaryDirectory(prefix="sage2_ref_") as tmp:
+        reads, k, cfg = sample_workload(args.workload, min(25.0, per_step), tmp)
+        for i in range(args.warmup + args.steps):
+            last = reference_run(reads, k, tmp)
+            if i >= args.warmup:
+                times.append(last["t_steps123"])
     ms = 1000.0 * float(np.mean(times))
     value = len(reads) / (ms / 1000.0)
     full = SHAPES.get(cfg["name"], (cfg["workload"],))[0]
@@ -376,7 +378,39 @@ class Job:
             self.dist.all_reduce(t, op=self.dist.ReduceOp.MAX)
         return float(t[0]), float(t[1]), api.kernel_launches() - l0, {a: b / steps for a, b in stage.items()}
 
-    def measure(self, steps: int, warmup: int, with_alt: bool, sample_clocks: bool) -> dict:
+    def dump_outputs(self, out_dir: str, max_rows: int = 1 << 19, seed: int = 0):
+        """What the last step left on this GPU, as float64 .npy files (38 MB at most; row samples are seeded, so two runs
+        of the same workload pick the same rows):
+          edges.npy     sampled rows of the edge list, in order: [row, from, to, type, delta, delta_twin]
+          reads.npy     sampled unique reads, in id order: [id, length, frequency]
+          counters.npy  good_reads, unique_reads, n_edges, contained_ext, contained_size, left_to_explore,
+                        edges_inserted_c, transitive_removed
+          digests.npy   digests of the whole edge list and of all reads (tests/digest.py), each as [high 32 bits, low 32 bits]"""
+        def sample(n):
+            if n <= max_rows:
+                return np.arange(n)
+            return np.sort(np.random.default_rng(seed).choice(n, size=max_rows, replace=False))
+
+        def save(name, *cols):      # one column: a vector; several: a table with one row per sampled item
+            a = np.stack([np.asarray(c, np.float64) for c in cols], axis=1) if len(cols) > 1 else cols[0]
+            np.save(os.path.join(out_dir, name + ".npy"), np.asarray(a, np.float64))
+
+        os.makedirs(out_dir, exist_ok=True)
+        gpu = self.gpu
+        e = gpu.edges()
+        rows = sample(len(e))
+        e = e[rows]
+        save("edges", rows, e["from"], e["to"], e["type"], e["delta"], e["delta_twin"])
+        r = gpu.reads()
+        rows = sample(len(r["length"]))
+        save("reads", rows + 1, r["length"][rows], r["frequency"][rows])
+        c = gpu.counters()
+        save("counters", [c[n] for n in ("good_reads", "unique_reads", "n_edges", "contained_ext", "contained_size",
+                                         "left_to_explore", "edges_inserted_c", "transitive_removed")])
+        d = gpu.digest()
+        save("digests", [d["edges"] >> 32, d["edges"] & 0xFFFFFFFF, d["reads"] >> 32, d["reads"] & 0xFFFFFFFF])
+
+    def measure(self, steps: int, warmup: int, with_alt: bool, sample_clocks: bool, dump_dir: str | None = None) -> dict:
         args, gpu, world = self.args, self.gpu, self.world
         for _ in range(max(3, warmup)):
             self.step_device()
@@ -387,6 +421,8 @@ class Job:
         clocks = sampler.stop() if sampler else None
         xwall = {kk: (vv / steps) for kk, vv in self.xstats.items()} if self.xstats else None
         self.check_parity("device_resident")
+        if dump_dir and self.rank == 0:
+            self.dump_outputs(dump_dir)
         self.step_host()
         e2e_dev_ms, e2e_wall_ms, _, _ = self.timed(self.step_host, steps)
         self.check_parity("e2e")
@@ -469,7 +505,7 @@ def run_ours(args):
     # N > 1: ONE read set for the whole job (same bytes on every rank); phase A is partitioned by read id and followed
     # by one NCCL exchange (sage2_b200/multi.py); reads and table are replicated (SURVEY.md 8(e), DESIGN.md section 4)
     job = Job(args, args.workload, torch, dist, rank, world, local)
-    m = job.measure(args.steps, args.warmup, with_alt=not args.no_alt_table, sample_clocks=True)
+    m = job.measure(args.steps, args.warmup, with_alt=not args.no_alt_table, sample_clocks=True, dump_dir=args.dump_outputs)
     parity = job.parity()
     roofline = job.roofline(m, with_gather=not args.no_gather) if rank == 0 else None
     n_reads, cfg, comm, sharded, per_step = job.n_reads, job.cfg, dict(job.comm), job.sharded, job.per_step
@@ -480,7 +516,7 @@ def run_ours(args):
     extra = None
     if world == 1 and args.workload != "cfg2" and not args.no_cfg2:
         j2 = Job(args, "cfg2", torch, dist, rank, world, local)
-        m2 = j2.measure(min(args.steps, 20), 3, with_alt=False, sample_clocks=False)
+        m2 = j2.measure(args.steps, 3, with_alt=False, sample_clocks=False)
         r2 = j2.roofline(m2, with_gather=False)
         ms2 = m2["dev_ms"] / m2["steps"]
         extra = {"workload": j2.cfg["workload"], "reads_per_step": j2.n_reads, "ms_per_step": ms2, "value": j2.n_reads / (ms2 / 1000.0),
@@ -511,9 +547,9 @@ def run_ours(args):
     # reference's CPU path on a bounded sample of the same workload (rank 0, N=1 only)
     cpu = None
     if world == 1 and not args.no_cpu_baseline:
-        tmp = tempfile.mkdtemp(prefix="sage2_cpu_")
-        s_reads, s_k, s_cfg = sample_workload(args.workload, 15.0, tmp)
-        d = reference_run(s_reads, s_k, tmp)
+        with tempfile.TemporaryDirectory(prefix="sage2_cpu_") as tmp:
+            s_reads, s_k, s_cfg = sample_workload(args.workload, 15.0, tmp)
+            d = reference_run(s_reads, s_k, tmp)
         cpu = {"value": d["input_reads"] / d["t_steps123"], "unit": UNIT, "cores": d.get("threads"), "kind": d["kind"],
                "sample": sample_text(s_cfg, len(s_reads), d["t_steps123"]),
                "breakdown_s": {k2: v for k2, v in d.items() if k2.startswith("t_")}}
@@ -575,7 +611,13 @@ def main():
     ap.add_argument("--batch-reads", type=int, default=1 << 20, help="reads per routed batch (--table sharded)")
     ap.add_argument("--no-gather", action="store_true", help="skip the random-gather ceiling microbenchmark")
     ap.add_argument("--read-order", default=None, choices=["id", "minhash"], help="phase-A schedule (default: the library's)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step of the headline workload computed to DIR/*.npy (Job.dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
     if args.impl == "reference":
         run_reference_arm(args)
     else:

@@ -28,7 +28,7 @@ def _get(name):
     return datasets.get(name) if name in datasets.DATASETS else synth.config(name)
 
 
-@pytest.mark.parametrize("name", ["mixed", "rep", "varlen_err", "k70", "cfg1"])
+@pytest.mark.parametrize("name", ["mixed", "rep", "varlen_err", "k70", "cfg1", "cfg4mini"])
 def test_cli_files_byte_identical_to_reference(name, tmp_path):
     reads, k = _get(name)
     fq = tmp_path / "in.fastq"
