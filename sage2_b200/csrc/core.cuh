@@ -88,17 +88,20 @@ SG_HD u64 rev2(u64 w)
 
 // Record of the reverse complement (utils.cpp:73-91 on packed words): reverse all 2-bit groups of
 // the SW*64-bit string, complement, shift the sequence back to the top, re-attach the length.
-SG_HD void revcomp_record(const u64 *F, u64 *R, int SW, int len)
+// Word w of it depends on two words of F only, so lanes that share a record can each produce their own words.
+SG_HD u64 revcomp_word(const u64 *F, int SW, int len, int w)
 {
     const int sh = 64 * SW - 2 * len;     // >= 16
     const int q = sh >> 6, r = sh & 63;
-    for (int w = 0; w < SW; ++w) {
-        const int i0 = w + q, i1 = w + q + 1;
-        const u64 a = i0 < SW ? rev2(~F[SW - 1 - i0]) : 0ull;
-        const u64 b = i1 < SW ? rev2(~F[SW - 1 - i1]) : 0ull;
-        R[w] = r == 0 ? a : ((a << r) | (b >> (64 - r)));
-    }
-    R[SW - 1] |= (u64)len;
+    const int i0 = w + q, i1 = w + q + 1;
+    const u64 a = i0 < SW ? rev2(~F[SW - 1 - i0]) : 0ull;
+    const u64 b = i1 < SW ? rev2(~F[SW - 1 - i1]) : 0ull;
+    const u64 x = r == 0 ? a : ((a << r) | (b >> (64 - r)));
+    return w == SW - 1 ? x | (u64)len : x;
+}
+SG_HD void revcomp_record(const u64 *F, u64 *R, int SW, int len)
+{
+    for (int w = 0; w < SW; ++w) R[w] = revcomp_word(F, SW, len, w);
 }
 
 // ---- prefix/suffix table ----------------------------------------------------------------------

@@ -4,6 +4,7 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 #include <stdio.h>
+#include <stdlib.h>
 #include <algorithm>
 #include <stdexcept>
 #include <string>
@@ -180,6 +181,9 @@ inline unsigned long long &launch_counter() { static unsigned long long n = 0; r
         ++sg::launch_counter();           \
         SG_CUDA(cudaGetLastError());      \
     } while (0)
+
+// SAGE2GPU_STAGE_STATS set: stages print the sizes their cost depends on to stderr (tools/stage_kernels.py collects them)
+inline bool stage_stats_enabled() { return getenv("SAGE2GPU_STAGE_STATS") != nullptr; }
 
 inline unsigned grid_for(u64 n, unsigned block, unsigned per_thread = 1)
 {

@@ -351,35 +351,64 @@ __global__ void gather_word_kernel(const u64 *__restrict__ rec, const u32 *__res
         key[i] = rec[(u64)perm[i] * SW + w];
 }
 
-__global__ void unique_flag_kernel(const u64 *__restrict__ rec, const u32 *__restrict__ perm, u64 n_good, int SW, u32 *__restrict__ flag)
+__device__ __forceinline__ bool rec_differs(const u64 *a, const u64 *b, int SW)
 {
-    for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n_good; i += (u64)gridDim.x * blockDim.x) {
-        u32 f = 1;
-        if (i > 0) {
-            const u64 *a = rec + (u64)perm[i] * SW, *b = rec + (u64)perm[i - 1] * SW;
-            f = 0;
-            for (int w = 0; w < SW; ++w) f |= (a[w] != b[w]);
-        }
-        flag[i] = f;
+    u64 d = 0;
+    for (int w = 0; w < SW; ++w) d |= a[w] ^ b[w];
+    return d != 0;
+}
+
+// F / RC records are written by groups of SWS / 4 lanes, one 256-bit store of four words per lane: the groups of a warp
+// cover consecutive unique ids, so a warp's stores are whole contiguous lines (a lane per record stored every word to
+// a different line).  The lanes of a group meet in shared memory to form the reverse complement.
+constexpr int UW_THREADS = 256;
+__device__ __forceinline__ void ld256(const u64 *p, u64 (&v)[4])
+{
+    asm volatile("ld.global.nc.v4.u64 {%0,%1,%2,%3}, [%4];" : "=l"(v[0]), "=l"(v[1]), "=l"(v[2]), "=l"(v[3]) : "l"(p));
+}
+__device__ __forceinline__ void st256(u64 *p, const u64 (&v)[4])
+{
+    asm volatile("st.global.v4.u64 [%0], {%1,%2,%3,%4};" :: "l"(p), "l"(v[0]), "l"(v[1]), "l"(v[2]), "l"(v[3]) : "memory");
+}
+// lane g of a group holds words 4g .. 4g+3 of its record in f and the whole record is in grp[]: store both strands' words
+template <bool WITH_RC>
+__device__ __forceinline__ void store_group_words(const u64 *grp, const u64 (&f)[4], int g, int SW, int len, u64 *Fdst, u64 *RCdst)
+{
+    st256(Fdst + 4 * g, f);
+    if (WITH_RC) {
+        u64 r[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) { const int w = 4 * g + j; r[j] = w < SW ? revcomp_word(grp, SW, len, w) : 0ull; }
+        st256(RCdst + 4 * g, r);
     }
 }
 
 template <bool WITH_RC>
-__global__ void unique_write_kernel(const u64 *__restrict__ rec, const u32 *__restrict__ perm, const u32 *__restrict__ flag,
-                                    const u32 *__restrict__ uidx, u64 n_good, int SW, int SWS,
-                                    u64 *__restrict__ F, u64 *__restrict__ RC, uint16_t *__restrict__ len, u32 *__restrict__ start)
+__global__ void __launch_bounds__(UW_THREADS) unique_write_kernel(const u64 *__restrict__ rec, const u32 *__restrict__ perm, const u32 *__restrict__ flag,
+                                                                   const u32 *__restrict__ uidx, u64 n_good, int SW, int SWS,
+                                                                   u64 *__restrict__ F, u64 *__restrict__ RC, uint16_t *__restrict__ len, u32 *__restrict__ start)
 {
-    for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n_good; i += (u64)gridDim.x * blockDim.x) {
-        if (!flag[i]) continue;
-        const u32 u = uidx[i];
-        const u64 *a = rec + (u64)perm[i] * SW;
-        u64 f[kMaxWords], r[kMaxWords];
-        for (int w = 0; w < SW; ++w) f[w] = a[w];
-        const int l = rec_len(f, SW);
-        if (WITH_RC) revcomp_record(f, r, SW, l);
-        for (int w = 0; w < SWS; ++w) { F[(u64)u * SWS + w] = w < SW ? f[w] : 0ull; if (WITH_RC) RC[(u64)u * SWS + w] = w < SW ? r[w] : 0ull; }
-        len[u] = (uint16_t)l;
-        start[u] = (u32)i;
+    __shared__ u64 sRec[UW_THREADS * 4];
+    const int G = SWS / 4, g = threadIdx.x & (G - 1);
+    const u64 per_block = UW_THREADS / G;
+    u64 *grp = sRec + 4 * (threadIdx.x - g);
+    for (u64 i0 = (u64)blockIdx.x * per_block; i0 < n_good; i0 += (u64)gridDim.x * per_block) {      // uniform trip count per block
+        const u64 i = i0 + threadIdx.x / G;
+        const bool active = i < n_good && flag[i];
+        u64 f[4] = { 0, 0, 0, 0 };
+        if (active) {
+            const u64 *a = rec + (u64)perm[i] * SW;
+#pragma unroll
+            for (int j = 0; j < 4; ++j) { const int w = 4 * g + j; if (w < SW) f[j] = a[w]; grp[4 * g + j] = f[j]; }
+        }
+        __syncwarp();
+        if (active) {
+            const u32 u = uidx[i];
+            const int l = rec_len(grp, SW);
+            store_group_words<WITH_RC>(grp, f, g, SW, l, F + (u64)u * SWS, WITH_RC ? RC + (u64)u * SWS : nullptr);
+            if (g == 0) { len[u] = (uint16_t)l; start[u] = (u32)i; }
+        }
+        __syncwarp();
     }
 }
 
@@ -411,9 +440,11 @@ __global__ void compact_good_kernel(const u64 *__restrict__ rec, const u32 *__re
         if (flag[i]) { key[idx[i]] = rec[i * SW]; val[idx[i]] = (u32)i; }
 }
 
-// After the sort by the leading bases: order every run of equal prefixes by the whole records.
+// After the sort by the leading bases: order every run of equal prefixes by the whole records, and flag the first read
+// of every distinct record (the dedupe).  A read whose prefix differs from its predecessor's is new without a look at
+// the records; only the members of runs are compared.
 // Runs are short (duplicate reads, shared 24-mers); a run longer than kTieLimit (an insertion sort by one thread would
-// be the tail of the kernel) raises `overflow` and is left to refine_long_runs.
+// be the tail of the kernel) raises `overflow` and is left to refine_long_runs, which flags its members too.
 constexpr int kTieLimit = 32;
 // The radix passes cover the top 64 - skip bits of the first word: enough bits that runs of equal prefixes stay short
 // for the number of reads at hand (n reads spread over 2^(64-skip) prefixes), in whole 8-bit passes: 32 bits (16 bases,
@@ -433,11 +464,13 @@ __device__ __forceinline__ bool rec_less(const u64 *a, const u64 *b, int SW)
     return false;
 }
 __global__ void __launch_bounds__(256) tie_fix_kernel(const u64 *__restrict__ rec, const u64 *__restrict__ key, u32 *__restrict__ perm, u64 n, int SW,
-                                                        int kSortSkipBits, u32 *__restrict__ overflow)
+                                                        int kSortSkipBits, u32 *__restrict__ flag, u32 *__restrict__ overflow)
 {
     for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x) {
         const u64 k = key[i] >> kSortSkipBits;
-        if ((i > 0 && (key[i - 1] >> kSortSkipBits) == k) || i + 1 >= n || (key[i + 1] >> kSortSkipBits) != k) continue;      // not the head of a run of >= 2
+        if (i > 0 && (key[i - 1] >> kSortSkipBits) == k) continue;      // a member: its run's head flags it
+        flag[i] = 1u;
+        if (i + 1 >= n || (key[i + 1] >> kSortSkipBits) != k) continue;      // not the head of a run of >= 2
         u64 e = i + 2;
         while (e < n && (key[e] >> kSortSkipBits) == k && e - i <= (u64)kTieLimit) ++e;
         if (e - i > (u64)kTieLimit) { *overflow = 1u; continue; }
@@ -448,6 +481,7 @@ __global__ void __launch_bounds__(256) tie_fix_kernel(const u64 *__restrict__ re
             while (b > i && rec_less(rx, rec + (u64)perm[b - 1] * SW, SW)) { perm[b] = perm[b - 1]; --b; }
             perm[b] = x;
         }
+        for (u64 a = i + 1; a < e; ++a) flag[a] = rec_differs(rec + (u64)perm[a] * SW, rec + (u64)perm[a - 1] * SW, SW) ? 1u : 0u;
     }
 }
 
@@ -481,27 +515,37 @@ __global__ void __launch_bounds__(256) run_scatter_kernel(const u32 *__restrict_
 {
     for (u64 j = (u64)blockIdx.x * blockDim.x + threadIdx.x; j < m; j += (u64)gridDim.x * blockDim.x) perm[pos[j]] = val[j];
 }
+// after the scatter: the dedupe flag of the members (a run's head is flagged by tie_fix_kernel already)
+__global__ void __launch_bounds__(256) run_member_flag_kernel(const u64 *__restrict__ rec, const u32 *__restrict__ pos, const u32 *__restrict__ bound,
+                                                              const u32 *__restrict__ perm, u64 m, int SW, u32 *__restrict__ flag)
+{
+    for (u64 j = (u64)blockIdx.x * blockDim.x + threadIdx.x; j < m; j += (u64)gridDim.x * blockDim.x) {
+        const u32 i = pos[j];
+        if (!bound[i]) flag[i] = rec_differs(rec + (u64)perm[i] * SW, rec + (u64)perm[i - 1] * SW, SW) ? 1u : 0u;
+    }
+}
 
-static void refine_long_runs(Context &c, const u64 *rec, const u64 *key, u32 *perm, u64 n, int SW, int kSortSkipBits)
+// returns m, the members of the runs longer than kTieLimit
+static u32 refine_long_runs(Context &c, const u64 *rec, const u64 *key, u32 *perm, u64 n, int SW, int kSortSkipBits, u32 *dedupe_flag)
 {
     cudaStream_t st = c.stream;
-    DevBuf<u32> flag(n, st), excl(n, st), cnt(n, st), lflag(n, st), lidx(n, st), d_m(1, st);
-    run_boundary_kernel<<<big_grid(n), 256, 0, st>>>(key, n, kSortSkipBits, flag.p);
+    DevBuf<u32> bound(n, st), excl(n, st), cnt(n, st), lflag(n, st), lidx(n, st), d_m(1, st);
+    run_boundary_kernel<<<big_grid(n), 256, 0, st>>>(key, n, kSortSkipBits, bound.p);
     SG_LAUNCHED();
-    exclusive_scan_u32(flag.p, excl.p, n, nullptr, st);
+    exclusive_scan_u32(bound.p, excl.p, n, nullptr, st);
     SG_CUDA(cudaMemsetAsync(cnt.p, 0, n * sizeof(u32), st));
-    run_count_kernel<<<big_grid(n), 256, 0, st>>>(flag.p, excl.p, n, cnt.p);
+    run_count_kernel<<<big_grid(n), 256, 0, st>>>(bound.p, excl.p, n, cnt.p);
     SG_LAUNCHED();
-    run_long_flag_kernel<<<big_grid(n), 256, 0, st>>>(flag.p, excl.p, cnt.p, n, lflag.p);
+    run_long_flag_kernel<<<big_grid(n), 256, 0, st>>>(bound.p, excl.p, cnt.p, n, lflag.p);
     SG_LAUNCHED();
     exclusive_scan_u32(lflag.p, lidx.p, n, d_m.p, st);
     u32 m = 0;
     SG_CUDA(cudaMemcpyAsync(&m, d_m.p, sizeof(u32), cudaMemcpyDeviceToHost, st));
     SG_CUDA(cudaStreamSynchronize(st));
-    if (m == 0) return;
+    if (m == 0) return 0;
     DevBuf<u32> pos(m, st), v0(m, st), v1(m, st);
     DevBuf<u64> a0(m, st), a1(m, st), b0(m, st), b1(m, st);
-    run_compact_kernel<<<big_grid(n), 256, 0, st>>>(lflag.p, lidx.p, flag.p, excl.p, perm, n, pos.p, v0.p, b0.p);
+    run_compact_kernel<<<big_grid(n), 256, 0, st>>>(lflag.p, lidx.p, bound.p, excl.p, perm, n, pos.p, v0.p, b0.p);
     SG_LAUNCHED();
     SortCols cols;
     cols.a[0] = a0.p; cols.a[1] = a1.p; cols.b[0] = b0.p; cols.b[1] = b1.p; cols.v[0] = v0.p; cols.v[1] = v1.p;
@@ -516,6 +560,9 @@ static void refine_long_runs(Context &c, const u64 *rec, const u64 *key, u32 *pe
     cur = radix_sort_bits(cols, cur, m, true, 0, id_bits, st);      // ... and the run last: members return to their run's positions
     run_scatter_kernel<<<big_grid(m), 256, 0, st>>>(pos.p, cols.v[cur], m, perm);
     SG_LAUNCHED();
+    run_member_flag_kernel<<<big_grid(m), 256, 0, st>>>(rec, pos.p, bound.p, perm, m, SW, dedupe_flag);
+    SG_LAUNCHED();
+    return m;
 }
 
 // ---- several GPUs: rank r organises the reads whose leading bases fall into its key range ------------------------
@@ -545,14 +592,29 @@ __global__ void __launch_bounds__(256) split_compact_kernel(const u64 *__restric
     for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x)
         if (flag[i]) { okey[idx[i]] = key[i]; oval[idx[i]] = val[i]; }
 }
-__global__ void __launch_bounds__(256) revcomp_range_kernel(const u64 *__restrict__ F, u64 *__restrict__ RC, const uint16_t *__restrict__ len,
-                                                            u64 lo, u64 hi, int SW, int SWS)
+__global__ void __launch_bounds__(UW_THREADS) revcomp_range_kernel(const u64 *__restrict__ F, u64 *__restrict__ RC, const uint16_t *__restrict__ len,
+                                                                   u64 U, int SW, int SWS)
 {
-    for (u64 u = lo + (u64)blockIdx.x * blockDim.x + threadIdx.x; u < hi; u += (u64)gridDim.x * blockDim.x) {
-        u64 f[kMaxWords], r[kMaxWords];
-        for (int w = 0; w < SW; ++w) f[w] = F[u * SWS + w];
-        revcomp_record(f, r, SW, (int)len[u]);
-        for (int w = 0; w < SWS; ++w) RC[u * SWS + w] = w < SW ? r[w] : 0ull;
+    __shared__ u64 sRec[UW_THREADS * 4];
+    const int G = SWS / 4, g = threadIdx.x & (G - 1);
+    const u64 per_block = UW_THREADS / G;
+    u64 *grp = sRec + 4 * (threadIdx.x - g);
+    for (u64 u0 = (u64)blockIdx.x * per_block; u0 < U; u0 += (u64)gridDim.x * per_block) {
+        const u64 u = u0 + threadIdx.x / G;
+        u64 f[4] = { 0, 0, 0, 0 };
+        if (u < U) {
+            ld256(F + u * SWS + 4 * g, f);
+#pragma unroll
+            for (int j = 0; j < 4; ++j) grp[4 * g + j] = f[j];
+        }
+        __syncwarp();
+        if (u < U) {
+            u64 r[4];
+#pragma unroll
+            for (int j = 0; j < 4; ++j) { const int w = 4 * g + j; r[j] = w < SW ? revcomp_word(grp, SW, (int)len[u], w) : 0ull; }
+            st256(RC + u * SWS + 4 * g, r);
+        }
+        __syncwarp();
     }
 }
 
@@ -617,26 +679,23 @@ void stage_organize_reads(Context &c, int rank, int world)
         if (n_good == 0) return;
     }
     cur = radix_sort_bits(cols, cur, n_good, false, kSortSkipBits, 64, st);      // 4 .. 6 passes on the leading bases
+    // dedupe flags: tie_fix_kernel writes all of them but those of the members of runs longer than kTieLimit, which
+    // refine_long_runs sorts again by the rest of the record and flags (high-copy repeats, low-complexity input)
     DevBuf<u32> d_flags(2, st);          // [0] tie-run overflow, [1] unique count
     SG_CUDA(cudaMemsetAsync(d_flags.p, 0, 2 * sizeof(u32), st));
-    {
-        tie_fix_kernel<<<big_grid(n_good), 256, 0, st>>>(rec.p, cols.a[cur], cols.v[cur], n_good, SW, kSortSkipBits, d_flags.p);
-        SG_LAUNCHED();
-    }
     DevBuf<u32> flag(n_good, st), uidx(n_good, st);
+    tie_fix_kernel<<<big_grid(n_good), 256, 0, st>>>(rec.p, cols.a[cur], cols.v[cur], n_good, SW, kSortSkipBits, flag.p, d_flags.p);
+    SG_LAUNCHED();
     u32 h_flags[2] = { 0, 0 };
-    for (int attempt = 0; attempt < 2; ++attempt) {
-        unique_flag_kernel<<<big_grid(n_good), 256, 0, st>>>(rec.p, cols.v[cur], n_good, SW, flag.p);
-        SG_LAUNCHED();
-        exclusive_scan_u32(flag.p, uidx.p, n_good, d_flags.p + 1, st);
-        SG_CUDA(cudaMemcpyAsync(h_flags, d_flags.p, sizeof(h_flags), cudaMemcpyDeviceToHost, st));
-        SG_CUDA(cudaStreamSynchronize(st));
-        if (!h_flags[0] || attempt == 1) break;
-        // runs of more than kTieLimit equal prefixes (high-copy repeats, low-complexity input): their members
-        // alone are sorted again by the rest of the record
-        SG_CUDA(cudaMemsetAsync(d_flags.p, 0, sizeof(u32), st));
-        refine_long_runs(c, rec.p, cols.a[cur], cols.v[cur], n_good, SW, kSortSkipBits);
-    }
+    SG_CUDA(cudaMemcpyAsync(h_flags, d_flags.p, sizeof(u32), cudaMemcpyDeviceToHost, st));
+    SG_CUDA(cudaStreamSynchronize(st));
+    u32 m_long = 0;
+    if (h_flags[0]) m_long = refine_long_runs(c, rec.p, cols.a[cur], cols.v[cur], n_good, SW, kSortSkipBits, flag.p);
+    exclusive_scan_u32(flag.p, uidx.p, n_good, d_flags.p + 1, st);
+    SG_CUDA(cudaMemcpyAsync(h_flags + 1, d_flags.p + 1, sizeof(u32), cudaMemcpyDeviceToHost, st));
+    SG_CUDA(cudaStreamSynchronize(st));
+    if (stage_stats_enabled())
+        fprintf(stderr, "sage2gpu stats: organize_reads reads=%llu long_run_members=%u unique=%u\n", (unsigned long long)n_good, m_long, h_flags[1]);
     const u32 *perm = cols.v[cur];
     const u32 U = h_flags[1];
     c.cnt.unique_reads = U;
@@ -649,11 +708,12 @@ void stage_organize_reads(Context &c, int rank, int world)
     lo.alloc(U, st);
     fo.alloc(U, st);
     DevBuf<u32> start(U, st);
+    const unsigned uw_grid = big_grid(n_good * (c.SWS / 4), UW_THREADS);
     if (world > 1) {
-        unique_write_kernel<false><<<big_grid(n_good, 128), 128, 0, st>>>(rec.p, perm, flag.p, uidx.p, n_good, SW, c.SWS, Fo.p, nullptr, lo.p, start.p);
+        unique_write_kernel<false><<<uw_grid, UW_THREADS, 0, st>>>(rec.p, perm, flag.p, uidx.p, n_good, SW, c.SWS, Fo.p, nullptr, lo.p, start.p);
     } else {
         c.RC.alloc((size_t)U * c.SWS, st);
-        unique_write_kernel<true><<<big_grid(n_good, 128), 128, 0, st>>>(rec.p, perm, flag.p, uidx.p, n_good, SW, c.SWS, Fo.p, c.RC.p, lo.p, start.p);
+        unique_write_kernel<true><<<uw_grid, UW_THREADS, 0, st>>>(rec.p, perm, flag.p, uidx.p, n_good, SW, c.SWS, Fo.p, c.RC.p, lo.p, start.p);
     }
     SG_LAUNCHED();
     freq_kernel<<<big_grid(U), 256, 0, st>>>(start.p, U, n_good, fo.p);
@@ -696,7 +756,7 @@ void stage_reads_gather_finish(Context &c)
     SG_CHECK(c.rp_world > 1, "sage2gpu_load_reads_partition must run first");
     const u64 U = c.rp_total;
     if (U) {
-        revcomp_range_kernel<<<big_grid(U, 128), 128, 0, st>>>(c.F.p, c.RC.p, c.len.p, 0, U, c.SW, c.SWS);
+        revcomp_range_kernel<<<big_grid(U * (c.SWS / 4), UW_THREADS), UW_THREADS, 0, st>>>(c.F.p, c.RC.p, c.len.p, U, c.SW, c.SWS);
         SG_LAUNCHED();
     }
     c.cnt.unique_reads = U;

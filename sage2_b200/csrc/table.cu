@@ -81,33 +81,40 @@ __global__ void __launch_bounds__(256) table_insert_kernel(const u64 *__restrict
 }
 
 // ---- bucketed build: (hash, entry) records of the keys this shard owns ---------------------------------------------------
+// A record carries what decides key equality, so that the build never goes back to the reads: hash_key() is a bijection
+// of v1 for a fixed v0 (mix64 is invertible), hence two keys are equal iff their hashes and their v0 words are.  For
+// h <= 32, v0 is always 0 and the hash alone decides; otherwise v0 travels in a column B of its own.
 // one thread per read: its four keys.  world <= 1: record 4 rid + type sits at its own index; else the owned records are
 // compacted (one atomicAdd per block and round)
 __global__ void __launch_bounds__(256) table_keys_kernel(const u64 *__restrict__ F, const u64 *__restrict__ RC, const uint16_t *__restrict__ len,
                                                           u64 U, int SW, int SWS, int h, int rank, int world,
-                                                          u64 *__restrict__ A, u32 *__restrict__ V, u64 room, unsigned long long *__restrict__ n_out)
+                                                          u64 *__restrict__ A, u64 *__restrict__ B, u32 *__restrict__ V, u64 room,
+                                                          unsigned long long *__restrict__ n_out)
 {
     __shared__ u32 s_warp[8];
     __shared__ unsigned long long s_base;
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     for (u64 r0 = (u64)blockIdx.x * 256; r0 < U; r0 += (u64)gridDim.x * 256) {
         const u64 rid = r0 + threadIdx.x;
-        u64 hs[4] = { 0, 0, 0, 0 };
+        u64 hs[4] = { 0, 0, 0, 0 }, ks[4] = { 0, 0, 0, 0 };
         u32 own = 0;
         if (rid < U) {
             const int l = len[rid];
 #pragma unroll
             for (int type = 0; type < 4; ++type) {
-                u64 v0, v1;
-                entry_key(F + rid * SWS, RC + rid * SWS, SW, l, h, type, v0, v1);
-                hs[type] = hash_key(v0, v1);
+                u64 v1;
+                entry_key(F + rid * SWS, RC + rid * SWS, SW, l, h, type, ks[type], v1);
+                hs[type] = hash_key(ks[type], v1);
                 if (world <= 1 || key_owner(hs[type], world) == rank) own |= 1u << type;
             }
         }
         if (world <= 1) {
             if (rid < U) {
 #pragma unroll
-                for (int type = 0; type < 4; ++type) { A[4 * rid + type] = hs[type]; V[4 * rid + type] = (u32)(4 * rid + type); }
+                for (int type = 0; type < 4; ++type) {
+                    A[4 * rid + type] = hs[type]; V[4 * rid + type] = (u32)(4 * rid + type);
+                    if (B) B[4 * rid + type] = ks[type];
+                }
             }
             continue;
         }
@@ -127,7 +134,7 @@ __global__ void __launch_bounds__(256) table_keys_kernel(const u64 *__restrict__
         if (pos + cnt <= room) {        // else: the host sees n_out > room and repeats the pass with room for all
 #pragma unroll
             for (int type = 0; type < 4; ++type)
-                if (own & (1u << type)) { A[pos] = hs[type]; V[pos] = (u32)(4 * rid + type); ++pos; }
+                if (own & (1u << type)) { A[pos] = hs[type]; V[pos] = (u32)(4 * rid + type); if (B) B[pos] = ks[type]; ++pos; }
         }
         __syncthreads();
     }
@@ -138,7 +145,10 @@ __global__ void __launch_bounds__(256) table_keys_kernel(const u64 *__restrict__
 // when it arrived, and slots are never freed: having reached an empty slot, the key is not in the index).  A short chain of
 // dependent accesses (record, sector, CAS) and no divergence; everything else (tag seen, sector full, CAS lost) is appended
 // to the block's segment of `retry` for the second round.
-__global__ void __launch_bounds__(256) table_claim_kernel(const u64 *__restrict__ A, const u32 *__restrict__ V, u64 n_rec,
+// While the records are inserted, a slot's payload is the index of its representative's RECORD: a tag match is confirmed
+// from that record (same bucket, L2-resident while the bucket is worked on) instead of the reads.  table_runs_kernel puts
+// the entries in place afterwards.
+__global__ void __launch_bounds__(256) table_claim_kernel(const u64 *__restrict__ A, u64 n_rec,
                                                            u64 *__restrict__ slots, u64 nsec, u32 *__restrict__ where,
                                                            u32 *__restrict__ retry, u32 *__restrict__ n_retry)
 {
@@ -146,7 +156,6 @@ __global__ void __launch_bounds__(256) table_claim_kernel(const u64 *__restrict_
     bool again = false;
     if (i < n_rec) {
         const u64 hsh = A[i];
-        const u32 t = V[i];
         const u64 tag = slot_tag(hsh);
         const u64 sec = home_sector(hsh, nsec);
         u64 *sp = slots + kSlotsPerSector * sec;
@@ -161,7 +170,7 @@ __global__ void __launch_bounds__(256) table_claim_kernel(const u64 *__restrict_
         }
         again = true;
         if (q >= 0 && !seen) {
-            const u64 old = atomicCAS((unsigned long long *)(sp + q), 0ull, (unsigned long long)slot_encode(hsh, 1, t));
+            const u64 old = atomicCAS((unsigned long long *)(sp + q), 0ull, (unsigned long long)slot_encode(hsh, 1, i));
             if (old == 0) { where[i] = (u32)(kSlotsPerSector * sec + q); again = false; }
         }
     }
@@ -179,13 +188,10 @@ __global__ void __launch_bounds__(256) table_claim_kernel(const u64 *__restrict_
     if (threadIdx.x == 0) n_retry[blockIdx.x] = total;
 }
 
-// second round: the whole find-or-claim loop of table_insert_kernel on the records of `retry`; the hash comes with the
-// record and the keys are extracted only when a tag matches (a prefix key does not need the read's length: one random
-// access less)
-__global__ void __launch_bounds__(64) table_insert_sorted_kernel(const u64 *__restrict__ A, const u32 *__restrict__ V, const u32 *__restrict__ retry,
+// second round: the whole find-or-claim loop of table_insert_kernel on the records of `retry`; a tag match is confirmed by the
+// hash and v0 of the representative's record (see table_keys_kernel)
+__global__ void __launch_bounds__(64) table_insert_sorted_kernel(const u64 *__restrict__ A, const u64 *__restrict__ B, const u32 *__restrict__ retry,
                                                                    const u32 *__restrict__ n_retry,
-                                                                   const u64 *__restrict__ F, const u64 *__restrict__ RC,
-                                                                   const uint16_t *__restrict__ len, int SW, int SWS, int h,
                                                                    u64 *__restrict__ slots, u64 nsec, u32 *__restrict__ where, u32 *__restrict__ overflow)
 {
     // block b (64 threads: 32 such blocks fill an SM's warp slots) takes the failures of block b of the first round: dense
@@ -194,28 +200,23 @@ __global__ void __launch_bounds__(64) table_insert_sorted_kernel(const u64 *__re
     for (u32 k = threadIdx.x; k < mine; k += blockDim.x) {
         const u64 i = retry[(u64)blockIdx.x * 256 + k];
         const u64 hsh = A[i];
-        const u32 t = V[i];
+        const u64 v0 = B ? B[i] : 0ull;
         const u64 tag = slot_tag(hsh);
         u64 sec = home_sector(hsh, nsec);
-        bool done = false, have_key = false;
-        u64 v0 = 0, v1 = 0;
+        bool done = false;
         u64 tries = 0;
         while (!done) {
             for (int q = 0; q < kSlotsPerSector && !done; ++q) {
                 u64 *sp = slots + kSlotsPerSector * sec + q;
                 u64 cur = load_slot(sp);
                 if (cur == 0) {
-                    const u64 old = atomicCAS((unsigned long long *)sp, 0ull, (unsigned long long)slot_encode(hsh, 1, t));
+                    const u64 old = atomicCAS((unsigned long long *)sp, 0ull, (unsigned long long)slot_encode(hsh, 1, i));
                     if (old == 0) { where[i] = (u32)(kSlotsPerSector * sec + q); done = true; break; }
                     cur = old;
                 }
                 if (slot_get_tag(cur) != tag) continue;
-                if (!have_key) { const u64 r1 = t >> 2; entry_key(F + r1 * SWS, RC + r1 * SWS, SW, (t & 1) ? (int)len[r1] : h, h, (int)(t & 3), v0, v1); have_key = true; }
-                const u32 rep = (u32)slot_get_payload(cur);
-                const u64 r2 = rep >> 2;
-                u64 w0, w1;
-                entry_key(F + r2 * SWS, RC + r2 * SWS, SW, (rep & 1) ? (int)len[r2] : h, h, (int)(rep & 3), w0, w1);
-                if (w0 != v0 || w1 != v1) continue;
+                const u64 rep = slot_get_payload(cur);
+                if (A[rep] != hsh || (B && B[rep] != v0)) continue;
                 while (slot_get_count(cur) < 127) {
                     const u64 old = atomicCAS((unsigned long long *)sp, (unsigned long long)cur, (unsigned long long)(cur + kCountOne));
                     if (old == cur) break;
@@ -244,14 +245,19 @@ __global__ void __launch_bounds__(256) table_fill_sorted_kernel(const u64 *__res
     }
 }
 
-// pass 2a: run length of every slot that owns a run in entries[]; distinct / masked key counters
-__global__ void __launch_bounds__(256) table_runs_kernel(const u64 *__restrict__ slots, u64 cap, u32 *__restrict__ run, unsigned long long *counters)
+// pass 2a: run length of every slot that owns a run in entries[]; distinct / masked key counters.  Bucketed build (recV):
+// the payload of a slot without a run, a record index so far, becomes the representative's entry (the record's slot
+// neighbours have neighbouring hashes, so recV is read within one bucket's range)
+__global__ void __launch_bounds__(256) table_runs_kernel(u64 *__restrict__ slots, u64 cap, const u32 *__restrict__ recV, u32 *__restrict__ run,
+                                                          unsigned long long *counters)
 {
     unsigned long long distinct = 0, over = 0;
     for (u64 s = (u64)blockIdx.x * blockDim.x + threadIdx.x; s < cap; s += (u64)gridDim.x * blockDim.x) {
         const u64 v = slots[s];
         const u32 c = v ? slot_get_count(v) : 0u;
-        run[s] = (c >= 2 && c < (u32)kHashThreshold) ? c : 0u;
+        const bool has_run = c >= 2 && c < (u32)kHashThreshold;
+        run[s] = has_run ? c : 0u;
+        if (recV && v && !has_run) slots[s] = (v & ~0x1FFFFFFFFull) | (u64)recV[slot_get_payload(v)];
         distinct += v != 0;
         over += c >= (u32)kHashThreshold;
     }
@@ -337,10 +343,12 @@ void stage_build_table(Context &c, int rank, int world, bool joint)
     // bucketed build when the index is far larger than L2 (see the header); SAGE2GPU_TABLE_BUILD=direct|bucketed overrides
     const char *env = getenv("SAGE2GPU_TABLE_BUILD");
     const int forced = !env ? 0 : (env[0] == 'd' ? 1 : 2);
-    // (not in low-memory mode: the records take 2.5 x the workspace of the direct build, and config #5 fits 180 GB with nothing to spare)
+    // (not in low-memory mode: the records take 2.75 x (h > 32: 3.75 x) the workspace of the direct build, and config #5 fits
+    // 180 GB with nothing to spare)
     const bool bucketed = forced ? forced == 2 : (!c.opt_low_memory && cap * sizeof(u64) >= ((size_t)256 << 20));
     DevBuf<u32> where, d_overflow(1, st), v0, v1;
-    DevBuf<u64> a0, a1;
+    DevBuf<u64> a0, a1, b0, b1;
+    const bool with_v0 = h > 32;       // v0 is always 0 otherwise (table_keys_kernel)
     const u32 *recV = nullptr;
     u64 n_rec = n;
     SG_CUDA(cudaMemsetAsync(d_overflow.p, 0, sizeof(u32), st));
@@ -354,8 +362,9 @@ void stage_build_table(Context &c, int rank, int world, bool joint)
         DevBuf<unsigned long long> d_nrec(1, st);
         for (;;) {
             a0.alloc(room + 1, st); v0.alloc(room + 1, st);
+            if (with_v0) b0.alloc(room + 1, st);
             SG_CUDA(cudaMemsetAsync(d_nrec.p, 0, sizeof(unsigned long long), st));
-            table_keys_kernel<<<big_grid(U), 256, 0, st>>>(c.F.p, c.RC.p, c.len.p, U, SW, c.SWS, h, rank, world, a0.p, v0.p, room, d_nrec.p);
+            table_keys_kernel<<<big_grid(U), 256, 0, st>>>(c.F.p, c.RC.p, c.len.p, U, SW, c.SWS, h, rank, world, a0.p, b0.p, v0.p, room, d_nrec.p);
             SG_LAUNCHED();
             if (world <= 1) break;
             unsigned long long h_nrec = 0;
@@ -366,8 +375,9 @@ void stage_build_table(Context &c, int rank, int world, bool joint)
             room = n_rec;               // a very uneven key split (one key in most reads): once more with room for all of them
         }
         a1.alloc(n_rec + 1, st); v1.alloc(n_rec + 1, st);
+        if (with_v0) b1.alloc(n_rec + 1, st);
         SortCols cols;
-        cols.a[0] = a0.p; cols.a[1] = a1.p; cols.b[0] = cols.b[1] = nullptr; cols.v[0] = v0.p; cols.v[1] = v1.p;
+        cols.a[0] = a0.p; cols.a[1] = a1.p; cols.b[0] = b0.p; cols.b[1] = b1.p; cols.v[0] = v0.p; cols.v[1] = v1.p;
         const int cur = radix_sort_bits(cols, 0, n_rec, false, 56, 64, st);
         recV = cols.v[cur];
         where.alloc(n_rec + 1, st);
@@ -376,18 +386,25 @@ void stage_build_table(Context &c, int rank, int world, bool joint)
         if (n_rec) {
             const unsigned blocks = grid_for(n_rec, 256);
             DevBuf<u32> retry((u64)blocks * 256, st), n_retry(blocks, st);
-            table_claim_kernel<<<blocks, 256, 0, st>>>(cols.a[cur], recV, n_rec, slots, nsec, where.p, retry.p, n_retry.p);
+            table_claim_kernel<<<blocks, 256, 0, st>>>(cols.a[cur], n_rec, slots, nsec, where.p, retry.p, n_retry.p);
             SG_LAUNCHED();
-            table_insert_sorted_kernel<<<blocks, 64, 0, st>>>(cols.a[cur], recV, retry.p, n_retry.p, c.F.p, c.RC.p, c.len.p, SW, c.SWS, h, slots, nsec,
-                                                               where.p, d_overflow.p);
+            table_insert_sorted_kernel<<<blocks, 64, 0, st>>>(cols.a[cur], cols.b[cur], retry.p, n_retry.p, slots, nsec, where.p, d_overflow.p);
             SG_LAUNCHED();
+            if (stage_stats_enabled()) {
+                std::vector<u32> h_retry(blocks);
+                SG_CUDA(cudaMemcpyAsync(h_retry.data(), n_retry.p, blocks * sizeof(u32), cudaMemcpyDeviceToHost, st));
+                SG_CUDA(cudaStreamSynchronize(st));
+                u64 tot = 0;
+                for (u32 x : h_retry) tot += x;
+                fprintf(stderr, "sage2gpu stats: build_table records=%llu retry_records=%llu\n", (unsigned long long)n_rec, (unsigned long long)tot);
+            }
         }
     }
 
     DevBuf<u32> run(cap, st), off(cap, st), d_total(1, st);
     DevBuf<unsigned long long> d_cnt(2, st);
     SG_CUDA(cudaMemsetAsync(d_cnt.p, 0, 2 * sizeof(unsigned long long), st));
-    table_runs_kernel<<<big_grid(cap), 256, 0, st>>>(slots, cap, run.p, d_cnt.p);
+    table_runs_kernel<<<big_grid(cap), 256, 0, st>>>(slots, cap, recV, run.p, d_cnt.p);
     SG_LAUNCHED();
     exclusive_scan_u32(run.p, off.p, cap, d_total.p, st);
     u32 M = 0;
