@@ -152,6 +152,11 @@ def map_queries(name: str, n: int = 4000, seed: int = 777):
     reads of the data set as they are, reverse-complemented, lower-cased, with one substitution (mostly absent),
     truncated / extended (absent or bad), with an N (bad), palindromes, and reads longer than any in the set."""
     reads, k = get(name)
+    return map_queries_of(reads, n, seed), k
+
+
+def map_queries_of(reads, n: int = 4000, seed: int = 777) -> list[bytes]:
+    """The queries of map_queries drawn from the read list `reads`."""
     reads = synth.to_list(reads) if not isinstance(reads, list) else reads
     rng = np.random.default_rng(seed)
     comp = {65: 84, 67: 71, 71: 67, 84: 65, 97: 116, 99: 103, 103: 99, 116: 97, 78: 78}
@@ -181,4 +186,4 @@ def map_queries(name: str, n: int = 4000, seed: int = 777):
         else:
             r = bytes(rng.choice(list(b"ACGT"), size=int(rng.integers(1, 400))).astype(np.uint8))
         out.append(r)
-    return out, k
+    return out

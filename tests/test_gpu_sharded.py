@@ -9,6 +9,7 @@ import pytest
 import torch
 
 import datasets
+import long_datasets
 from oracle import oracle
 from sage2_b200 import api, multi, synth
 from test_gpu_parity import _compare, BIG
@@ -17,7 +18,12 @@ pytestmark = pytest.mark.gpu
 
 
 def _sharded(name, world, batch_reads=1 << 19, p2p=False):
-    reads, k = datasets.get(name) if name in datasets.DATASETS else synth.config(name)
+    if name in datasets.DATASETS:
+        reads, k = datasets.get(name)
+    elif name in long_datasets.LONG_DATASETS:
+        reads, k = long_datasets.get(name)
+    else:
+        reads, k = synth.config(name)
     b, off = synth.concat(reads)
     o = oracle.OracleRun(b, off, k)
     dev = torch.device("cuda", 0)
