@@ -183,6 +183,20 @@ int sage2gpu_table_gather_finish(sage2gpu_ctx *ctx, const uint64_t *entry_counts
  * phase_a_import       rank src_rank's slice of the phase-A arrays of `src` into `ctx` (+ element-wise maximum of the
  *                        containment ids): the exchange of sage2gpu_phase_a_buffers */
 int sage2gpu_load_finish_packed(sage2gpu_ctx *ctx, uint64_t *n_reads, int *max_read_length, uint64_t *good_reads, uint64_t *total_bp);
+/* A streamed upload spread over several contexts (each received a part of the input through _append / _append_text):
+ *   load_max_length      the longest read appended to this context since sage2gpu_load_begin (nothing is packed)
+ *   [maximum over the contexts]
+ *   load_finish_slice    = pack_slice on the uploaded reads: filtered and packed at the record stride of max_read_length (the
+ *                        longest read of the WHOLE read set), this context's slice for raw_gather_layout; *n_reads = its reads */
+int sage2gpu_load_max_length(sage2gpu_ctx *ctx, int *max_read_length);
+int sage2gpu_load_finish_slice(sage2gpu_ctx *ctx, int max_read_length, uint64_t *n_reads, uint64_t *good_reads, uint64_t *total_bp,
+                               uint64_t *record_words);
+/* After sage2gpu_reads_gather_finish (or any load that organised the reads): the bytes of the table this context would hold
+ * with `world` contexts, replicated (build_hash_table_part + table_gather_*: all shards) or sharded (build_hash_table_shard: one
+ * shard).  Slot bytes are exact; entry bytes are an upper bound (4 entries per unique read).  *device_free_bytes (may be NULL) =
+ * cudaMemGetInfo's free memory of the context's GPU, shared by all contexts on it.  For choosing between the two layouts. */
+int sage2gpu_table_bytes(sage2gpu_ctx *ctx, int world, uint64_t *replicated_slot_bytes, uint64_t *replicated_entry_bytes,
+                         uint64_t *sharded_slot_bytes, uint64_t *sharded_entry_bytes, uint64_t *device_free_bytes);
 int sage2gpu_peer_copy(sage2gpu_ctx *dst, void *dst_ptr, sage2gpu_ctx *src, const void *src_ptr, uint64_t n_bytes);
 int sage2gpu_phase_a_import(sage2gpu_ctx *ctx, sage2gpu_ctx *src, int src_rank);
 
@@ -223,7 +237,8 @@ int sage2gpu_phase_a_sharded_end(sage2gpu_ctx *ctx);
 /* The same exchange over PEER MEMORY (NVLink / NVSwitch P2P) instead of an all-to-all of the host: every rank owns a
  * "mailbox" in its device memory which the other ranks map (CUDA IPC between processes: hand the 64-byte
  * ipc_handle_out of mailbox_create to the other ranks and pass it to their mailbox_open; inside one process pass
- * *local_ptr instead).  The mailbox holds, per peer, room for the windows of max_reads_per_batch reads.
+ * *local_ptr instead: a mailbox on another GPU gets peer access enabled, and mailbox_open fails when the two GPUs cannot
+ * access each other's memory).  The mailbox holds, per peer, room for the windows of max_reads_per_batch reads.
  *   route_post     = route_begin, but the routing kernel stores every query straight into its owner's mailbox
  *   [barrier between the ranks]
  *   answer_post    = shard_answer out of the own mailbox; answers and bucket entries are copied into the sources' mailboxes
@@ -264,7 +279,9 @@ int sage2gpu_digest(sage2gpu_ctx *ctx, uint64_t *reads_digest, uint64_t *edges_d
  * 1 = min-hash order (reads that share k-mers are searched together, so slot sectors and partner records hit L2),
  * -1 = the default.  "low_memory": 1 = the large buffers are released (and returned to the driver) as soon as no later stage of the step
  * needs them -- the packed input after organizeReads, the table before the edge sort; 2 = the workspace too, after every
- * call (for read sets near the capacity of the GPU).  "fast_scan": 1 = phase A tries the superstring scan first (default), 0 = hit-by-hit kernel only. */
+ * call (for read sets near the capacity of the GPU).  Switched on when the reads are already organised (and gathered), it
+ * releases at once what it would have released by then: the packed input, the context's packed slice and unique run, the
+ * workspace.  "fast_scan": 1 = phase A tries the superstring scan first (default), 0 = hit-by-hit kernel only. */
 int sage2gpu_set_option(sage2gpu_ctx *ctx, const char *name, int64_t value);
 
 int sage2gpu_get_counters(const sage2gpu_ctx *ctx, sage2gpu_counters *out);

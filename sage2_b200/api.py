@@ -57,7 +57,7 @@ EXPORTS = ["sage2gpu_create", "sage2gpu_destroy", "sage2gpu_last_error", "sage2g
            "sage2gpu_table_shard_info", "sage2gpu_table_gather_layout", "sage2gpu_table_gather_finish",
            "sage2gpu_pack_slice", "sage2gpu_raw_gather_layout", "sage2gpu_raw_gather_finish", "sage2gpu_organize_partition",
            "sage2gpu_synth_reads", "sage2gpu_build_hash_table_part", "sage2gpu_load_finish_packed", "sage2gpu_peer_copy",
-           "sage2gpu_phase_a_import"]
+           "sage2gpu_phase_a_import", "sage2gpu_load_max_length", "sage2gpu_load_finish_slice", "sage2gpu_table_bytes"]
 
 _lib = None
 
@@ -91,6 +91,9 @@ def load_library():
         lib.sage2gpu_load_count.argtypes = [vp, u64p]
         lib.sage2gpu_load_remove.argtypes = [vp, C.c_uint64, C.c_uint64]
         lib.sage2gpu_load_finish.argtypes = [vp]
+        lib.sage2gpu_load_max_length.argtypes = [vp, C.POINTER(C.c_int)]
+        lib.sage2gpu_load_finish_slice.argtypes = [vp, C.c_int, u64p, u64p, u64p, u64p]
+        lib.sage2gpu_table_bytes.argtypes = [vp, C.c_int, u64p, u64p, u64p, u64p, u64p]
         lib.sage2gpu_host_alloc.argtypes = [C.c_uint64]
         lib.sage2gpu_host_alloc.restype = vp
         lib.sage2gpu_host_free.argtypes = [vp]
@@ -205,6 +208,38 @@ class Sage2Gpu:
             self._check(self._lib.sage2gpu_load_append(self._h, bases.ctypes.data, offsets[r0:r1 + 1].ctypes.data, r1 - r0),
                         "load_append")
         self._check(self._lib.sage2gpu_load_finish(self._h), "load_finish")
+
+    def load_begin(self, min_overlap: int):
+        self._check(self._lib.sage2gpu_load_begin(self._h, int(min_overlap)), "load_begin")
+
+    def load_append(self, bases: np.ndarray, offsets: np.ndarray):
+        """One chunk of a streamed upload: read r = bases[offsets[r], offsets[r+1]).  The buffers are kept alive until the
+        next call on this context (the library may still be copying them)."""
+        bases = np.ascontiguousarray(bases, dtype=np.uint8)
+        offsets = np.ascontiguousarray(offsets, dtype=np.int64)
+        self._keep = (bases, offsets)
+        self._check(self._lib.sage2gpu_load_append(self._h, bases.ctypes.data, offsets.ctypes.data, len(offsets) - 1), "load_append")
+
+    def load_max_length(self) -> int:
+        """Longest read appended since load_begin (nothing is packed)."""
+        m = C.c_int()
+        self._check(self._lib.sage2gpu_load_max_length(self._h, C.byref(m)), "load_max_length")
+        return int(m.value)
+
+    def load_finish_slice(self, max_read_length: int) -> dict:
+        """The streamed upload packed as this context's slice, at the stride of the read set's longest read (as pack_slice)."""
+        n, g, b, w = (C.c_uint64() for _ in range(4))
+        self._check(self._lib.sage2gpu_load_finish_slice(self._h, int(max_read_length), C.byref(n), C.byref(g), C.byref(b), C.byref(w)),
+                    "load_finish_slice")
+        return {"n_reads": int(n.value), "good_reads": int(g.value), "total_bp": int(b.value), "record_words": int(w.value)}
+
+    def table_bytes(self, world: int) -> dict:
+        """Bytes of the table this context would hold with `world` contexts, replicated or sharded (slots exact, entries an
+        upper bound), and the free memory of its GPU."""
+        v = [C.c_uint64() for _ in range(5)]
+        self._check(self._lib.sage2gpu_table_bytes(self._h, int(world), *(C.byref(x) for x in v)), "table_bytes")
+        return {"replicated_slots": int(v[0].value), "replicated_entries": int(v[1].value), "sharded_slots": int(v[2].value),
+                "sharded_entries": int(v[3].value), "device_free": int(v[4].value)}
 
     def build_hash_table(self):
         self._check(self._lib.sage2gpu_build_hash_table(self._h), "build_hash_table")

@@ -252,6 +252,57 @@ int sage2gpu_load_finish_packed(sage2gpu_ctx *ctx, uint64_t *n_reads, int *max_r
     });
 }
 
+int sage2gpu_load_max_length(sage2gpu_ctx *ctx, int *max_read_length)
+{
+    return guarded(ctx, [&](sg::Context &c) {
+        SG_CHECK(c.up_open, "sage2gpu_load_begin must be called first");
+        SG_CHECK(max_read_length != nullptr, "null argument");
+        SG_CUDA(cudaEventSynchronize(c.up_event));
+        *max_read_length = sg::stage_uploaded_max_len(c);
+    });
+}
+
+int sage2gpu_load_finish_slice(sage2gpu_ctx *ctx, int max_read_length, uint64_t *n_reads, uint64_t *good_reads, uint64_t *total_bp,
+                               uint64_t *record_words)
+{
+    return guarded(ctx, [&](sg::Context &c) {
+        SG_CHECK(c.up_open, "sage2gpu_load_begin must be called first");
+        SG_CHECK(max_read_length >= 1, "the longest read of the whole read set must be given");
+        c.up_open = false;
+        SG_CUDA(cudaEventSynchronize(c.up_event));
+        StageTimer t(c.stream);
+        sg::stage_ingest_ascii(c, c.up_d_bases.p, c.up_d_offsets.p, (int64_t)c.up_reads, true, max_read_length);
+        c.up_d_bases.release(); c.up_d_offsets.release();
+        c.tm.ingest = t.stop();
+        if (n_reads) *n_reads = c.n_input;
+        if (good_reads) *good_reads = c.cnt.good_reads;
+        if (total_bp) *total_bp = c.cnt.total_bp;
+        if (record_words) *record_words = (uint64_t)c.SW;
+    });
+}
+
+int sage2gpu_table_bytes(sage2gpu_ctx *ctx, int world, uint64_t *replicated_slot_bytes, uint64_t *replicated_entry_bytes,
+                         uint64_t *sharded_slot_bytes, uint64_t *sharded_entry_bytes, uint64_t *device_free_bytes)
+{
+    return guarded(ctx, [&](sg::Context &c) {
+        SG_CHECK(c.have_reads, "the reads must be organised first");
+        SG_CHECK(world >= 1 && world <= sg::kMaxWorld, "bad world");
+        const sg::u64 U = c.cnt.unique_reads;
+        // stage_build_table: no table for an empty read set; at most 4U entries (one per key of a bucket), in any shard
+        const sg::u64 shard = U ? sg::table_shard_slots(U, world) * sizeof(sg::u64) : 0, entries = 4 * U * sizeof(sg::u32);
+        if (replicated_slot_bytes) *replicated_slot_bytes = shard * (sg::u64)world;
+        if (replicated_entry_bytes) *replicated_entry_bytes = entries;
+        if (sharded_slot_bytes) *sharded_slot_bytes = shard;
+        if (sharded_entry_bytes) *sharded_entry_bytes = entries;
+        if (device_free_bytes) {
+            size_t fr = 0, tot = 0;
+            SG_CUDA(cudaStreamSynchronize(c.stream));
+            SG_CUDA(cudaMemGetInfo(&fr, &tot));
+            *device_free_bytes = fr;
+        }
+    });
+}
+
 int sage2gpu_peer_copy(sage2gpu_ctx *dst, void *dst_ptr, sage2gpu_ctx *src, const void *src_ptr, uint64_t n_bytes)
 {
     if (!dst || !src) return SAGE2GPU_ERR_ARG;
@@ -777,7 +828,18 @@ int sage2gpu_set_option(sage2gpu_ctx *ctx, const char *name, int64_t value)
         SG_CHECK(name != nullptr, "null option name");
         const std::string n(name);
         if (n == "read_order") { SG_CHECK(value >= -1 && value <= 1, "read_order: -1 default, 0 id order, 1 min-hash order"); c.opt_read_order = (int)value; }
-        else if (n == "low_memory") { SG_CHECK(value >= 0 && value <= 2, "low_memory: 0, 1 or 2"); c.opt_low_memory = (int)value; c.arena.tight = value > 0; }
+        else if (n == "low_memory") {
+            SG_CHECK(value >= 0 && value <= 2, "low_memory: 0, 1 or 2");
+            c.opt_low_memory = (int)value; c.arena.tight = value > 0;
+            if (value > 0 && c.have_reads) {
+                // switched on after the reads were organised: release now what the mode would have released by then -- the packed
+                // input, this context's packed slice and its unique run before the gather -- and the workspace
+                SG_CUDA(cudaStreamSynchronize(c.stream));
+                c.raw.release(); c.raw_slice.release(); c.F_loc.release(); c.len_loc.release(); c.freq_loc.release();
+                c.arena.destroy();
+                sg::trim_default_pool(c.device, c.stream);
+            }
+        }
         else if (n == "fast_scan") { SG_CHECK(value >= -1 && value <= 1, "fast_scan: -1 default, 0 off, 1 on"); c.opt_fast_scan = (int)value; }
         else throw sg::CudaError("unknown option: " + n);
     });

@@ -141,6 +141,7 @@ void stage_raw_gather_finish(Context &c, u64 total_reads, u64 good_reads, u64 to
 // synth.cu: synthetic paired-end reads generated on the device (measurement aid)
 void stage_synth_reads(Context &c, uint8_t *d_bases, int64_t *d_offsets, u64 first_pair, u64 n_pairs, u64 genome_bp, int read_len, float mu, float sigma, u64 seed);
 void stage_upload_chunk(Context &c, const uint8_t *bases, const int64_t *offsets, int64_t n_reads);
+int stage_uploaded_max_len(Context &c);     // longest read of the streamed upload so far
 // parse.cu: record splitting of raw FASTA/FASTQ text on the device; false = irregular layout, nothing appended
 bool stage_parse_text_chunk(Context &c, const uint8_t *text, u64 n_bytes, bool final, int &marker, u64 max_records, u64 &consumed, u64 &n_records);
 void stage_remove_uploaded(Context &c, u64 first, u64 count);
@@ -148,6 +149,7 @@ void stage_organize_reads(Context &c, int rank = 0, int world = 1);   // world >
 void stage_reads_gather_layout(Context &c, const u64 *counts, void **F, void **len, void **freq, u64 *first, u64 *total);
 void stage_reads_gather_finish(Context &c);
 void stage_build_table(Context &c, int rank = 0, int world = 1, bool joint = false);   // key-hash shard `rank` of `world` (SURVEY 8(e)); joint: inside an array with room for all shards
+u64 table_shard_slots(u64 unique_reads, int world);     // slots of one key-hash shard of `world` (of the whole table when world = 1)
 void stage_table_gather_layout(Context &c, const u64 *entry_counts, void **slots, void **entries, u64 *slots_per_shard, u64 *entries_first);
 void stage_table_gather_finish(Context &c, const u64 *entry_counts, const u64 *distinct, const u64 *over);
 void stage_phase_a(Context &c, int rank = 0, int world = 1);

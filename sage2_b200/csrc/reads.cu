@@ -250,6 +250,26 @@ void stage_upload_chunk(Context &c, const uint8_t *bases, const int64_t *offsets
     c.up_bases += (u64)nb;
 }
 
+// longest of the n reads whose (device) offsets are d_o (caller holds an ArenaScope)
+static int longest_read(const int64_t *d_o, u64 n, cudaStream_t st)
+{
+    DevBuf<int> d_max(1, st);
+    SG_CUDA(cudaMemsetAsync(d_max.p, 0, sizeof(int), st));
+    unsigned g = grid_for(n, K1_WARPS * 32, 4);
+    if (g > kSMs * 8) g = kSMs * 8;
+    if (n > 0) { max_len_kernel<<<g, K1_WARPS * 32, 0, st>>>(d_o, n, d_max.p); SG_LAUNCHED(); }
+    int max_len = 0;
+    SG_CUDA(cudaMemcpyAsync(&max_len, d_max.p, sizeof(int), cudaMemcpyDeviceToHost, st));
+    SG_CUDA(cudaStreamSynchronize(st));
+    return max_len;
+}
+
+int stage_uploaded_max_len(Context &c)
+{
+    ArenaScope arena_scope(c.arena, c.stream);
+    return longest_read(c.up_d_offsets.p, c.up_reads, c.stream);
+}
+
 void stage_ingest_ascii(Context &c, const uint8_t *bases, const int64_t *offsets, int64_t n_reads, bool device_resident, int forced_max_len)
 {
     cudaStream_t st = c.stream;
@@ -277,14 +297,7 @@ void stage_ingest_ascii(Context &c, const uint8_t *bases, const int64_t *offsets
         d_b = c.d_bases.p; d_o = c.d_offsets.p;
     }
     // longest read decides the record stride
-    DevBuf<int> d_max(1, st);
-    SG_CUDA(cudaMemsetAsync(d_max.p, 0, sizeof(int), st));
-    unsigned g = grid_for((u64)n_reads, K1_WARPS * 32, 4);
-    if (g > kSMs * 8) g = kSMs * 8;
-    if (n_reads > 0) { max_len_kernel<<<g, K1_WARPS * 32, 0, st>>>(d_o, (u64)n_reads, d_max.p); SG_LAUNCHED(); }
-    int max_len = 0;
-    SG_CUDA(cudaMemcpyAsync(&max_len, d_max.p, sizeof(int), cudaMemcpyDeviceToHost, st));
-    SG_CUDA(cudaStreamSynchronize(st));
+    int max_len = longest_read(d_o, (u64)n_reads, st);
     // The reference has no length limit; this build packs reads of up to 1016 bases (kMaxWords 64-bit words per record).
     // Dropping a longer read silently would renumber every read after it, so the call fails instead.
     SG_CHECK(max_len <= 32 * kMaxWords - 8, "a read is longer than 1016 bases: not supported by this build of libsage2gpu");

@@ -549,6 +549,18 @@ void stage_mailbox_open(Context &c, int peer_rank, const void *ipc_handle, void 
         m.peer[peer_rank] = (char *)p; m.ipc[peer_rank] = true;
     } else {
         SG_CHECK(ptr != nullptr, "null peer pointer");
+        // a mailbox on another GPU of this process: the routing and barrier kernels store into it, which needs peer access
+        cudaPointerAttributes a;
+        SG_CUDA(cudaPointerGetAttributes(&a, ptr));
+        if (a.type == cudaMemoryTypeDevice && a.device != c.device) {
+            int can = 0;
+            SG_CUDA(cudaDeviceCanAccessPeer(&can, c.device, a.device));
+            SG_CHECK(can, "GPU " + std::to_string(c.device) + " cannot access the memory of GPU " + std::to_string(a.device) +
+                              " (no peer access between them): the mailbox of rank " + std::to_string(peer_rank) + " cannot be used");
+            const cudaError_t e = cudaDeviceEnablePeerAccess(a.device, 0);
+            if (e == cudaErrorPeerAccessAlreadyEnabled) cudaGetLastError();
+            else SG_CUDA(e);
+        }
         m.peer[peer_rank] = (char *)ptr; m.ipc[peer_rank] = false;
     }
 }

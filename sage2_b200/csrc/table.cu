@@ -311,6 +311,17 @@ static unsigned big_grid(u64 n, unsigned block = 256)
     return g > kSMs * 16u ? kSMs * 16u : g;
 }
 
+u64 table_shard_slots(u64 U, int world)
+{
+    // load factor <= 2/3 even if all 4U keys are distinct (typically ~0.5)
+    // (a shard expects 1/world of the keys; 10 % head room for the imbalance of the split)
+    const u64 n = 4 * U;
+    u64 nsec = (n + n / 2 + kSlotsPerSector - 1) / kSlotsPerSector;
+    if (world > 1) nsec = nsec / (u64)world + nsec / (10 * (u64)world) + 1;
+    if (nsec < 256) nsec = 256;
+    return nsec * kSlotsPerSector;
+}
+
 // rank / world: the key-hash shard this context holds (0 / 1 = the whole table).  A shard indexes only the keys
 // with key_owner(hash) == rank; every context still streams all 4U entries (the reads are replicated).
 void stage_build_table(Context &c, int rank, int world, bool joint)
@@ -326,13 +337,7 @@ void stage_build_table(Context &c, int rank, int world, bool joint)
     if (U == 0) { c.slots.release(); c.entries.release(); c.have_table = true; return; }
     const u64 n = 4 * U;
     SG_CHECK(n < 0xFFFFFFFFull, "at most 2^30-1 unique reads per context");
-
-    // load factor <= 2/3 even if all 4U keys are distinct (typically ~0.5)
-    // (a shard expects 1/world of the keys; 10 % head room for the imbalance of the split)
-    u64 nsec = (n + n / 2 + kSlotsPerSector - 1) / kSlotsPerSector;
-    if (world > 1) nsec = nsec / (u64)world + nsec / (10 * (u64)world) + 1;
-    if (nsec < 256) nsec = 256;
-    const u64 cap = nsec * kSlotsPerSector;
+    const u64 cap = table_shard_slots(U, world), nsec = cap / kSlotsPerSector;
     SG_CHECK(cap < 0xFFFFFFFFull, "slot index too large for one context");
     // joint: the shard is built in its place inside an array with room for all shards (stage_table_gather_* completes it)
     c.slots.alloc(c.tb_joint ? cap * (u64)world : cap, st);

@@ -8,8 +8,11 @@
 // Flags are the reference's: -f/--fileInput, -l/--listInput, -k/--minOverlap, -o/--outputDir,
 // -p/--prefix, -i/--inputPrefix, -m/--minStep, -M/--maxStep, -s/--saveAll, -d/--debug, -h/--help.
 // Added: --device N (CUDA ordinal), --reference PATH, --devices LIST (several GPUs in ONE process: one context per listed
-// device, every stage partitioned -- reads organised by key range, table built by key-hash shard, search by id slice --
-// and the all-gathers between the stages done as peer copies; no NCCL, no Python; same files out).
+// device; the input is dealt to the contexts piece by piece as it is read and each packs its part; every stage partitioned --
+// reads organised by key range, search by id slice -- and the all-gathers between the stages done as peer copies; no NCCL,
+// no Python; same files out).  The table is replicated on every context (built by key-hash shard, all-gathered) when it fits
+// beside the later stages on every GPU, otherwise sharded by key hash with the window probes routed through peer-memory
+// mailboxes (low-memory mode); SAGE2GPU_TABLE_LAYOUT=replicated|sharded forces the choice, the log states it.
 //
 // Differences, all stated in the log: steps 1-3 are one device pass, so a restart at -m 2 / -m 3
 // recomputes from the input files instead of loading <prefix>.reads / <prefix>.hashTable (results are
@@ -25,11 +28,15 @@
 #include <sys/wait.h>
 #include <unistd.h>
 
+#include <algorithm>
 #include <chrono>
+#include <condition_variable>
 #include <fstream>
 #include <iomanip>
 #include <iostream>
 #include <functional>
+#include <map>
+#include <mutex>
 #include <sstream>
 #include <stdexcept>
 #include <string>
@@ -181,19 +188,42 @@ struct Chunk {
     int64_t *offsets = nullptr;
     size_t cap_bases = 0, cap_reads = 0, n_reads = 0, n_bases = 0;
     bool pinned = false;
+    int owner = -1;             // context whose _append may still be reading the buffers
+    uint64_t call = 0;          // number of that call (Uploader::touch)
 };
 
+// reads [first, first + count) of context `ctx`'s upload came from one stretch of a file, in file order
+struct Segment {
+    int ctx;
+    uint64_t first, count;
+};
+
+// bytes of a text piece and of a sequential-parser chunk; SAGE2GPU_UPLOAD_PIECE_BYTES makes them smaller, so that a small
+// file is spread over several contexts (tests)
+size_t pieceBytes()
+{
+    static const size_t v = [] {
+        const char *e = getenv("SAGE2GPU_UPLOAD_PIECE_BYTES");
+        const long long x = e ? atoll(e) : 0;
+        return x >= 4096 ? (size_t)x : (size_t)32 << 20;
+    }();
+    return v;
+}
+
+// One context, or several that receive the pieces of the input in turn (read ids are ranks in the sorted set, so the
+// upload order is free).  The segments of the file being read say which context holds which of its records.
 class Uploader {
 public:
-    Uploader(sage2gpu_ctx *ctx, int k) : ctx_(ctx)
+    Uploader(const std::vector<sage2gpu_ctx *> &ctx, int k) : ctx_(ctx), received_(ctx.size(), 0), last_(ctx.size(), 0)
     {
-        if (!ctx_) return;          // --parse-only
+        if (ctx_.empty()) return;   // --parse-only
         for (Chunk &c : chunk_) {
-            c.cap_bases = (size_t)64 << 20;
+            c.cap_bases = std::min<size_t>((size_t)64 << 20, 2 * pieceBytes());
             c.cap_reads = (size_t)1 << 19;
             alloc(c);
         }
-        if (sage2gpu_load_begin(ctx_, k) != 0) printError("CUDA", sage2gpu_last_error(ctx_));
+        for (size_t r = 0; r < ctx_.size(); ++r)
+            if (sage2gpu_load_begin(ctx_[r], k) != 0) fail((int)r);
     }
     ~Uploader()
     {
@@ -214,41 +244,61 @@ public:
         c->n_reads++;
         c->offsets[c->n_reads] = (int64_t)c->n_bases;
     }
+    // one context: filter, pack, sort, dedupe (organizeReads)
     void finish()
     {
         flush();
-        if (sage2gpu_load_finish(ctx_) != 0) printError("CUDA", sage2gpu_last_error(ctx_));
+        if (sage2gpu_load_finish(ctx_[0]) != 0) fail(0);
     }
-    // several GPUs: filter + pack only; organizeReads follows partitioned over the contexts
-    void finishPacked(uint64_t &n_reads, int &max_len, uint64_t &good, uint64_t &bp)
-    {
-        flush();
-        if (sage2gpu_load_finish_packed(ctx_, &n_reads, &max_len, &good, &bp) != 0) printError("CUDA", sage2gpu_last_error(ctx_));
-    }
-    // everything added so far is on the device after this
+    // everything added so far is on the device after this, and no pinned buffer is in use
     void sync()
     {
-        if (!ctx_) return;
+        if (ctx_.empty()) return;
         flush();
-        if (sage2gpu_load_append(ctx_, nullptr, nullptr, 0) != 0) printError("CUDA", sage2gpu_last_error(ctx_));
+        for (size_t r = 0; r < ctx_.size(); ++r) {
+            if (sage2gpu_load_append(ctx_[r], nullptr, nullptr, 0) != 0) fail((int)r);
+            touch((int)r);
+        }
     }
-    sage2gpu_ctx *ctx() const { return ctx_; }
-    uint64_t count()
+    bool active() const { return !ctx_.empty(); }
+    // the context the next piece goes to
+    int next() const { return next_; }
+    sage2gpu_ctx *ctx(int r) const { return ctx_[r]; }
+    // device record splitting of one text piece on context next(); see sage2gpu_load_append_text
+    int appendText(const uint8_t *text, size_t n, bool final, int *marker, uint64_t max_records, uint64_t &consumed, uint64_t &nrec)
     {
-        uint64_t n = 0;
-        if (sage2gpu_load_count(ctx_, &n) != 0) printError("CUDA", sage2gpu_last_error(ctx_));
-        return n;
+        const int r = next_;
+        const int rc = sage2gpu_load_append_text(ctx_[r], text, n, final ? 1 : 0, marker, max_records, &consumed, &nrec);
+        touch(r);
+        if (rc == 0 && nrec) appended(r, nrec);
+        return rc;
     }
     // pinned buffer for raw file text (device-side record splitting)
     uint8_t *text(size_t &cap)
     {
-        if (!text_) { text_ = (uint8_t *)sage2gpu_host_alloc(kTextCap); if (!text_) printError("MEM_ALLOC", "pinned text buffer"); }
-        cap = kTextCap;
+        if (!text_) { text_ = (uint8_t *)sage2gpu_host_alloc(pieceBytes()); if (!text_) printError("MEM_ALLOC", "pinned text buffer"); }
+        cap = pieceBytes();
         return text_;
     }
+    std::vector<Segment> takeSegments() { std::vector<Segment> s; s.swap(segs_); return s; }
+    // drops the records [keep, end) of a file, in file order, from the contexts that hold them
+    void removeTail(const std::vector<Segment> &file, uint64_t keep)
+    {
+        uint64_t end = 0;
+        for (const Segment &s : file) end += s.count;
+        for (size_t i = file.size(); i-- > 0 && end > keep;) {     // from the back: the earlier segments of a context keep their place
+            const Segment &s = file[i];
+            const uint64_t start = end - s.count, from = std::max(start, keep);
+            if (sage2gpu_load_remove(ctx_[s.ctx], s.first + (from - start), end - from) != 0) fail(s.ctx);
+            touch(s.ctx);
+            received_[s.ctx] -= end - from;
+            end = start;
+        }
+    }
+    const std::vector<uint64_t> &received() const { return received_; }
+    [[noreturn]] void fail(int r) { printError("CUDA", sage2gpu_last_error(ctx_[r])); }
 
 private:
-    static constexpr size_t kTextCap = (size_t)32 << 20;
     uint8_t *text_ = nullptr;
     void alloc(Chunk &c)
     {
@@ -265,21 +315,43 @@ private:
         sage2gpu_host_free(c.offsets);
         c.bases = nullptr; c.offsets = nullptr;
     }
+    uint64_t touch(int r) { return last_[r] = ++calls_; }
+    void appended(int r, uint64_t n)
+    {
+        if (!segs_.empty() && segs_.back().ctx == r && segs_.back().first + segs_.back().count == received_[r]) segs_.back().count += n;
+        else segs_.push_back(Segment{ r, received_[r], n });
+        received_[r] += n;
+        next_ = (next_ + 1) % (int)ctx_.size();
+    }
     void flush()
     {
         Chunk &c = chunk_[cur_];
         if (c.n_reads) {
-            // returns once the PREVIOUS chunk's copy is complete; this chunk's copy runs while the parser fills the other buffer
-            if (sage2gpu_load_append(ctx_, c.bases, c.offsets, (int64_t)c.n_reads) != 0) printError("CUDA", sage2gpu_last_error(ctx_));
+            // returns once the copy of that context's PREVIOUS chunk is complete; this chunk's copy runs while the parser fills
+            // the other buffer
+            const int r = next_;
+            if (sage2gpu_load_append(ctx_[r], c.bases, c.offsets, (int64_t)c.n_reads) != 0) fail(r);
+            c.owner = r;
+            c.call = touch(r);
+            appended(r, c.n_reads);
         }
         cur_ ^= 1;
         Chunk &n = chunk_[cur_];
+        // a chunk's buffers are free once a LATER call on the context it went to has returned
+        if (n.owner >= 0 && last_[n.owner] <= n.call) {
+            if (sage2gpu_load_append(ctx_[n.owner], nullptr, nullptr, 0) != 0) fail(n.owner);
+            touch(n.owner);
+        }
+        n.owner = -1;
         n.n_reads = n.n_bases = 0;
         n.offsets[0] = 0;
     }
-    sage2gpu_ctx *ctx_;
+    std::vector<sage2gpu_ctx *> ctx_;
+    std::vector<uint64_t> received_, last_;     // reads per context; number of the latest call on it
+    std::vector<Segment> segs_;
     Chunk chunk_[2];
-    int cur_ = 0;
+    int cur_ = 0, next_ = 0;
+    uint64_t calls_ = 0;
 };
 
 // --parse-only: the input side alone (no device): record count, base count and an FNV-1a checksum of the
@@ -315,7 +387,7 @@ uint64_t parseSequential(Uploader &up, sg_host::FastAQStream &in, uint64_t max_r
 uint64_t readFile(Uploader &up, const std::string &path, uint64_t max_records, bool &used_device_parser)
 {
     used_device_parser = false;
-    if (!up.ctx()) {                       // --parse-only
+    if (!up.active()) {                    // --parse-only
         sg_host::FastAQStream in(path);
         return parseSequential(up, in, max_records);
     }
@@ -332,10 +404,10 @@ uint64_t readFile(Uploader &up, const std::string &path, uint64_t max_records, b
     }
     size_t cap = 0, have = 0;
     uint8_t *buf = up.text(cap);
-    int marker = 0;
+    int marker = 0;                        // the file's record layout ('@' / '>'), found in its first piece; the same for every context
     bool eof = false;
     uint64_t total = 0;
-    up.sync();                             // keep the upload order: everything added before is on the device
+    up.sync();                             // the records of this file form segments of their own
     for (;;) {
         while (have < cap && !eof) {
             const long n = is_gz ? (long)gzread(gz, buf + have, (unsigned)(cap - have)) : (long)read(fd, buf + have, cap - have);
@@ -343,7 +415,8 @@ uint64_t readFile(Uploader &up, const std::string &path, uint64_t max_records, b
         }
         if (have == 0) break;
         uint64_t consumed = 0, nrec = 0;
-        const int rc = sage2gpu_load_append_text(up.ctx(), buf, have, eof ? 1 : 0, &marker, max_records - total, &consumed, &nrec);
+        const int r = up.next();
+        const int rc = up.appendText(buf, have, eof, &marker, max_records - total, consumed, nrec);
         if (rc == SAGE2GPU_ERR_FORMAT || (rc == 0 && consumed == 0 && !eof)) {
             if (!gz) gz = gzdopen(fd, "r");                   // transparent mode, continues at the descriptor's offset
             if (!gz) { close(fd); throw std::runtime_error("cannot read " + path); }
@@ -352,7 +425,7 @@ uint64_t readFile(Uploader &up, const std::string &path, uint64_t max_records, b
             up.sync();
             return total;
         }
-        if (rc != 0) printError("CUDA", sage2gpu_last_error(up.ctx()));
+        if (rc != 0) up.fail(r);
         used_device_parser = true;
         total += nrec;
         have -= (size_t)consumed;
@@ -373,7 +446,8 @@ uint64_t readDataset(Uploader &up, const std::string &f1, const std::string &f2)
         bool dev1 = false, dev2 = false;
         if (f2.empty()) {
             n = readFile(up, f1, UINT64_MAX, dev1);
-        } else if (!up.ctx()) {
+            up.takeSegments();
+        } else if (!up.active()) {
             sg_host::MatePairStream in(f1, f2);     // --parse-only keeps the reference's alternating order
             std::vector<uint8_t> seq;
             uint64_t len = 0;
@@ -381,14 +455,16 @@ uint64_t readDataset(Uploader &up, const std::string &f1, const std::string &f2)
         } else {
             // The reference alternates mate 1 / mate 2 and stops when a file ends (inputReader.cpp:26-49): with n1 and n2
             // records it keeps min(n1, n2 + 1) of file 1 and min(n2, n1) of file 2.  Read ids are ranks in the sorted set,
-            // so the upload order is free: file 1, then file 2 capped at n1, then the surplus of file 1 is dropped.
-            const uint64_t start1 = up.count();
+            // so the upload order is free: file 1, then file 2 capped at n1, then the surplus of file 1 (its last records, in
+            // whichever contexts they went to) is dropped.
             const uint64_t n1 = readFile(up, f1, UINT64_MAX, dev1);
+            const std::vector<Segment> file1 = up.takeSegments();
             const uint64_t n2 = readFile(up, f2, n1, dev2);
+            up.takeSegments();
             uint64_t keep1 = n1;
             if (n1 > n2 + 1) {
                 keep1 = n2 + 1;
-                if (sage2gpu_load_remove(up.ctx(), start1 + keep1, n1 - keep1) != 0) printError("CUDA", sage2gpu_last_error(up.ctx()));
+                up.removeTail(file1, keep1);
             }
             n = keep1 + n2;
         }
@@ -453,11 +529,12 @@ int runReference(const Options &o, int fromStep)
 }  // namespace
 
 // ---- several GPUs in one process ---------------------------------------------------------------------------------
-// One context per device, one host thread per context and stage (the library calls block), peer copies between the
-// stages.  The steps are those of sage2_b200/multi.py::partitioned_slice_steps with context 0 holding the whole input as
-// its "slice" (it received the streamed upload) and the others an empty one.
+// One context per listed device, one host thread per context (the library calls block), peer copies between the stages.
+// The input is spread over the contexts as it is read; the steps are those of sage2_b200/multi.py::partitioned_slice_steps
+// (table replicated) or partitioned_slice_sharded_steps (table sharded, low-memory mode), whichever fits.
 struct MultiGpu {
     std::vector<sage2gpu_ctx *> ctx;
+    std::vector<int> device;
     int G() const { return (int)ctx.size(); }
     void each(const std::function<void(int)> &fn)
     {
@@ -476,31 +553,137 @@ struct MultiGpu {
     }
 };
 
-// steps 1 (after the upload into context 0) to 3; the result is complete in every context
-void runPartitioned(MultiGpu &m, Uploader &up, int k)
+// Rendezvous of the G threads of one sharded build: every thread passes its value and gets the maximum over all of them.
+class HostSync {
+public:
+    explicit HostSync(int n) : n_(n) {}
+    uint64_t max(uint64_t v)
+    {
+        std::unique_lock<std::mutex> lk(mu_);
+        const uint64_t gen = gen_;
+        acc_ = std::max(acc_, v);
+        if (++arrived_ == n_) { result_ = acc_; acc_ = 0; arrived_ = 0; ++gen_; cv_.notify_all(); }
+        else cv_.wait(lk, [&] { return gen_ != gen; });
+        return result_;
+    }
+    void wait() { max(0); }
+
+private:
+    std::mutex mu_;
+    std::condition_variable cv_;
+    const int n_;
+    int arrived_ = 0;
+    uint64_t gen_ = 0, acc_ = 0, result_ = 0;
+};
+
+// Reads per routed batch of the sharded table (as tools/run_cfg5.py); SAGE2GPU_ROUTE_BATCH_READS makes it smaller (tests).
+uint64_t routeBatchReads()
+{
+    const char *e = getenv("SAGE2GPU_ROUTE_BATCH_READS");
+    const long long v = e ? atoll(e) : 0;
+    return v > 0 ? (uint64_t)v : (uint64_t)1 << 18;
+}
+
+// Memory the stages after the table need beside it, per unique read of a context: phase-A arrays, phase-B records and
+// workspace.  From the per-GPU sizes of config #5 (DESIGN.md section 4c): at full size 20 + 17.6 + 25 GB for 562 M unique
+// reads (111 B per read); at half size the replicated peak of 99.8 GB less the reads (F + RC, 36 GB) and the table
+// (15 GB) leaves 49 GB for 281 M unique reads (174 B per read).  Rounded up; how close it comes has not been measured.
+constexpr uint64_t kReserveBytesPerUniqueRead = 192;
+
+// One thread of the sharded build (multi.py::sharded_graph_steps over peer-memory mailboxes).  Every library call returns
+// with its stream drained, so the rendezvous of the threads (HostSync) separates the steps of a routed batch; the device
+// barrier (sage2gpu_mailbox_barrier) is for ranks in different processes.  Inside one process it could stall: its kernel
+// spins on the device until the peers arrive, and a synchronous free of another context on the same GPU waits for it.
+void shardedSteps(MultiGpu &m, HostSync &hs, std::vector<void *> &box, int r, uint64_t batch, uint64_t &redo_max, uint64_t &list_max)
 {
     const int G = m.G();
-    uint64_t N = 0, good = 0, bp = 0;
-    int max_len = 0;
-    up.finishPacked(N, max_len, good, bp);
-    std::vector<uint64_t> counts(G, 0), zero(G, 0);
-    counts[0] = N;
-    m.each([&](int r) {
-        if (r > 0) m.check(r, sage2gpu_pack_slice(m.ctx[r], nullptr, nullptr, 0, k, 1, max_len > 0 ? max_len : 1, nullptr, nullptr, nullptr));
-    });
-    sage2gpu_counters c0;
-    sage2gpu_get_counters(m.ctx[0], &c0);
-    const uint64_t SW = c0.record_words;
+    uint64_t box_reads = 0;
+    auto openMailboxes = [&](uint64_t reads) {
+        hs.wait();                  // nobody stores into the old mailboxes any more
+        m.check(r, sage2gpu_mailbox_create(m.ctx[r], r, G, reads, nullptr, &box[r]));
+        hs.wait();
+        for (int q = 0; q < G; ++q) if (q != r) m.check(r, sage2gpu_mailbox_open(m.ctx[r], q, nullptr, box[q]));
+        hs.wait();
+        box_reads = reads;
+    };
+    auto route = [&](int what, uint64_t first, uint64_t count, int exact, bool posted) {
+        if (!posted) m.check(r, sage2gpu_route_post(m.ctx[r], what, first, count, exact, nullptr, nullptr));
+        hs.wait();
+        m.check(r, sage2gpu_answer_post(m.ctx[r], exact, nullptr));
+        hs.wait();
+        m.check(r, sage2gpu_route_collect(m.ctx[r]));
+    };
+    // a list batch (redo reads, reads left for phase C) travels as ONE batch: the mailboxes of all contexts grow to the largest list
+    auto fitMailbox = [&](uint64_t n_list) {
+        const uint64_t need = hs.max(n_list);
+        if (need > box_reads) openMailboxes(need);
+        return need;
+    };
+
+    sage2gpu_counters c;
+    sage2gpu_get_counters(m.ctx[r], &c);
+    const uint64_t U = c.unique_reads, chunk = U ? (U + G - 1) / G : 0;
+    m.check(r, sage2gpu_build_hash_table_shard(m.ctx[r], r, G));
+    openMailboxes(std::max<uint64_t>(1, std::min(batch, chunk)));      // no batch is larger than a context's slice
+    uint64_t first = 0, count = 0;
+    m.check(r, sage2gpu_phase_a_sharded_begin(m.ctx[r], r, G, &first, &count));
+    const uint64_t n_batches = chunk ? (chunk + batch - 1) / batch : 0;      // the same on every context: the steps stay in lockstep
+    uint64_t redo = 0;
+    for (uint64_t b = 0; b < n_batches; ++b) {
+        const uint64_t lo = std::min(first + b * batch, first + count), n = std::min(batch, first + count - lo);
+        route(0, lo, n, 0, false);
+        uint64_t nr = 0;
+        m.check(r, sage2gpu_phase_a_routed(m.ctx[r], &nr));
+        redo += nr;
+    }
+    const uint64_t redo_all = hs.max(redo);
+    if (redo_all) {
+        // 24-bit tag collisions: those reads once more, with probes the owners verify
+        fitMailbox(redo);
+        route(2, 0, 0, 1, false);
+        uint64_t left = 0;
+        m.check(r, sage2gpu_phase_a_routed(m.ctx[r], &left));
+        if (left) printError("CUDA", "device context " + std::to_string(r) + ": " + std::to_string(left) + " reads still unresolved after the verified pass");
+    }
+    m.check(r, sage2gpu_phase_a_sharded_end(m.ctx[r]));
+    hs.wait();
+    for (int q = 0; q < G; ++q) if (q != r) m.check(r, sage2gpu_phase_a_import(m.ctx[r], m.ctx[q], q));
+    hs.wait();
+    m.check(r, sage2gpu_phase_b(m.ctx[r]));
+    sage2gpu_get_counters(m.ctx[r], &c);
+    const uint64_t list = fitMailbox(c.left_to_explore);
+    uint64_t n_list = 0;
+    m.check(r, sage2gpu_route_post(m.ctx[r], 1, 0, 0, 1, &n_list, nullptr));      // reads left for phase C: the same list everywhere
+    if (n_list) route(1, 0, 0, 1, true);
+    m.check(r, sage2gpu_finish_graph(m.ctx[r]));
+    if (r == 0) { redo_max = redo_all; list_max = list; }
+}
+
+// steps 1 (after the upload spread over the contexts) to 3; the result is complete in every context.  Returns whether the
+// table was replicated (else every context holds one shard of it).
+bool runPartitioned(MultiGpu &m, int k)
+{
+    const int G = m.G();
+    // the contexts agree on the longest read: it fixes the record stride of every slice
+    std::vector<int> ml(G, 0);
+    m.each([&](int r) { m.check(r, sage2gpu_load_max_length(m.ctx[r], &ml[r])); });
+    const int max_len = std::max(1, *std::max_element(ml.begin(), ml.end()));
+    std::vector<uint64_t> counts(G, 0), good(G, 0), bp(G, 0), sw(G, 0);
+    m.each([&](int r) { m.check(r, sage2gpu_load_finish_slice(m.ctx[r], max_len, &counts[r], &good[r], &bp[r], &sw[r])); });
+    uint64_t N = 0, good_all = 0, bp_all = 0;
+    for (int r = 0; r < G; ++r) { N += counts[r]; good_all += good[r]; bp_all += bp[r]; }
+    const uint64_t SW = sw[0];
     std::vector<void *> p(G, nullptr), p2(G, nullptr), p3(G, nullptr);
     m.each([&](int r) { m.check(r, sage2gpu_raw_gather_layout(m.ctx[r], r, G, counts.data(), &p[r], nullptr, nullptr)); });
     {
         std::vector<uint64_t> off(G, 0), bytes(G, 0);
-        bytes[0] = N * SW * 8;
+        uint64_t acc = 0;
+        for (int q = 0; q < G; ++q) { off[q] = acc * SW * 8; bytes[q] = counts[q] * SW * 8; acc += counts[q]; }
         m.gather(p, off, bytes);
     }
     std::vector<uint64_t> uloc(G, 0);
     m.each([&](int r) {
-        m.check(r, sage2gpu_raw_gather_finish(m.ctx[r], N, good, bp));
+        m.check(r, sage2gpu_raw_gather_finish(m.ctx[r], N, good_all, bp_all));
         m.check(r, sage2gpu_organize_partition(m.ctx[r], r, G, &uloc[r]));
     });
     std::vector<uint64_t> stride(G, 0);
@@ -513,9 +696,50 @@ void runPartitioned(MultiGpu &m, Uploader &up, int k)
         m.gather(p2, off2, bytes2);
         m.gather(p3, off2, bytes2);
     }
+    m.each([&](int r) { m.check(r, sage2gpu_reads_gather_finish(m.ctx[r])); });
+
+    // the layout: the table replicated on every context (faster) when it fits beside the later stages on every GPU, else sharded
+    sage2gpu_counters c0;
+    sage2gpu_get_counters(m.ctx[0], &c0);
+    std::map<int, uint64_t> need, avail;
+    uint64_t rs = 0, re = 0, ss = 0, se = 0;
+    for (int r = 0; r < G; ++r) {
+        uint64_t fr = 0;
+        m.check(r, sage2gpu_table_bytes(m.ctx[r], G, &rs, &re, &ss, &se, &fr));
+        need[m.device[r]] += rs + re + kReserveBytesPerUniqueRead * c0.unique_reads;
+        avail[m.device[r]] = fr;
+    }
+    bool replicated = true;
+    for (const auto &d : need) replicated = replicated && d.second <= avail[d.first];
+    const char *forced = getenv("SAGE2GPU_TABLE_LAYOUT");
+    if (forced && strcmp(forced, "replicated") && strcmp(forced, "sharded")) printError("ARGUMENT", "SAGE2GPU_TABLE_LAYOUT must be replicated or sharded");
+    const bool fits = replicated;
+    if (forced) replicated = !strcmp(forced, "replicated");
+    logStream << "Table layout: " << (replicated ? "replicated" : "sharded") << (forced ? " (SAGE2GPU_TABLE_LAYOUT)" : "") << ". Per context: replicated table "
+              << rs + re << " bytes (slots " << rs << ", entries <= " << re << "), sharded table " << ss + se << " bytes (slots " << ss
+              << ", entries <= " << se << "), reserve for the later stages " << kReserveBytesPerUniqueRead * c0.unique_reads << " bytes ("
+              << kReserveBytesPerUniqueRead << " per unique read).\n";
+    for (const auto &d : need)
+        logStream << "\tGPU " << d.first << ": replicated table + reserve of its contexts " << d.second << " bytes, free " << avail[d.first] << " bytes: "
+                  << (d.second <= avail[d.first] ? "fits" : "does not fit") << "\n";
+    logStream << "\tThe replicated table " << (fits ? "fits" : "does not fit") << " on every GPU.\n";
+    logStream.flush();
+
+    if (!replicated) {
+        HostSync hs(G);
+        std::vector<void *> box(G, nullptr);
+        const uint64_t batch = routeBatchReads();
+        uint64_t redo = 0, list = 0;
+        m.each([&](int r) {
+            m.check(r, sage2gpu_set_option(m.ctx[r], "low_memory", 1));
+            shardedSteps(m, hs, box, r, batch, redo, list);
+        });
+        logStream << "\tSharded table: " << G << " shards, routed batches of " << batch << " reads; reads of the verified redo pass (max over the contexts): "
+                  << redo << "; list batch of the reads left for phase C: " << list << " reads\n";
+        return false;
+    }
     std::vector<uint64_t> ec(G, 0), dk(G, 0), ov(G, 0), sps(G, 0);
     m.each([&](int r) {
-        m.check(r, sage2gpu_reads_gather_finish(m.ctx[r]));
         m.check(r, sage2gpu_build_hash_table_part(m.ctx[r], r, G));
         m.check(r, sage2gpu_table_shard_info(m.ctx[r], nullptr, &ec[r], &dk[r], &ov[r]));
     });
@@ -535,6 +759,7 @@ void runPartitioned(MultiGpu &m, Uploader &up, int k)
         for (int q = 0; q < G; ++q) if (q != r) m.check(r, sage2gpu_phase_a_import(m.ctx[r], m.ctx[q], q));
     });
     m.each([&](int r) { m.check(r, sage2gpu_finish_graph(m.ctx[r])); });
+    return true;
 }
 
 // --devices with more than one entry: steps 1-3 partitioned over the listed GPUs, the same files and log lines out
@@ -545,28 +770,42 @@ int runOnSeveralDevices(const Options &o, const std::string &base)
         sage2gpu_ctx *c = nullptr;
         if (sage2gpu_create(&c, d) != 0) printError("CUDA", "no usable CUDA device " + std::to_string(d) + " (libsage2gpu has no CPU fallback)");
         m.ctx.push_back(c);
+        m.device.push_back(d);
     }
-    logStream << "Devices: " << m.G() << " contexts (one per listed GPU), every stage partitioned, peer copies between the stages.\n";
+    logStream << "Devices: " << m.G() << " contexts (one per listed GPU), the input spread over them, every stage partitioned, peer copies between the stages.\n";
     banner("STEP 1", "                                          organizing reads");
     auto t0 = std::chrono::steady_clock::now();
     {
-        Uploader up(m.ctx[0], o.minOverlap);
+        Uploader up(m.ctx, o.minOverlap);
         if (!o.listInput.empty()) loadFromList(up, o.listInput);
         else readDataset(up, o.fileInput, "");
+        up.sync();
         logStream << "Parsed and uploaded in " << seconds_since(t0) << " sec.\n";
-        banner("STEPS 2-3", "                             building hash table and overlap graph");
-        auto t1 = std::chrono::steady_clock::now();
-        runPartitioned(m, up, o.minOverlap);
-        logStream << "Functions organizeReads() .. sortEconomyGraph() on " << m.G() << " devices in " << seconds_since(t1) << " sec.\n";
+        logStream << "\tReads received per context:";
+        for (uint64_t n : up.received()) logStream << " " << n;
+        logStream << "\n";
     }
+    banner("STEPS 2-3", "                             building hash table and overlap graph");
+    auto t1 = std::chrono::steady_clock::now();
+    const bool replicated = runPartitioned(m, o.minOverlap);
+    logStream << "Functions organizeReads() .. sortEconomyGraph() on " << m.G() << " devices in " << seconds_since(t1) << " sec.\n";
     sage2gpu_counters cnt;
     sage2gpu_get_counters(m.ctx[0], &cnt);
+    if (!replicated) {      // one shard per context: the table is the sum of the shards
+        cnt.table_capacity = cnt.distinct_keys = cnt.keys_over_threshold = 0;
+        for (sage2gpu_ctx *c : m.ctx) {
+            sage2gpu_counters s;
+            sage2gpu_get_counters(c, &s);
+            cnt.table_capacity += s.table_capacity; cnt.distinct_keys += s.distinct_keys; cnt.keys_over_threshold += s.keys_over_threshold;
+        }
+    }
     logStream << std::setw(20) << "Total reads: " << cnt.total_reads << "\n";
     logStream << std::setw(20) << "Good reads: " << cnt.good_reads << "\n";
     logStream << std::setw(20) << "Bad reads: " << cnt.total_reads - cnt.good_reads << "\n";
     logStream << "\t" << std::setw(21) << "Average read length: " << cnt.avg_len << "\n";
     logStream << "\tNumber of unique reads: " << cnt.unique_reads << "\n";
-    logStream << "\tSize of hash table: " << cnt.table_capacity << " slots, " << cnt.distinct_keys << " distinct keys\n";
+    logStream << "\tSize of hash table: " << cnt.table_capacity << " slots, " << cnt.distinct_keys << " distinct keys"
+              << (replicated ? "" : " (sum over the shards)") << "\n";
     logStream << "\tNumber of hashes over threshold: " << cnt.keys_over_threshold << "\n";
     logStream << "\tTotal reads contained by extension: " << cnt.contained_ext << "\n";
     logStream << "\tTotal reads contained by size: " << cnt.contained_size << "\n";
@@ -607,7 +846,7 @@ int main(int argc, char **argv)
         ParseSink sink;
         g_parse_sink = &sink;
         logStream.open("/dev/null");
-        Uploader none(nullptr, o.minOverlap);
+        Uploader none({}, o.minOverlap);
         if (!o.listInput.empty()) loadFromList(none, o.listInput);
         else readDataset(none, o.fileInput, "");
         printf("{\"reads\": %llu, \"bases\": %llu, \"fnv1a\": \"%016llx\"}\n", (unsigned long long)sink.reads,
@@ -648,7 +887,7 @@ int main(int argc, char **argv)
     banner("STEP 1", "                                          organizing reads");
     auto t0 = std::chrono::steady_clock::now();
     {
-        Uploader up(ctx, o.minOverlap);
+        Uploader up({ ctx }, o.minOverlap);
         if (!o.listInput.empty()) loadFromList(up, o.listInput);
         else readDataset(up, o.fileInput, "");
         logStream << "Parsed and uploaded in " << seconds_since(t0) << " sec.\n";
