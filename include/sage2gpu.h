@@ -25,7 +25,8 @@ extern "C" {
 typedef struct sage2gpu_ctx sage2gpu_ctx;
 
 enum { SAGE2GPU_OK = 0, SAGE2GPU_ERR_CUDA = 1, SAGE2GPU_ERR_ARG = 2, SAGE2GPU_ERR_STATE = 3, SAGE2GPU_ERR_IO = 4,
-       SAGE2GPU_ERR_FORMAT = 5 /* sage2gpu_load_append_text: not the regular 4-line FASTQ / 2-line FASTA layout */ };
+       SAGE2GPU_ERR_FORMAT = 5 /* sage2gpu_load_append_text: not the regular 4-line FASTQ / 2-line FASTA layout;
+                                  sage2gpu_*saved_reads*: the file breaks the grammar of a saved .reads file */ };
 
 /* Log counters of the reference (readLoader.cpp:164-169,257; hashTable.cpp:86,124;
  * economyGraph.cpp:485-487,569-571) plus the workload sizes the roofline needs. */
@@ -101,6 +102,40 @@ int sage2gpu_load_remove(sage2gpu_ctx *ctx, uint64_t first, uint64_t count);
 /* Page-locked host memory for the buffers above (plain malloc'ed memory works too, synchronously). */
 void *sage2gpu_host_alloc(uint64_t n_bytes);
 void sage2gpu_host_free(void *p);
+
+/* ---- Restart from a saved .reads file ----------------------------------------------------------------------------------
+ * replaces: ReadLoader::loadReadsFromFile (readLoader.cpp:289), which SAGE2 -m 2 / -m 3 calls.  The file is what
+ * ReadLoader::saveReadsInFile writes (readLoader.cpp:270-287, and sage2gpu_write_reads byte for byte): a line with the number of
+ * reads U, then U lines "FREQ	LEN	F	R
+".  Accepted is exactly that: FREQ a decimal in 0..65535, LEN in 1..1016 (the limit of
+ * this build) and greater than min_overlap, both without leading zeros; F and R of LEN upper-case ACGT characters, R the reverse
+ * complement of F, F <= R (the strand insertReadIntoList keeps, readLoader.cpp:195); the F records strictly increasing in
+ * Read::operator< order (line n + 1 is read id n); U lines.  Anything else -- a truncated file, lower case, N, '', extra lines,
+ * gzip -- fails with SAGE2GPU_ERR_FORMAT and nothing loaded; sage2gpu_last_error names the 1-based line and the rule.  Parsing and
+ * checks run on the device, in pieces of the file.  After success the context is as after sage2gpu_load_finish: unique_reads = U,
+ * good_reads = total_reads = sum of FREQ, total_bp = sum of FREQ * LEN, avg_len = total_bp / good_reads (0 when the sum is 0).
+ * Those equal a run from the input files unless a read occurred 65,536 times or more: its FREQ is the uint16_t count wrapped
+ * (readLoader.cpp:234), so the sums count it modulo 65,536. */
+int sage2gpu_load_saved_reads(sage2gpu_ctx *ctx, const char *path, int min_overlap);
+/* The same over several contexts (body = the file without its first line):
+ *   saved_reads_info        U (*n_reads) and the size of the body in bytes
+ *   saved_reads_slice       the lines whose first byte lies in [byte_begin, byte_end) of the body, parsed and checked on this
+ *                           context; *n_lines, *max_read_length = its longest read.  On SAGE2GPU_ERR_FORMAT *bad_line = the line
+ *                           counted from the slice's first line (its file line = 1 + the lines of the slices before + *bad_line)
+ *   [maximum over the contexts]
+ *   saved_reads_pack        the slice packed at the record stride of max_read_length (the longest read of ALL slices) as this
+ *                           context's unique run, as sage2gpu_organize_partition leaves it (world = 1: the reads themselves);
+ *                           *unique_local = its lines, *good_reads / *total_bp = its sums of FREQ and FREQ * LEN
+ *   [world > 1: sage2gpu_reads_gather_layout, the all-gather, sage2gpu_reads_gather_finish]
+ *   saved_reads_finish      the sums over the contexts: checks the count against U and the order of the complete reads (pairs
+ *                           that straddle two slices too) and sets the counters; on SAGE2GPU_ERR_FORMAT *bad_line = the file line.
+ * sage2gpu_load_saved_reads = info + slice(0, body) + pack(0, 1) + finish. */
+int sage2gpu_saved_reads_info(sage2gpu_ctx *ctx, const char *path, uint64_t *n_reads, uint64_t *body_bytes);
+int sage2gpu_saved_reads_slice(sage2gpu_ctx *ctx, const char *path, int min_overlap, uint64_t byte_begin, uint64_t byte_end, uint64_t *n_lines,
+                               int *max_read_length, uint64_t *bad_line);
+int sage2gpu_saved_reads_pack(sage2gpu_ctx *ctx, int rank, int world, int max_read_length, uint64_t *unique_local, uint64_t *good_reads,
+                              uint64_t *total_bp);
+int sage2gpu_saved_reads_finish(sage2gpu_ctx *ctx, uint64_t n_reads, uint64_t good_reads, uint64_t total_bp, uint64_t *bad_line);
 
 /* replaces: HashTable::hashPrefixesAndSuffix (hashTable.cpp:70-128) */
 int sage2gpu_build_hash_table(sage2gpu_ctx *ctx);

@@ -19,7 +19,12 @@ LIB_PATH = os.path.join(HERE, "libsage2gpu.so")
 
 
 class Sage2GpuError(RuntimeError):
-    pass
+    """`code` = the library's return code (include/sage2gpu.h: 5 = SAGE2GPU_ERR_FORMAT), `bad_line` = the line a format error names."""
+    code = 0
+    bad_line = 0
+
+
+ERR_FORMAT = 5
 
 
 class Counters(C.Structure):
@@ -57,7 +62,9 @@ EXPORTS = ["sage2gpu_create", "sage2gpu_destroy", "sage2gpu_last_error", "sage2g
            "sage2gpu_table_shard_info", "sage2gpu_table_gather_layout", "sage2gpu_table_gather_finish",
            "sage2gpu_pack_slice", "sage2gpu_raw_gather_layout", "sage2gpu_raw_gather_finish", "sage2gpu_organize_partition",
            "sage2gpu_synth_reads", "sage2gpu_build_hash_table_part", "sage2gpu_load_finish_packed", "sage2gpu_peer_copy",
-           "sage2gpu_phase_a_import", "sage2gpu_load_max_length", "sage2gpu_load_finish_slice", "sage2gpu_table_bytes"]
+           "sage2gpu_phase_a_import", "sage2gpu_load_max_length", "sage2gpu_load_finish_slice", "sage2gpu_table_bytes",
+           "sage2gpu_load_saved_reads", "sage2gpu_saved_reads_info", "sage2gpu_saved_reads_slice", "sage2gpu_saved_reads_pack",
+           "sage2gpu_saved_reads_finish"]
 
 _lib = None
 
@@ -94,6 +101,11 @@ def load_library():
         lib.sage2gpu_load_max_length.argtypes = [vp, C.POINTER(C.c_int)]
         lib.sage2gpu_load_finish_slice.argtypes = [vp, C.c_int, u64p, u64p, u64p, u64p]
         lib.sage2gpu_table_bytes.argtypes = [vp, C.c_int, u64p, u64p, u64p, u64p, u64p]
+        lib.sage2gpu_load_saved_reads.argtypes = [vp, C.c_char_p, C.c_int]
+        lib.sage2gpu_saved_reads_info.argtypes = [vp, C.c_char_p, u64p, u64p]
+        lib.sage2gpu_saved_reads_slice.argtypes = [vp, C.c_char_p, C.c_int, C.c_uint64, C.c_uint64, u64p, C.POINTER(C.c_int), u64p]
+        lib.sage2gpu_saved_reads_pack.argtypes = [vp, C.c_int, C.c_int, C.c_int, u64p, u64p, u64p]
+        lib.sage2gpu_saved_reads_finish.argtypes = [vp, C.c_uint64, C.c_uint64, C.c_uint64, u64p]
         lib.sage2gpu_host_alloc.argtypes = [C.c_uint64]
         lib.sage2gpu_host_alloc.restype = vp
         lib.sage2gpu_host_free.argtypes = [vp]
@@ -179,10 +191,12 @@ class Sage2Gpu:
         except Exception:
             pass
 
-    def _check(self, rc: int, what: str):
+    def _check(self, rc: int, what: str, bad_line: int = 0):
         if rc != 0:
             msg = self._lib.sage2gpu_last_error(self._h)
-            raise Sage2GpuError(f"{what} failed ({rc}): {msg.decode() if msg else ''}")
+            err = Sage2GpuError(f"{what} failed ({rc}): {msg.decode() if msg else ''}")
+            err.code, err.bad_line = rc, int(bad_line)
+            raise err
 
     # ---- steps --------------------------------------------------------------------------------
     def load_reads(self, bases: np.ndarray, offsets: np.ndarray, min_overlap: int):
@@ -219,6 +233,38 @@ class Sage2Gpu:
         offsets = np.ascontiguousarray(offsets, dtype=np.int64)
         self._keep = (bases, offsets)
         self._check(self._lib.sage2gpu_load_append(self._h, bases.ctypes.data, offsets.ctypes.data, len(offsets) - 1), "load_append")
+
+    # ---- restart from a saved .reads file (ReadLoader::loadReadsFromFile, readLoader.cpp:289) ---------------------------
+    def load_saved_reads(self, path: str, min_overlap: int):
+        """The reads of a saved .reads file (what write_reads / the reference's saveReadsInFile write), parsed and checked on the
+        device.  A file that breaks the grammar raises Sage2GpuError with code ERR_FORMAT; the message names the line."""
+        self._check(self._lib.sage2gpu_load_saved_reads(self._h, path.encode(), int(min_overlap)), "load_saved_reads")
+
+    def saved_reads_info(self, path: str) -> tuple:
+        """(U of the first line, bytes of the body)."""
+        u, b = C.c_uint64(), C.c_uint64()
+        self._check(self._lib.sage2gpu_saved_reads_info(self._h, path.encode(), C.byref(u), C.byref(b)), "saved_reads_info")
+        return int(u.value), int(b.value)
+
+    def saved_reads_slice(self, path: str, min_overlap: int, byte_begin: int, byte_end: int) -> dict:
+        """The lines whose first byte lies in [byte_begin, byte_end) of the body; on a format error `bad_line` counts from the
+        slice's first line."""
+        n, m, bad = C.c_uint64(), C.c_int(), C.c_uint64()
+        rc = self._lib.sage2gpu_saved_reads_slice(self._h, path.encode(), int(min_overlap), int(byte_begin), int(byte_end), C.byref(n),
+                                                  C.byref(m), C.byref(bad))
+        self._check(rc, "saved_reads_slice", bad.value)
+        return {"n_lines": int(n.value), "max_read_length": int(m.value)}
+
+    def saved_reads_pack(self, rank: int, world: int, max_read_length: int) -> dict:
+        u, g, b = C.c_uint64(), C.c_uint64(), C.c_uint64()
+        self._check(self._lib.sage2gpu_saved_reads_pack(self._h, int(rank), int(world), int(max_read_length), C.byref(u), C.byref(g), C.byref(b)),
+                    "saved_reads_pack")
+        return {"unique_local": int(u.value), "good_reads": int(g.value), "total_bp": int(b.value)}
+
+    def saved_reads_finish(self, n_reads: int, good_reads: int, total_bp: int):
+        bad = C.c_uint64()
+        rc = self._lib.sage2gpu_saved_reads_finish(self._h, int(n_reads), int(good_reads), int(total_bp), C.byref(bad))
+        self._check(rc, "saved_reads_finish", bad.value)
 
     def load_max_length(self) -> int:
         """Longest read appended since load_begin (nothing is packed)."""
@@ -518,6 +564,14 @@ class ReadLoader:
 
     def saveReadsInFile(self, path: str):
         self.gpu.write_reads(path)
+
+    def loadReadsFromFile(self, path: str):
+        """readLoader.cpp:289: the reads of a saved .reads file (SAGE2 -m 2 / -m 3) instead of readDatasetInBytes + organizeReads.
+        numberOfReads is the sum of the file's frequencies (each a uint16_t count, wrapped at 65,536 copies)."""
+        self.gpu.load_saved_reads(path, self.minOverlap)
+        c = self.gpu.counters()
+        self.numberOfReads, self.numberOfUniqueReads, self.totalBP = c["good_reads"], c["unique_reads"], c["total_bp"]
+        self.averageReadLength = c["avg_len"]
 
     def getIdOfRead(self, reads):
         """readLoader.cpp:319-353 for a batch: signed ids (0 = absent; bad reads, which step 6 never looks up, give 0)."""

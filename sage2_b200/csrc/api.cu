@@ -45,6 +45,12 @@ int guarded(sage2gpu_ctx *ctx, Fn fn)
         }
         ctx->c.last_error.clear();
         return SAGE2GPU_OK;
+    } catch (const sg::FormatError &e) {
+        ctx->c.last_error = e.what();
+        return SAGE2GPU_ERR_FORMAT;
+    } catch (const sg::IoError &e) {
+        ctx->c.last_error = e.what();
+        return SAGE2GPU_ERR_IO;
     } catch (const sg::CudaError &e) {
         ctx->c.last_error = e.what();
         cudaGetLastError();
@@ -147,7 +153,7 @@ void sage2gpu_destroy(sage2gpu_ctx *ctx)
     cudaStreamSynchronize(st);
     {
         sg::Context &c = ctx->c;
-        c.d_bases.release(); c.d_offsets.release(); c.up_d_bases.release(); c.up_d_offsets.release(); c.raw.release(); c.F.release(); c.RC.release(); c.len.release(); c.freq.release();
+        c.d_bases.release(); c.d_offsets.release(); c.up_d_bases.release(); c.up_d_offsets.release(); c.up_d_freq.release(); c.raw.release(); c.F.release(); c.RC.release(); c.len.release(); c.freq.release();
         c.slots.release(); c.entries.release(); c.extR.release(); c.extL.release(); c.flag5.release();
         c.cont_max.release(); c.explored.release(); c.edges.release();
         sg::stage_mailbox_destroy(c);
@@ -462,6 +468,94 @@ int sage2gpu_load_finish(sage2gpu_ctx *ctx)
             c.tm.sort_reads = t.stop();
         }
     });
+}
+
+// ---- a saved .reads file (ReadLoader::loadReadsFromFile, readLoader.cpp:289): parse.cu, reads.cu ----------------------------
+int sage2gpu_saved_reads_info(sage2gpu_ctx *ctx, const char *path, uint64_t *n_reads, uint64_t *body_bytes)
+{
+    return guarded(ctx, [&](sg::Context &c) {
+        SG_CHECK(path != nullptr, "null path");
+        sg::u64 u = 0, off = 0, body = 0;
+        sg::saved_reads_header(path, u, off, body);
+        if (n_reads) *n_reads = u;
+        if (body_bytes) *body_bytes = body;
+    });
+}
+
+int sage2gpu_saved_reads_slice(sage2gpu_ctx *ctx, const char *path, int min_overlap, uint64_t byte_begin, uint64_t byte_end, uint64_t *n_lines,
+                               int *max_read_length, uint64_t *bad_line)
+{
+    return guarded(ctx, [&](sg::Context &c) {
+        SG_CHECK(path != nullptr, "null path");
+        SG_CHECK(min_overlap >= 1 && min_overlap < 65535, "min_overlap out of range");
+        if (bad_line) *bad_line = 0;
+        c.min_overlap = min_overlap;
+        c.tm = sg::Timers();
+        c.up_open = false;
+        c.have_reads = c.have_table = c.have_graph = false;
+        StageTimer t(c.stream);
+        sg::u64 n = 0;
+        int ml = 0;
+        try {
+            sg::stage_parse_saved_reads(c, path, byte_begin, byte_end, n, ml);
+        } catch (const sg::FormatError &e) {
+            if (bad_line) *bad_line = e.line;
+            c.up_reads = c.up_bases = 0;
+            c.up_d_bases.release(); c.up_d_offsets.release(); c.up_d_freq.release();
+            throw;
+        }
+        c.tm.ingest = t.stop();
+        if (n_lines) *n_lines = n;
+        if (max_read_length) *max_read_length = ml;
+    });
+}
+
+int sage2gpu_saved_reads_pack(sage2gpu_ctx *ctx, int rank, int world, int max_read_length, uint64_t *unique_local, uint64_t *good_reads,
+                              uint64_t *total_bp)
+{
+    return guarded(ctx, [&](sg::Context &c) {
+        const sg::u64 good = c.sr_good, bp = c.sr_bp;
+        StageTimer t(c.stream);
+        sg::stage_pack_saved_reads(c, rank, world, max_read_length);
+        c.tm.sort_reads = t.stop();
+        if (c.opt_low_memory) { SG_CUDA(cudaStreamSynchronize(c.stream)); c.arena.destroy(); }
+        if (unique_local) *unique_local = c.rp_local;
+        if (good_reads) *good_reads = good;
+        if (total_bp) *total_bp = bp;
+    });
+}
+
+int sage2gpu_saved_reads_finish(sage2gpu_ctx *ctx, uint64_t n_reads, uint64_t good_reads, uint64_t total_bp, uint64_t *bad_line)
+{
+    return guarded(ctx, [&](sg::Context &c) {
+        if (bad_line) *bad_line = 0;
+        StageTimer t(c.stream);
+        try {
+            sg::stage_check_saved_reads(c, n_reads, good_reads, total_bp);
+        } catch (const sg::FormatError &e) {
+            if (bad_line) *bad_line = e.line;
+            throw;
+        }
+        c.tm.sort_reads += t.stop();
+    });
+}
+
+int sage2gpu_load_saved_reads(sage2gpu_ctx *ctx, const char *path, int min_overlap)
+{
+    // the one-slice case of the calls above; a line of the slice is line + 1 of the file (line 1 is the number of reads)
+    uint64_t U = 0, body = 0, n = 0, good = 0, bp = 0, bad = 0;
+    int ml = 0;
+    int rc = sage2gpu_saved_reads_info(ctx, path, &U, &body);
+    if (rc == 0) {
+        rc = sage2gpu_saved_reads_slice(ctx, path, min_overlap, 0, body, &n, &ml, &bad);
+        if (rc == SAGE2GPU_ERR_FORMAT) {
+            const std::string m = ctx->c.last_error;
+            ctx->c.last_error = "line " + std::to_string(bad + 1) + m.substr(m.find(':'));
+        }
+    }
+    if (rc == 0) rc = sage2gpu_saved_reads_pack(ctx, 0, 1, ml, nullptr, &good, &bp);
+    if (rc == 0) rc = sage2gpu_saved_reads_finish(ctx, U, good, bp, nullptr);
+    return rc;
 }
 
 void *sage2gpu_host_alloc(uint64_t n_bytes)

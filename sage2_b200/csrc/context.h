@@ -45,7 +45,7 @@ struct Context {
     Context()
     {
         // everything a context keeps between stages is persistent; stage-local temporaries use `arena`
-        d_bases.persistent = d_offsets.persistent = up_d_bases.persistent = up_d_offsets.persistent = true;
+        d_bases.persistent = d_offsets.persistent = up_d_bases.persistent = up_d_offsets.persistent = up_d_freq.persistent = true;
         raw.persistent = F.persistent = RC.persistent = len.persistent = freq.persistent = true;
         F_loc.persistent = len_loc.persistent = freq_loc.persistent = raw_slice.persistent = entries_loc.persistent = true;
         slots.persistent = entries.persistent = true;
@@ -75,6 +75,9 @@ struct Context {
     DevBuf<int64_t> up_d_offsets;   // [up_reads + 1], absolute
     u64 up_reads = 0, up_bases = 0;
     bool up_open = false;
+    // a saved .reads file (sage2gpu_saved_reads_*): the frequency column of the parsed lines, beside up_d_bases / up_d_offsets
+    DevBuf<uint16_t> up_d_freq;
+    u64 sr_good = 0, sr_bp = 0;     // sums of FREQ and FREQ * LEN over the lines this context parsed
     cudaEvent_t up_event = nullptr;
 
     DevBuf<u64> raw;            // [n_input*SW] packed canonical records in input order (step 1, before the sort)
@@ -134,6 +137,19 @@ struct Context {
     DevBuf<u32> an_entries;
 };
 
+// A file that breaks the grammar of a saved .reads file: `line` = the 1-based line (of the file, or of a context's slice)
+struct FormatError : public std::runtime_error {
+    u64 line;
+    std::string rule;
+    FormatError(u64 l, const std::string &r, bool in_slice = false)
+        : std::runtime_error("line " + std::to_string(l) + (in_slice ? " of this context's slice: " : ": ") + r), line(l), rule(r) {}
+};
+
+// A file that cannot be opened or read
+struct IoError : public std::runtime_error {
+    explicit IoError(const std::string &m) : std::runtime_error(m) {}
+};
+
 // stages (each throws sg::CudaError)
 void stage_ingest_ascii(Context &c, const uint8_t *bases, const int64_t *offsets, int64_t n_reads, bool device_resident, int forced_max_len = 0);
 void stage_raw_gather_layout(Context &c, int rank, int world, const u64 *counts, void **raw, u64 *first, u64 *total);
@@ -145,6 +161,15 @@ int stage_uploaded_max_len(Context &c);     // longest read of the streamed uplo
 // parse.cu: record splitting of raw FASTA/FASTQ text on the device; false = irregular layout, nothing appended
 bool stage_parse_text_chunk(Context &c, const uint8_t *text, u64 n_bytes, bool final, int &marker, u64 max_records, u64 &consumed, u64 &n_records);
 void stage_remove_uploaded(Context &c, u64 first, u64 count);
+// parse.cu: a saved .reads file (ReadLoader::loadReadsFromFile, readLoader.cpp:289).  Header: the declared number of reads and the
+// byte offset of the body.  Slice: the lines whose first byte lies in [begin, end) of the body, parsed and checked on the device into
+// the upload buffers + the frequency column; throws FormatError with the line counted from the slice's first line.
+void saved_reads_header(const char *path, u64 &n_reads, u64 &body_offset, u64 &body_bytes);
+void stage_parse_saved_reads(Context &c, const char *path, u64 begin, u64 end, u64 &n_lines, int &max_len);
+// reads.cu: the parsed lines packed at the stride of max_len (the longest read of all slices) and written as this context's unique run
+// (world > 1: F_loc / len_loc / freq_loc, as stage_organize_reads leaves them), then the checks over the complete reads
+void stage_pack_saved_reads(Context &c, int rank, int world, int max_len);
+void stage_check_saved_reads(Context &c, u64 n_reads, u64 good_reads, u64 total_bp);
 void stage_organize_reads(Context &c, int rank = 0, int world = 1);   // world > 1: this rank's key range of the reads only
 void stage_reads_gather_layout(Context &c, const u64 *counts, void **F, void **len, void **freq, u64 *first, u64 *total);
 void stage_reads_gather_finish(Context &c);

@@ -808,4 +808,90 @@ void stage_raw_gather_finish(Context &c, u64 total_reads, u64 good_reads, u64 to
     if (c.opt_low_memory) { SG_CUDA(cudaStreamSynchronize(c.stream)); c.raw_slice.release(); }
 }
 
+// ---- a saved .reads file (parse.cu): its lines are the unique reads already, in id order -------------------------------
+// Packed by K1 at the stride of the longest read of all slices, then written by the F / RC writer of organizeReads with the
+// identity as the sorted order and every read flagged new; the frequencies are the file's.
+void stage_pack_saved_reads(Context &c, int rank, int world, int max_len)
+{
+    cudaStream_t st = c.stream;
+    ArenaScope arena_scope(c.arena, st);
+    SG_CHECK(world >= 1 && world <= kMaxWorld && rank >= 0 && rank < world, "bad rank / world");
+    SG_CHECK(world == 1 || max_len >= 1, "the longest read of the whole read set must be given");
+    const u64 n = c.up_reads;
+    // the parse already applied isGoodRead's rules (longer than k, ACGT only, at most 1016 bases) and canonical orientation,
+    // so K1 drops nothing and keeps F as it is
+    stage_ingest_ascii(c, c.up_d_bases.p, c.up_d_offsets.p, (int64_t)n, true, world == 1 && n == 0 ? 0 : max_len);
+    SG_CHECK(c.cnt.good_reads == n, "a parsed line was dropped by the pack");
+    c.up_d_bases.release(); c.up_d_offsets.release();
+    c.rp_rank = rank; c.rp_world = world; c.rp_local = n;
+    c.cnt.unique_reads = world == 1 ? n : 0;
+    c.SWS = storage_words(c.SW);
+    c.have_reads = false;
+    if (n == 0) {
+        if (world == 1) { c.F.release(); c.RC.release(); c.len.release(); c.freq.release(); }
+        c.up_d_freq.release();
+        return;
+    }
+    DevBuf<u64> &Fo = world > 1 ? c.F_loc : c.F;
+    DevBuf<uint16_t> &lo = world > 1 ? c.len_loc : c.len, &fo = world > 1 ? c.freq_loc : c.freq;
+    Fo.alloc((size_t)n * c.SWS, st);
+    lo.alloc(n, st);
+    fo.alloc(n, st);
+    DevBuf<u32> ids(n, st), ones(n, st), start(n, st);
+    iota_kernel<<<big_grid(n), 256, 0, st>>>(ids.p, n);
+    SG_LAUNCHED();
+    SG_CUDA(cudaMemsetAsync(ones.p, 0x01, n * sizeof(u32), st));
+    const unsigned uw_grid = big_grid(n * (c.SWS / 4), UW_THREADS);
+    if (world > 1) {
+        unique_write_kernel<false><<<uw_grid, UW_THREADS, 0, st>>>(c.raw_slice.p, ids.p, ones.p, ids.p, n, c.SW, c.SWS, Fo.p, nullptr, lo.p, start.p);
+    } else {
+        c.RC.alloc((size_t)n * c.SWS, st);
+        unique_write_kernel<true><<<uw_grid, UW_THREADS, 0, st>>>(c.raw_slice.p, ids.p, ones.p, ids.p, n, c.SW, c.SWS, Fo.p, c.RC.p, lo.p, start.p);
+    }
+    SG_LAUNCHED();
+    SG_CUDA(cudaMemcpyAsync(fo.p, c.up_d_freq.p, n * sizeof(uint16_t), cudaMemcpyDeviceToDevice, st));
+    SG_CUDA(cudaStreamSynchronize(st));
+    c.up_d_freq.release();
+    if (c.opt_low_memory) { c.raw_slice.release(); trim_default_pool(c.device, st); }
+}
+
+// first i >= 1 with record i-1 not below record i (Read::operator<: strictly increasing ids, no duplicates)
+__global__ void __launch_bounds__(256) order_check_kernel(const u64 *__restrict__ F, u64 U, int SW, int SWS, unsigned long long *first_bad)
+{
+    for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x + 1; i < U; i += (u64)gridDim.x * blockDim.x)
+        if (!rec_less(F + (i - 1) * SWS, F + i * SWS, SW)) atomicMin(first_bad, (unsigned long long)i);
+}
+
+// The complete reads (one context, or after reads_gather_finish): their order, their count against the first line, and the
+// counters of step 1 -- good reads = total reads = sum of FREQ, total_bp = sum of FREQ * LEN (readLoader.cpp:161-169)
+void stage_check_saved_reads(Context &c, u64 n_reads, u64 good_reads, u64 total_bp)
+{
+    cudaStream_t st = c.stream;
+    ArenaScope arena_scope(c.arena, st);
+    SG_CHECK(c.rp_world == 1 || c.have_reads, "sage2gpu_reads_gather_finish must run first");
+    const u64 U = c.rp_world == 1 ? c.rp_local : c.cnt.unique_reads;
+    c.have_reads = c.have_table = c.have_graph = false;
+    if (U > 1) {
+        DevBuf<unsigned long long> d_bad(1, st);
+        SG_CUDA(cudaMemsetAsync(d_bad.p, 0xFF, sizeof(unsigned long long), st));
+        order_check_kernel<<<big_grid(U), 256, 0, st>>>(c.F.p, U, c.SW, c.SWS, d_bad.p);
+        SG_LAUNCHED();
+        unsigned long long bad = 0;
+        SG_CUDA(cudaMemcpyAsync(&bad, d_bad.p, sizeof(bad), cudaMemcpyDeviceToHost, st));
+        SG_CUDA(cudaStreamSynchronize(st));
+        if (bad != ~0ull)
+            throw FormatError(bad + 2, "F is not greater than the F of the line before: the reads must be unique and in increasing order (Read::operator<)");
+    }
+    if (U < n_reads)
+        throw FormatError(U + 2, "the file ends after " + std::to_string(U) + " reads; its first line says " + std::to_string(n_reads));
+    if (U > n_reads) throw FormatError(n_reads + 2, "more reads than the " + std::to_string(n_reads) + " its first line says");
+    c.cnt.unique_reads = U;
+    c.cnt.total_reads = c.cnt.good_reads = good_reads;
+    c.cnt.total_bp = total_bp;
+    c.cnt.avg_len = good_reads ? total_bp / good_reads : 0;        // readLoader.cpp:161 integer division
+    c.h = hash_len_for(c.min_overlap);
+    c.cnt.hash_len = (u64)c.h;
+    c.have_reads = true;
+}
+
 }  // namespace sg

@@ -14,9 +14,14 @@
 // beside the later stages on every GPU, otherwise sharded by key hash with the window probes routed through peer-memory
 // mailboxes (low-memory mode); SAGE2GPU_TABLE_LAYOUT=replicated|sharded forces the choice, the log states it.
 //
-// Differences, all stated in the log: steps 1-3 are one device pass, so a restart at -m 2 / -m 3
-// recomputes from the input files instead of loading <prefix>.reads / <prefix>.hashTable (results are
-// identical); <prefix>.hashTable is not written (the reference's slot order is an artefact of its own
+// Restarts: -m 2 and -m 3 load <outputDir><inputPrefix>.reads (ReadLoader::loadReadsFromFile, readLoader.cpp:289) -- parsed
+// and checked on the device, spread over the contexts with --devices -- and do not open the -f / -l inputs in steps 1-3 (the
+// flags stay required, as in the reference's checkRequired).  When that file does not exist, step 1 runs from the input files.
+// A file that is not exactly what saveReadsInFile writes stops the program with a FORMAT error naming the line.  <prefix>.reads is
+// written when it is not the loaded file, so that `-m 4 -i <prefix>` finds it.
+//
+// Differences, all stated in the log: -m 3 runs as -m 2, the table is rebuilt from the reads instead of loaded from
+// <prefix>.hashTable, and <prefix>.hashTable is not written (the reference's slot order is an artefact of its own
 // hash function and is read by nothing but its -m 3 restart).  There is no CPU fallback: without a
 // CUDA device the program stops with an error, like the reference's printError (utils.cpp:36-40).
 #include <fcntl.h>
@@ -87,7 +92,9 @@ void printListOfArgs()
                  "\t-o|--outputDir <dir>    output directory\n"
                  "\t-p|--prefix <name>      prefix of the output files [untitled]\n"
                  "\t-i|--inputPrefix <name> prefix of the files a restart reads [= prefix]\n"
-                 "\t-m|--minStep <1..7>     first step to run [1]\n"
+                 "\t-m|--minStep <1..7>     first step to run [1]; 2 and 3 load <outputDir><inputPrefix>.reads when it exists\n"
+                 "\t                        (checked on the GPU; -m 3 rebuilds the hash table); without it step 1 runs\n"
+                 "\t                        from the input files\n"
                  "\t-M|--maxStep <1..7>     last step to run [7]\n"
                  "\t-s|--saveAll            save the intermediate files of every step\n"
                  "\t-d|--debug\n"
@@ -659,9 +666,9 @@ void shardedSteps(MultiGpu &m, HostSync &hs, std::vector<void *> &box, int r, ui
     if (r == 0) { redo_max = redo_all; list_max = list; }
 }
 
-// steps 1 (after the upload spread over the contexts) to 3; the result is complete in every context.  Returns whether the
-// table was replicated (else every context holds one shard of it).
-bool runPartitioned(MultiGpu &m, int k)
+// step 1 after the upload spread over the contexts: every context packs its part, the parts are all-gathered and every
+// context organises its key range.  Returns the unique reads of every context's run.
+std::vector<uint64_t> organizePartitioned(MultiGpu &m)
 {
     const int G = m.G();
     // the contexts agree on the longest read: it fixes the record stride of every slice
@@ -673,7 +680,7 @@ bool runPartitioned(MultiGpu &m, int k)
     uint64_t N = 0, good_all = 0, bp_all = 0;
     for (int r = 0; r < G; ++r) { N += counts[r]; good_all += good[r]; bp_all += bp[r]; }
     const uint64_t SW = sw[0];
-    std::vector<void *> p(G, nullptr), p2(G, nullptr), p3(G, nullptr);
+    std::vector<void *> p(G, nullptr);
     m.each([&](int r) { m.check(r, sage2gpu_raw_gather_layout(m.ctx[r], r, G, counts.data(), &p[r], nullptr, nullptr)); });
     {
         std::vector<uint64_t> off(G, 0), bytes(G, 0);
@@ -686,6 +693,51 @@ bool runPartitioned(MultiGpu &m, int k)
         m.check(r, sage2gpu_raw_gather_finish(m.ctx[r], N, good_all, bp_all));
         m.check(r, sage2gpu_organize_partition(m.ctx[r], r, G, &uloc[r]));
     });
+    return uloc;
+}
+
+// FORMAT error of a saved .reads file (utils.cpp:36-40: log, exit); `msg` names the line and the rule
+[[noreturn]] void savedReadsError(const std::string &path, const std::string &msg) { printError("FORMAT", path + ", " + msg); }
+
+// step 1 of a restart over the contexts (ReadLoader::loadReadsFromFile): context r parses the lines that start in the r-th of G
+// equal byte ranges of the file's body, in its own thread; the contexts agree on the longest read and pack their lines as their
+// unique runs.  Returns the lines of every context; U = the number of reads the file declares, good / bp = the sums of the slices.
+std::vector<uint64_t> loadSavedPartitioned(MultiGpu &m, const std::string &path, int k, uint64_t &U, uint64_t &good, uint64_t &bp)
+{
+    const int G = m.G();
+    uint64_t body = 0;
+    if (const int rc = sage2gpu_saved_reads_info(m.ctx[0], path.c_str(), &U, &body)) {
+        if (rc == SAGE2GPU_ERR_FORMAT) savedReadsError(path, sage2gpu_last_error(m.ctx[0]));
+        printError("OPEN_FILE", sage2gpu_last_error(m.ctx[0]));
+    }
+    std::vector<uint64_t> lines(G, 0), bad(G, 0);
+    std::vector<int> ml(G, 0), rc(G, 0);
+    m.each([&](int r) {
+        rc[r] = sage2gpu_saved_reads_slice(m.ctx[r], path.c_str(), k, body * r / G, body * (r + 1) / G, &lines[r], &ml[r], &bad[r]);
+    });
+    uint64_t before = 1;        // line 1 holds the number of reads
+    for (int r = 0; r < G; ++r) {
+        if (rc[r] == SAGE2GPU_ERR_FORMAT) {       // the first broken line: the slices before this one were parsed completely
+            const std::string e = sage2gpu_last_error(m.ctx[r]);
+            savedReadsError(path, "line " + std::to_string(before + bad[r]) + e.substr(e.find(": ")));
+        }
+        if (rc[r] == SAGE2GPU_ERR_IO) printError("OPEN_FILE", sage2gpu_last_error(m.ctx[r]));
+        m.check(r, rc[r]);
+        before += lines[r];
+    }
+    const int max_len = *std::max_element(ml.begin(), ml.end());
+    std::vector<uint64_t> uloc(G, 0), g(G, 0), b(G, 0);
+    m.each([&](int r) { m.check(r, sage2gpu_saved_reads_pack(m.ctx[r], r, G, std::max(1, max_len), &uloc[r], &g[r], &b[r])); });
+    good = bp = 0;
+    for (int r = 0; r < G; ++r) { good += g[r]; bp += b[r]; }
+    return uloc;
+}
+
+// every context's unique run all-gathered: the complete reads in every context
+void gatherReads(MultiGpu &m, const std::vector<uint64_t> &uloc)
+{
+    const int G = m.G();
+    std::vector<void *> p(G, nullptr), p2(G, nullptr), p3(G, nullptr);
     std::vector<uint64_t> stride(G, 0);
     m.each([&](int r) { m.check(r, sage2gpu_reads_gather_layout(m.ctx[r], uloc.data(), &p[r], &p2[r], &p3[r], nullptr, nullptr, &stride[r])); });
     {
@@ -697,7 +749,14 @@ bool runPartitioned(MultiGpu &m, int k)
         m.gather(p3, off2, bytes2);
     }
     m.each([&](int r) { m.check(r, sage2gpu_reads_gather_finish(m.ctx[r])); });
+}
 
+// steps 2 and 3 with the complete reads in every context; the result is complete in every context.  Returns whether the
+// table was replicated (else every context holds one shard of it).
+bool graphPartitioned(MultiGpu &m)
+{
+    const int G = m.G();
+    std::vector<void *> p(G, nullptr), p2(G, nullptr);
     // the layout: the table replicated on every context (faster) when it fits beside the later stages on every GPU, else sharded
     sage2gpu_counters c0;
     sage2gpu_get_counters(m.ctx[0], &c0);
@@ -762,6 +821,20 @@ bool runPartitioned(MultiGpu &m, int k)
     return true;
 }
 
+// -m 2 / -m 3: the file a restart loads, <outputDir><inputPrefix>.reads (ReadLoader::loadReadsFromFile, readLoader.cpp:289)
+std::string savedReadsPath(const Options &o) { return o.outputDir + o.inputPrefix + ".reads"; }
+
+// the restart loads that file when it exists; otherwise step 1 runs from the input files
+bool restartFromSavedReads(const Options &o) { return o.minStep >= 2 && o.minStep <= 3 && access(savedReadsPath(o).c_str(), F_OK) == 0; }
+
+// <prefix>.reads of a restart: written (from the device, byte-identical to the loaded file) unless it IS the loaded file
+bool writeReadsAfterRestart(const Options &o, const std::string &base)
+{
+    if (base + ".reads" != savedReadsPath(o)) return true;
+    logStream << "NOTE: " << base << ".reads is the file this restart loaded: not rewritten.\n";
+    return false;
+}
+
 // --devices with more than one entry: steps 1-3 partitioned over the listed GPUs, the same files and log lines out
 int runOnSeveralDevices(const Options &o, const std::string &base)
 {
@@ -773,9 +846,18 @@ int runOnSeveralDevices(const Options &o, const std::string &base)
         m.device.push_back(d);
     }
     logStream << "Devices: " << m.G() << " contexts (one per listed GPU), the input spread over them, every stage partitioned, peer copies between the stages.\n";
-    banner("STEP 1", "                                          organizing reads");
+    const bool restart = restartFromSavedReads(o);
     auto t0 = std::chrono::steady_clock::now();
-    {
+    std::vector<uint64_t> uloc;
+    uint64_t declared = 0, good = 0, bp = 0;
+    if (restart) {
+        banner("STEP 1", "                                     loading reads from file");
+        uloc = loadSavedPartitioned(m, savedReadsPath(o), o.minOverlap, declared, good, bp);
+        logStream << "\tLines parsed per context:";
+        for (uint64_t n : uloc) logStream << " " << n;
+        logStream << "\n";
+    } else {
+        banner("STEP 1", "                                          organizing reads");
         Uploader up(m.ctx, o.minOverlap);
         if (!o.listInput.empty()) loadFromList(up, o.listInput);
         else readDataset(up, o.fileInput, "");
@@ -787,7 +869,19 @@ int runOnSeveralDevices(const Options &o, const std::string &base)
     }
     banner("STEPS 2-3", "                             building hash table and overlap graph");
     auto t1 = std::chrono::steady_clock::now();
-    const bool replicated = runPartitioned(m, o.minOverlap);
+    if (!restart) uloc = organizePartitioned(m);
+    gatherReads(m, uloc);
+    if (restart) {      // the count and the order of the complete reads (pairs across two slices too), then the counters
+        std::vector<uint64_t> bad(m.G(), 0);
+        std::vector<int> rc(m.G(), 0);
+        m.each([&](int r) { rc[r] = sage2gpu_saved_reads_finish(m.ctx[r], declared, good, bp, &bad[r]); });
+        for (int r = 0; r < m.G(); ++r) {
+            if (rc[r] == SAGE2GPU_ERR_FORMAT) savedReadsError(savedReadsPath(o), sage2gpu_last_error(m.ctx[r]));
+            m.check(r, rc[r]);
+        }
+        logStream << "Function loadReadsFromFile() on " << m.G() << " devices in " << seconds_since(t0) << " sec.\n";
+    }
+    const bool replicated = graphPartitioned(m);
     logStream << "Functions organizeReads() .. sortEconomyGraph() on " << m.G() << " devices in " << seconds_since(t1) << " sec.\n";
     sage2gpu_counters cnt;
     sage2gpu_get_counters(m.ctx[0], &cnt);
@@ -813,7 +907,8 @@ int runOnSeveralDevices(const Options &o, const std::string &base)
     logStream << "\tTotal edges inserted: " << cnt.edges_inserted_c << "\n";
     logStream << "\tTotal transitive edges removed: " << cnt.transitive_removed << "\n";
     logStream << "\tEdges in the overlap graph: " << cnt.n_edges << "\n";
-    if (sage2gpu_write_reads(m.ctx[0], (base + ".reads").c_str()) != 0) printError("OPEN_FILE", sage2gpu_last_error(m.ctx[0]));
+    if ((!restart || writeReadsAfterRestart(o, base)) && sage2gpu_write_reads(m.ctx[0], (base + ".reads").c_str()) != 0)
+        printError("OPEN_FILE", sage2gpu_last_error(m.ctx[0]));
     // the graph from the LAST context: every context must hold the complete result
     if (sage2gpu_write_graph3(m.ctx[m.G() - 1], (base + ".graph3").c_str()) != 0) printError("OPEN_FILE", sage2gpu_last_error(m.ctx[m.G() - 1]));
     logStream.flush();
@@ -872,8 +967,15 @@ int main(int argc, char **argv)
     logStream << "\t         END STEP: " << o.maxStep << "\n";
     logStream << "\t   SAVE ALL FILES: " << (o.saveAll ? "TRUE" : "FALSE") << "\n";
     logStream << "***********************************************************************************************************\n\n";
-    if (o.minStep > 1)
-        logStream << "NOTE: steps 1-3 are one device pass; -m " << o.minStep << " recomputes them from the input files (same result).\n";
+    const bool restart = restartFromSavedReads(o);
+    if (restart) {
+        logStream << "Restart at step " << o.minStep << ": the reads are loaded from " << savedReadsPath(o)
+                  << " (ReadLoader::loadReadsFromFile); the input files are not read.\n";
+        if (o.minStep == 3)
+            logStream << "NOTE: -m 3 runs as -m 2: the hash table is rebuilt from the reads (" << o.inputPrefix << ".hashTable is not read).\n";
+    } else if (o.minStep > 1) {
+        logStream << "NOTE: " << savedReadsPath(o) << " does not exist: -m " << o.minStep << " runs step 1 from the input files (same result).\n";
+    }
     logStream.flush();
 
     if (o.devices.size() > 1) return runOnSeveralDevices(o, base);
@@ -884,9 +986,17 @@ int main(int argc, char **argv)
     sage2gpu_counters cnt;
 
     // ---- step 1 -------------------------------------------------------------------------------------
-    banner("STEP 1", "                                          organizing reads");
     auto t0 = std::chrono::steady_clock::now();
-    {
+    if (restart) {
+        banner("STEP 1", "                                     loading reads from file");
+        const std::string path = savedReadsPath(o);
+        if (const int rc = sage2gpu_load_saved_reads(ctx, path.c_str(), o.minOverlap)) {
+            if (rc == SAGE2GPU_ERR_FORMAT) savedReadsError(path, sage2gpu_last_error(ctx));
+            printError(rc == SAGE2GPU_ERR_IO ? "OPEN_FILE" : "CUDA", sage2gpu_last_error(ctx));
+        }
+        logStream << "Function loadReadsFromFile() in " << seconds_since(t0) << " sec.\n";
+    } else {
+        banner("STEP 1", "                                          organizing reads");
         Uploader up({ ctx }, o.minOverlap);
         if (!o.listInput.empty()) loadFromList(up, o.listInput);
         else readDataset(up, o.fileInput, "");
@@ -902,7 +1012,8 @@ int main(int argc, char **argv)
     logStream << "\t" << std::setw(21) << "Average read length: " << cnt.avg_len << "\n";
     logStream << "\tNumber of unique reads: " << cnt.unique_reads << "\n";
     logStream.flush();
-    const bool saveReads = o.maxStep <= 3 || o.saveAll || o.maxStep > 3;      // steps 4-7 continue from the files
+    const bool saveReads = (o.maxStep <= 3 || o.saveAll || o.maxStep > 3) &&      // steps 4-7 continue from the files
+                           (!restart || writeReadsAfterRestart(o, base));
     if (saveReads) {
         auto t = std::chrono::steady_clock::now();
         if (sage2gpu_write_reads(ctx, (base + ".reads").c_str()) != 0) printError("OPEN_FILE", sage2gpu_last_error(ctx));
