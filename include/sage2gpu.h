@@ -110,7 +110,8 @@ void sage2gpu_host_free(void *p);
 ".  Accepted is exactly that: FREQ a decimal in 0..65535, LEN in 1..1016 (the limit of
  * this build) and greater than min_overlap, both without leading zeros; F and R of LEN upper-case ACGT characters, R the reverse
  * complement of F, F <= R (the strand insertReadIntoList keeps, readLoader.cpp:195); the F records strictly increasing in
- * Read::operator< order (line n + 1 is read id n); U lines.  Anything else -- a truncated file, lower case, N, '', extra lines,
+ * Read::operator< order (line n + 1 is read id n); U lines.  Anything else -- a truncated file, lower case, N, '
+', extra lines,
  * gzip -- fails with SAGE2GPU_ERR_FORMAT and nothing loaded; sage2gpu_last_error names the 1-based line and the rule.  Parsing and
  * checks run on the device, in pieces of the file.  After success the context is as after sage2gpu_load_finish: unique_reads = U,
  * good_reads = total_reads = sum of FREQ, total_bp = sum of FREQ * LEN, avg_len = total_bp / good_reads (0 when the sum is 0).
@@ -311,8 +312,8 @@ int sage2gpu_measure_gather(sage2gpu_ctx *ctx, uint64_t footprint_bytes, int gra
 int sage2gpu_digest(sage2gpu_ctx *ctx, uint64_t *reads_digest, uint64_t *edges_digest);
 
 /* Run-time options.  "read_order": schedule of the phase-A search (results do not depend on it): 0 = id order,
- * 1 = min-hash order (reads that share k-mers are searched together, so slot sectors and partner records hit L2),
- * -1 = the default.  "low_memory": 1 = the large buffers are released (and returned to the driver) as soon as no later stage of the step
+ * 1 = minimizer order (reads that share bases are searched together, so slot sectors and partner records hit L2),
+ * -1 = the default: minimizer order when the records and the slot index take 1 GiB or more, id order below.  "low_memory": 1 = the large buffers are released (and returned to the driver) as soon as no later stage of the step
  * needs them -- the packed input after organizeReads, the table before the edge sort; 2 = the workspace too, after every
  * call (for read sets near the capacity of the GPU).  Switched on when the reads are already organised (and gathered), it
  * releases at once what it would have released by then: the packed input, the context's packed slice and unique run, the

@@ -109,8 +109,8 @@ __device__ __forceinline__ u64 make_item(int jj, bool first, bool inl, u64 paylo
 // ------------------------------------------------------------------------------------------------
 // K4: phase A
 // ------------------------------------------------------------------------------------------------
-// ORDERED (experimental, off by default): the batch is processed in the order of the id list P.ids instead of id order
-// (a min-hash order that keeps overlapping reads together in time, DESIGN.md section 6); results do not depend on it.
+// ORDERED: the batch is processed in the order of the id list P.ids instead of id order (the reads the superstring scan
+// left, or the minimizer order that keeps overlapping reads together in time, DESIGN.md section 3); results do not depend on it.
 template <int SW, int MINB, bool ROUTED, bool ORDERED = false>
 __global__ void __launch_bounds__(SearchCfg<SW>::WARPS * 32, MINB)
 phase_a_kernel(SearchParams P, u64 *__restrict__ extR, u64 *__restrict__ extL, uint8_t *__restrict__ flag5,
@@ -539,46 +539,89 @@ static void launch_phase_a_ordered(Context &c, const SearchParams &P, unsigned l
                                                                                                                    c.cont_max.p, d_counters);
 }
 
-// ---- experimental read schedule (SAGE2GPU_READ_ORDER=minhash): min-hash of the window keys per read, ids sorted by it ----
-__global__ void __launch_bounds__(256) minhash_kernel(const u64 *__restrict__ F, int SW, int SWS, int h, u64 lo, u64 n,
-                                                      u64 *__restrict__ key, u32 *__restrict__ id)
+#define SG_DISPATCH_SW(SWV, CALL)                                                       \
+    switch (SWV) {                                                                      \
+        case 2: { constexpr int SWC = 2; CALL; } break;                                 \
+        case 3: { constexpr int SWC = 3; CALL; } break;                                 \
+        case 4: { constexpr int SWC = 4; CALL; } break;                                 \
+        case 5: { constexpr int SWC = 5; CALL; } break;                                 \
+        case 6: { constexpr int SWC = 6; CALL; } break;                                 \
+        case 8: { constexpr int SWC = 8; CALL; } break;                                 \
+        case 12: { constexpr int SWC = 12; CALL; } break;                               \
+        case 16: { constexpr int SWC = 16; CALL; } break;                               \
+        case 32: { constexpr int SWC = 32; CALL; } break;                               \
+        default: throw CudaError("unsupported record stride");                         \
+    }
+
+// ---- read schedule (read_order = 1): reads sorted by their minimizer, so that reads sharing bases are searched together ----
+// The key of a read is the least hash over its 32-base words (m = 32: one u64, cut out by a constant funnel shift); the
+// hash is one 64-bit multiply, top 32 bits.  Forward words only: canonical words (the smaller of a word and its reverse
+// complement) gave the same search time at cfg4 and cost 3.4 times as much to compute (DESIGN.md section 3).
+constexpr u64 kMinimizerMul = 0x9e3779b97f4a7c15ull;
+
+// One thread per read: a warp loads its 32 consecutive records with coalesced loads into shared memory (rows padded to
+// an odd stride), then every lane scans its own record.
+template <int SW>
+__global__ void __launch_bounds__((SearchCfg<SW>::SWS <= 16 ? 8 : 4) * 32)
+minimizer_kernel(const u64 *__restrict__ F, u64 lo, u64 n, u64 *__restrict__ key, u32 *__restrict__ id)
 {
-    __shared__ u64 sX[8][kMaxWords];
+    constexpr int SWS = SearchCfg<SW>::SWS, ROW = SWS + 1, WARPS = SWS <= 16 ? 8 : 4;
+    __shared__ u64 sX[WARPS][32 * ROW];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     u64 *X = sX[warp];
-    const u64 nwarps = (u64)gridDim.x * 8;
-    for (u64 s = (u64)blockIdx.x * 8 + warp; s < n; s += nwarps) {
-        const u64 i = lo + s;
+    const u64 ngroups = (n + 31) / 32, nwarps = (u64)gridDim.x * WARPS;
+    for (u64 g = (u64)blockIdx.x * WARPS + warp; g < ngroups; g += nwarps) {
+        const u64 s0 = g * 32;
+        const int nr = n - s0 < 32 ? (int)(n - s0) : 32;
+        const u64 *src = F + (lo + s0) * SWS;
         __syncwarp();
-        for (int w = lane; w < SW; w += 32) X[w] = F[i * SWS + w];
-        __syncwarp();
-        const int W = rec_len(X, SW) - h + 1;
-        u64 m = ~0ull;
-        for (int j = lane; j < W; j += 32) {
-            u64 v0, v1;
-            extract_key(X, SW, j, h, v0, v1);
-            const u64 hsh = hash_key(v0, v1);
-            m = hsh < m ? hsh : m;
-        }
 #pragma unroll
-        for (int o = 16; o > 0; o >>= 1) { const u64 y = __shfl_xor_sync(0xffffffffu, m, o); m = y < m ? y : m; }
-        if (lane == 0) { key[s] = m; id[s] = (u32)i; }
+        for (int t = 0; t < SWS; ++t) {
+            const int k = 32 * t + lane, r = k / SWS, w = k % SWS;
+            if (r < nr) X[r * ROW + w] = __ldg(&src[k]);
+        }
+        __syncwarp();
+        if (lane < nr) {
+            const u64 *x = X + lane * ROW;
+            const int last = (int)(x[SW - 1] & 0xFFFF) - 32;      // start of the last whole word of the read
+            u32 m = 0xFFFFFFFFu;
+#pragma unroll(SW <= 8 ? SW : 1)
+            for (int w = 0; w < SW; ++w) {
+                const u64 a = x[w], b = x[w + 1];                 // x[SW]: storage or row padding, masked off below
+#pragma unroll
+                for (int sh = 0; sh < 32; ++sh) {
+                    const u64 win = sh == 0 ? a : ((a << (2 * sh)) | (b >> (64 - 2 * sh)));
+                    const u32 hv = (u32)((win * kMinimizerMul) >> 32);
+                    m = (32 * w + sh <= last && hv < m) ? hv : m;
+                }
+            }
+            key[s0 + lane] = m;
+            id[s0 + lane] = (u32)(lo + s0 + lane);
+        }
     }
 }
 
-// ids of [lo, hi) in min-hash order -> out (device array owned by the caller's arena scope)
-static const u32 *minhash_order(Context &c, u64 lo, u64 hi, DevBuf<u64> &ka, DevBuf<u64> &kb, DevBuf<u32> &va, DevBuf<u32> &vb)
+// ids of [lo, hi) in minimizer order (device array owned by the caller's arena scope).  The sort is stable: reads with
+// one key keep id order.
+template <int SW>
+static void launch_minimizer(Context &c, u64 lo, u64 n, u64 *key, u32 *id)
+{
+    constexpr int WARPS = SearchCfg<SW>::SWS <= 16 ? 8 : 4;
+    u64 g = (n + 32 * WARPS - 1) / (32 * WARPS);
+    if (g > (u64)kSMs * 16) g = (u64)kSMs * 16;
+    minimizer_kernel<SW><<<(unsigned)g, WARPS * 32, 0, c.stream>>>(c.F.p, lo, n, key, id);
+}
+
+static const u32 *minimizer_order(Context &c, u64 lo, u64 hi, DevBuf<u64> &ka, DevBuf<u64> &kb, DevBuf<u32> &va, DevBuf<u32> &vb)
 {
     cudaStream_t st = c.stream;
     const u64 n = hi - lo;
     ka.alloc(n, st); kb.alloc(n, st); va.alloc(n, st); vb.alloc(n, st);
-    u64 g = (n + 7) / 8;
-    if (g > (u64)kSMs * 8) g = (u64)kSMs * 8;
-    minhash_kernel<<<(unsigned)g, 256, 0, st>>>(c.F.p, c.SW, c.SWS, c.h, lo, n, ka.p, va.p);
+    SG_DISPATCH_SW(c.SW, launch_minimizer<SWC>(c, lo, n, ka.p, va.p));
     SG_LAUNCHED();
     SortCols cols;
     cols.a[0] = ka.p; cols.a[1] = kb.p; cols.b[0] = cols.b[1] = nullptr; cols.v[0] = va.p; cols.v[1] = vb.p;
-    const int cur = radix_sort_bits(cols, 0, n, false, 32, 64, st);      // the top 32 bits cluster well enough
+    const int cur = radix_sort_bits(cols, 0, n, false, 0, 32, st);
     return cols.v[cur];
 }
 
@@ -603,19 +646,15 @@ static void launch_phase_c(Context &c, const SearchParams &P, const u32 *s_ids, 
     }
 }
 
-#define SG_DISPATCH_SW(SWV, CALL)                                                       \
-    switch (SWV) {                                                                      \
-        case 2: { constexpr int SWC = 2; CALL; } break;                                 \
-        case 3: { constexpr int SWC = 3; CALL; } break;                                 \
-        case 4: { constexpr int SWC = 4; CALL; } break;                                 \
-        case 5: { constexpr int SWC = 5; CALL; } break;                                 \
-        case 6: { constexpr int SWC = 6; CALL; } break;                                 \
-        case 8: { constexpr int SWC = 8; CALL; } break;                                 \
-        case 12: { constexpr int SWC = 12; CALL; } break;                               \
-        case 16: { constexpr int SWC = 16; CALL; } break;                               \
-        case 32: { constexpr int SWC = 32; CALL; } break;                               \
-        default: throw CudaError("unsupported record stride");                         \
-    }
+// Default schedule: the minimizer order pays once the records and the slot index the search reads at random are far
+// larger than L2 (cfg4, 4.9 GB: faster in that order; cfg2, 0.4 GB: slower, DESIGN.md section 3).
+constexpr u64 kReadOrderMinBytes = (u64)1 << 30;
+
+static bool read_order_pays(const Context &c)
+{
+    const u64 bytes = 2 * c.cnt.unique_reads * (u64)c.SWS * sizeof(u64) + c.cap * sizeof(u64);
+    return bytes >= kReadOrderMinBytes;
+}
 
 static SearchParams make_params(const Context &c)
 {
@@ -664,15 +703,17 @@ void stage_phase_a(Context &c, int rank, int world)
     cudaEvent_t e0, e1;
     SG_CUDA(cudaEventCreate(&e0)); SG_CUDA(cudaEventCreate(&e1));
     SG_CUDA(cudaEventRecord(e0, st));
-    static const bool env_minhash = [] { const char *e = getenv("SAGE2GPU_READ_ORDER"); return e && e[0] == 'm'; }();
+    // SAGE2GPU_READ_ORDER=id|minimizer ("minhash" is read as minimizer); unset: by footprint
+    static const int env_order = [] { const char *e = getenv("SAGE2GPU_READ_ORDER"); return !e ? -1 : (e[0] == 'm' ? 1 : 0); }();
     static const bool env_fast = [] { const char *e = getenv("SAGE2GPU_PA_FAST"); return !(e && e[0] == '0'); }();
-    const bool by_minhash = c.opt_read_order < 0 ? env_minhash : c.opt_read_order == 1;
+    const int order = c.opt_read_order >= 0 ? c.opt_read_order : env_order;
+    const bool by_minimizer = order >= 0 ? order == 1 : read_order_pays(c);
     const bool fast = (c.opt_fast_scan < 0 ? env_fast : c.opt_fast_scan == 1) && c.SW <= 8;
     DevBuf<u64> oka, okb;
     DevBuf<u32> ova, ovb, redo_ids;
     DevBuf<unsigned> redo_n;
-    if (P.hi > P.lo && by_minhash) {        // schedule that keeps overlapping reads together in time (DESIGN.md section 3)
-        P.ids = minhash_order(c, P.lo, P.hi, oka, okb, ova, ovb);
+    if (P.hi > P.lo && by_minimizer) {      // schedule that keeps overlapping reads together in time (DESIGN.md section 3)
+        P.ids = minimizer_order(c, P.lo, P.hi, oka, okb, ova, ovb);
         SG_CUDA(cudaEventRecord(e0, st));    // the ordering is not part of the search kernel's time (it is part of the stage's)
     }
     if (P.hi > P.lo && fast) {
@@ -684,7 +725,7 @@ void stage_phase_a(Context &c, int rank, int world)
         P2.ids = redo_ids.p; P2.n_dev = redo_n.p;
         SG_DISPATCH_SW(c.SW, launch_phase_a_ordered<SWC>(c, P2, d_counters.p));
         SG_LAUNCHED();
-    } else if (P.hi > P.lo && by_minhash) {
+    } else if (P.hi > P.lo && by_minimizer) {
         SG_DISPATCH_SW(c.SW, launch_phase_a_ordered<SWC>(c, P, d_counters.p));
         SG_LAUNCHED();
     } else if (P.hi > P.lo) {

@@ -103,11 +103,26 @@ __device__ __forceinline__ bool tail_equal(const u64 *S, int s, const u64 *Y, in
     return acc == 0;
 }
 
+// 32 bases of a shared-memory row starting at base s >= 0, without bounds checks: the row holds word (s >> 5) + 1
+// (superstring rows: two records and a word; partner rows: the storage stride and a word).  Bases past the data are
+// garbage that callers mask off.
+__device__ __forceinline__ u64 row_window32(const u64 *X, int s)
+{
+    const unsigned sh = (unsigned)(s & 31) * 2;
+    return funnel64(X[s >> 5], X[(s >> 5) + 1], sh >= 32, sh & 31);
+}
+
+// t_extract_key on a row (the key lies inside the read, so the word after it is within the row)
+__device__ __forceinline__ void row_extract_key(const u64 *X, int j, int h, u64 &v0, u64 &v1)
+{
+    if (h <= 32) { v0 = 0; v1 = row_window32(X, j) >> (64 - 2 * h); }
+    else { v0 = row_window32(X, j) >> (64 - 2 * (h - 32)); v1 = row_window32(X, j + h - 32); }
+}
+
 // 32 bases of record M starting at base s (may be negative: bases before the record read as 0)
-template <int SW>
 __device__ __forceinline__ u64 window_signed(const u64 *M, int s)
 {
-    if (s >= 0) return t_window32<SW>(M, s);
+    if (s >= 0) return row_window32(M, s);
     if (s <= -32) return 0ull;
     return M[0] >> (2 * (-s));
 }
@@ -131,6 +146,7 @@ phase_a_fast_kernel(SearchParams P, u64 *__restrict__ extR, u64 *__restrict__ ex
     u32 *ents = sEnt[warp];
     uint8_t *wins = sWin[warp];
     const u64 nwarps = (u64)gridDim.x * WARPS;
+    const unsigned lt_mask = (1u << lane) - 1u;
     unsigned calls = 0, probes = 0;
 
     const u64 n_batch = P.hi - P.lo;
@@ -162,36 +178,45 @@ phase_a_fast_kernel(SearchParams P, u64 *__restrict__ extR, u64 *__restrict__ ex
             u32 cnt = 0;
             if (j < W) {
                 u64 v0, v1;
-                t_extract_key<SW>(SR, j, P.h, v0, v1);
+                row_extract_key(SR, j, P.h, v0, v1);
                 if (!probe_sectors(P, hash_key(v0, v1), payload, cnt)) probe_window<SW>(P, v0, v1, false, payload, cnt);
                 my_probes++;
             }
-            const bool gR = gate_right(j, len1, P.k), gL = gate_left(j, P.k, P.h);
-            u32 nR = 0, nL = 0;
-            for (u32 e = 0; e < cnt; ++e) {
-                const u32 ent = cnt == 1 ? (u32)payload : __ldg(&P.entries[payload + e]);
-                const bool right = !(ent & 1u);
-                const bool keep = e == 0 || ((ent >> 2) != (u32)i && (right ? gR : gL));
-                if (keep) { if (right) nR++; else nL++; }
-            }
-            u32 incl = nR | (nL << 16);
-            const u32 own = incl;
+            // The chunk's bucket sizes are scanned once; the warp then walks the chunk's entries 32 at a time, one per
+            // lane (a bucket's entries are contiguous, so the loads are near-coalesced).  A lane finds its window by a
+            // binary search over the scan, and the kept entries are compacted by ballot: both lists stay in window
+            // order, then bucket order.
+            u32 incl = cnt;
 #pragma unroll
             for (int o = 1; o < 32; o <<= 1) { const u32 y = __shfl_up_sync(FULL, incl, o); if (lane >= o) incl += y; }
+            const u32 excl = incl - cnt;
             const u32 tot = __shfl_sync(FULL, incl, 31);
-            if (Tr + Tl + (int)(tot & 0xFFFF) + (int)(tot >> 16) > kFastCap) { punt = true; break; }
-            u32 posR = (u32)Tr + ((incl - own) & 0xFFFF), posL = (u32)Tl + ((incl - own) >> 16);
-            for (u32 e = 0; e < cnt; ++e) {
-                const u32 ent = cnt == 1 ? (u32)payload : __ldg(&P.entries[payload + e]);
-                const bool right = !(ent & 1u);
-                const bool keep = e == 0 || ((ent >> 2) != (u32)i && (right ? gR : gL));
-                if (keep) {
-                    const u32 at = right ? posR++ : (u32)kFastCap - 1 - posL++;
-                    ents[at] = ent;
-                    wins[at] = (uint8_t)(j | (e == 0 ? 0x80 : 0));
+            for (u32 t0 = 0; t0 < tot; t0 += 32) {
+                const u32 t = t0 + lane;
+                int lo = 0;
+#pragma unroll
+                for (int step = 16; step > 0; step >>= 1) {
+                    const u32 pm = __shfl_sync(FULL, incl, lo + step - 1);
+                    if (pm <= t) lo += step;
                 }
+                const u32 e = t - __shfl_sync(FULL, excl, lo), c = __shfl_sync(FULL, cnt, lo);
+                const u64 pay = __shfl_sync(FULL, payload, lo);
+                const int jw = base + lo;
+                const bool valid = t < tot;
+                u32 ent = 0;
+                if (valid) ent = c == 1 ? (u32)pay : __ldg(&P.entries[pay + e]);
+                const bool right = !(ent & 1u);
+                const bool keep = valid && (e == 0 || ((ent >> 2) != (u32)i && (right ? gate_right(jw, len1, P.k) : gate_left(jw, P.k, P.h))));
+                const unsigned kR = __ballot_sync(FULL, keep && right), kL = __ballot_sync(FULL, keep && !right);
+                const int nR = __popc(kR), nL = __popc(kL);
+                if (Tr + Tl + nR + nL > kFastCap) { punt = true; break; }
+                if (keep) {
+                    const int at = right ? Tr + __popc(kR & lt_mask) : kFastCap - 1 - (Tl + __popc(kL & lt_mask));
+                    ents[at] = ent;
+                    wins[at] = (uint8_t)(jw | (e == 0 ? 0x80 : 0));
+                }
+                Tr += nR; Tl += nL;
             }
-            Tr += (int)(tot & 0xFFFF); Tl += (int)(tot >> 16);
         }
         const int T = Tr + Tl;
         __syncwarp();
@@ -272,7 +297,7 @@ phase_a_fast_kernel(SearchParams P, u64 *__restrict__ extR, u64 *__restrict__ ex
                     const int sM = __shfl_sync(FULL, s, laneM);
                     const int lo = 32 * lane;
                     if (lane < SS && lo + 32 > old && lo < reachM) {
-                        const u64 nb = window_signed<SW>(Qs + laneM * SWP, lo - sM);
+                        const u64 nb = window_signed(Qs + laneM * SWP, lo - sM);
                         u64 mask = ~0ull;
                         if (old > lo) mask &= ~0ull >> (2 * (old - lo));
                         if (reachM < lo + 32) mask &= ~(~0ull >> (2 * (reachM - lo)));
