@@ -147,6 +147,13 @@ int sage2gpu_build_hash_table(sage2gpu_ctx *ctx);
  * sage2gpu_write_graph3 bring it to the host. */
 int sage2gpu_build_overlap_graph(sage2gpu_ctx *ctx);
 
+/* Read-only view of the table this context holds (after any build_hash_table* call, and after table_gather_finish):
+ * device pointers to the slot index (*n_slots uint64 words, `shards` key-hash shards of *sectors_per_shard sectors of 4 slots
+ * each, back to back) and to the entry runs (*n_entries uint32), as core.cuh lays them out.  A context of the sharded layout
+ * (build_hash_table_shard) holds one shard: the keys it owns. */
+int sage2gpu_table_view(sage2gpu_ctx *ctx, const void **slots, uint64_t *n_slots, const void **entries, uint64_t *n_entries,
+                        uint64_t *sectors_per_shard, uint64_t *shards);
+
 /* Multi-GPU form of the same step (SURVEY.md 8(e)): phase A is independent per read
  * (the reference's `omp for`, economyGraph.cpp:71), so with the reads and the table present on every GPU rank
  * `rank` of `world` searches only read ids [rank*chunk, (rank+1)*chunk), chunk = ceil(U/world).

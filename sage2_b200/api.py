@@ -64,7 +64,7 @@ EXPORTS = ["sage2gpu_create", "sage2gpu_destroy", "sage2gpu_last_error", "sage2g
            "sage2gpu_synth_reads", "sage2gpu_build_hash_table_part", "sage2gpu_load_finish_packed", "sage2gpu_peer_copy",
            "sage2gpu_phase_a_import", "sage2gpu_load_max_length", "sage2gpu_load_finish_slice", "sage2gpu_table_bytes",
            "sage2gpu_load_saved_reads", "sage2gpu_saved_reads_info", "sage2gpu_saved_reads_slice", "sage2gpu_saved_reads_pack",
-           "sage2gpu_saved_reads_finish"]
+           "sage2gpu_saved_reads_finish", "sage2gpu_table_view"]
 
 _lib = None
 
@@ -115,6 +115,7 @@ def load_library():
         lib.sage2gpu_phase_a_partition.argtypes = [vp, C.c_int, C.c_int]
         lib.sage2gpu_phase_a_buffers.argtypes = [vp] + [C.POINTER(vp)] * 4 + [u64p, u64p]
         lib.sage2gpu_finish_graph.argtypes = [vp]
+        lib.sage2gpu_table_view.argtypes = [vp, C.POINTER(vp), u64p, C.POINTER(vp), u64p, u64p, u64p]
         lib.sage2gpu_build_hash_table_shard.argtypes = [vp, C.c_int, C.c_int]
         lib.sage2gpu_phase_a_sharded_begin.argtypes = [vp, C.c_int, C.c_int, u64p, u64p]
         lib.sage2gpu_route_begin.argtypes = [vp, C.c_int, C.c_uint64, C.c_uint64, C.c_int, C.c_int, C.POINTER(vp), u64p, u64p]
@@ -307,6 +308,16 @@ class Sage2Gpu:
 
     def finish_graph(self):
         self._check(self._lib.sage2gpu_finish_graph(self._h), "finish_graph")
+
+    def table_view(self) -> dict:
+        """Device pointers and sizes of the table this context holds: "slots" (uint64 x n_slots, `shards` shards of
+        sectors_per_shard sectors of 4 slots) and "entries" (uint32 x n_entries)."""
+        ps, pe = C.c_void_p(), C.c_void_p()
+        v = [C.c_uint64() for _ in range(4)]
+        self._check(self._lib.sage2gpu_table_view(self._h, C.byref(ps), C.byref(v[0]), C.byref(pe), C.byref(v[1]), C.byref(v[2]), C.byref(v[3])),
+                    "table_view")
+        return {"slots": ps.value or 0, "n_slots": int(v[0].value), "entries": pe.value or 0, "n_entries": int(v[1].value),
+                "sectors_per_shard": int(v[2].value), "shards": int(v[3].value)}
 
     # ---- several GPUs, every stage partitioned (include/sage2gpu.h) --------------------------------------------
     def load_reads_partition(self, bases_ptr: int, offsets_ptr: int, n_reads: int, min_overlap: int, device: bool, rank: int, world: int) -> int:

@@ -614,6 +614,21 @@ int sage2gpu_phase_a_buffers(sage2gpu_ctx *ctx, void **right_ext, void **left_ex
     });
 }
 
+int sage2gpu_table_view(sage2gpu_ctx *ctx, const void **slots, uint64_t *n_slots, const void **entries, uint64_t *n_entries,
+                        uint64_t *sectors_per_shard, uint64_t *shards)
+{
+    return guarded(ctx, [&](sg::Context &c) {
+        SG_CHECK(c.have_table, "no table built");
+        SG_CHECK(!c.tb_joint || c.tb_shards > 1, "sage2gpu_table_gather_finish must run first");
+        if (slots) *slots = c.slots.p;
+        if (n_slots) *n_slots = c.cap;
+        if (entries) *entries = c.entries.p;
+        if (n_entries) *n_entries = c.tb_entries;
+        if (sectors_per_shard) *sectors_per_shard = c.cap / sg::kSlotsPerSector / (sg::u64)c.tb_shards;
+        if (shards) *shards = (uint64_t)c.tb_shards;
+    });
+}
+
 int sage2gpu_finish_graph(sage2gpu_ctx *ctx)
 {
     return guarded(ctx, [&](sg::Context &c) { finish_graph(c); });

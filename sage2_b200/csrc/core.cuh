@@ -110,7 +110,7 @@ SG_HD void revcomp_record(const u64 *F, u64 *R, int SW, int len)
 // (key, readId, type) so that every key's entries are contiguous and already in the reference's
 // bucket order (insertion order, hashTable.cpp:94-109).  The open-addressing index maps
 // key -> bucket with one 64-bit slot per distinct key:
-//   [63:40] 24-bit tag of the key hash   [39:33] min(count,127)
+//   [63:40] tag: the low SG_SLOT_TAG_BITS (24) bits of the key hash   [39:33] min(count,127)
 //   [32:0]  count == 1: the entry itself (no second hop);  count > 1: offset of the first entry
 // A slot is never 0 when occupied (count >= 1).  count >= 100 means "masked" (hashTable.cpp:116-121).
 // Slots are grouped in 32-byte SECTORS of 4: a key's home is a sector (one DRAM sector per probe),
@@ -131,7 +131,13 @@ SG_HD u64 mulhi64(u64 a, u64 b)
 }
 constexpr int kSlotsPerSector = 4;
 SG_HD u64 home_sector(u64 hsh, u64 nsec) { return mulhi64(hsh, nsec); }
-SG_HD u64 slot_tag(u64 hsh) { return hsh & 0xFFFFFFull; }
+// Bits of the key hash a slot keeps as its tag.  The product uses all 24; the test suite builds variants with fewer
+// (-DSG_SLOT_TAG_BITS=0 / 8) so that tag collisions, which every search must resolve, happen on small data sets too.
+#ifndef SG_SLOT_TAG_BITS
+#define SG_SLOT_TAG_BITS 24
+#endif
+static_assert(SG_SLOT_TAG_BITS >= 0 && SG_SLOT_TAG_BITS <= 24, "a slot has room for a tag of at most 24 bits");
+SG_HD u64 slot_tag(u64 hsh) { return hsh & ((1ull << SG_SLOT_TAG_BITS) - 1); }
 SG_HD u64 slot_encode(u64 hsh, u64 count, u64 payload)
 {
     return (slot_tag(hsh) << 40) | ((count > 127 ? 127ull : count) << 33) | payload;

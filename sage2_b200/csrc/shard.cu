@@ -123,8 +123,6 @@ __global__ void __launch_bounds__(RT_WARPS * 32) route_kernel(const u64 *__restr
 // ---- owner: answers -------------------------------------------------------------------------------------------
 // hashTableSearch on this shard's sector index.  Tag probes take the first slot whose 24-bit tag matches (proven by
 // the source's search kernel); verified probes confirm the key from the bucket's first read and skip masked keys.
-// fake_mask (test knob SAGE2GPU_FAKE_TAG_COLLISIONS): tag probes whose hash has none of these bits take the first
-// occupied slot they see, i.e. behave like a tag collision.
 constexpr u32 kEntryChunk = 1024;     // entries a warp of answer_fused_kernel reserves at a time (one atomic per ~1000 entries)
 
 struct ShardView {
@@ -134,7 +132,6 @@ struct ShardView {
     const u64 *F, *RC;
     const uint16_t *len;
     int SW, SWS, h;
-    u64 fake_mask;
 };
 
 // answer word of query p (payload = OWNER-side offset for a 2..99-entry bucket, whose length comes back in `run`)
@@ -143,14 +140,13 @@ __device__ __forceinline__ u64 answer_one(const ShardView &T, const u64 *__restr
     const u64 *slots = T.slots, *F = T.F, *RC = T.RC;
     const u32 *entries = T.entries;
     const uint16_t *len = T.len;
-    const u64 nsec = T.nsec, fake_mask = T.fake_mask;
+    const u64 nsec = T.nsec;
     const int SW = T.SW, SWS = T.SWS, h = T.h;
     {
         u64 v0 = 0, v1 = 0, hsh;
         if (exact) { v0 = queries[2 * p]; v1 = queries[2 * p + 1]; hsh = hash_key(v0, v1); }
         else hsh = queries[p];
         const u64 tag = slot_tag(hsh);
-        const bool fake = !exact && fake_mask != 0 && (hsh & fake_mask) == 0;
         u64 answer = 0;
         run = 0;
         bool done = nsec == 0;
@@ -163,7 +159,7 @@ __device__ __forceinline__ u64 answer_one(const ShardView &T, const u64 *__restr
                 if (done) continue;
                 const u64 slot = s[t];
                 if (slot == 0) { done = true; continue; }
-                if (slot_get_tag(slot) != tag && !fake) continue;
+                if (slot_get_tag(slot) != tag) continue;
                 const u32 c = slot_get_count(slot);
                 const u64 pay = slot_get_payload(slot);
                 if (exact) {
@@ -287,11 +283,11 @@ __global__ void __launch_bounds__(256) compact_list_kernel(const u32 *__restrict
         if (flag[i]) out[idx[i]] = base + (u32)i;
 }
 
-static ShardView shard_view(const Context &c, u64 fake_mask)
+static ShardView shard_view(const Context &c)
 {
     ShardView T;
     T.slots = c.slots.p; T.nsec = c.cap / kSlotsPerSector; T.entries = c.entries.p; T.F = c.F.p; T.RC = c.RC.p; T.len = c.len.p;
-    T.SW = c.SW; T.SWS = c.SWS; T.h = c.h; T.fake_mask = fake_mask;
+    T.SW = c.SW; T.SWS = c.SWS; T.h = c.h;
     return T;
 }
 
@@ -416,13 +412,11 @@ void stage_shard_answer(Context &c, const void *queries, const u64 *counts_per_s
     *responses = nullptr; *entries = nullptr;
     if (nq == 0) return;
     SG_CHECK(queries != nullptr, "null query buffer");
-    const char *fake_env = getenv("SAGE2GPU_FAKE_TAG_COLLISIONS");
-    const u64 fake_mask = fake_env ? strtoull(fake_env, nullptr, 0) : 0ull;
     c.an_resp.alloc(nq, st);
     DevBuf<u32> runlen(nq + 1, st), off(nq + 1, st), d_total(1, st);
     DevBuf<u64> d_seg(world + 1, st), d_ecnt(world, st);
     SG_CUDA(cudaMemcpyAsync(d_seg.p, h_seg, (world + 1) * sizeof(u64), cudaMemcpyHostToDevice, st));
-    const ShardView T = shard_view(c, fake_mask);
+    const ShardView T = shard_view(c);
     answer_kernel<<<sm_grid(nq, 256, 8), 256, 0, st>>>((const u64 *)queries, nq, exact, T, c.an_resp.p, runlen.p);
     SG_LAUNCHED();
     // up to 99 entries per query: the grand total is checked in 64 bits before the 32-bit scan is trusted
@@ -690,10 +684,8 @@ void stage_answer_post(Context &c, int exact, u64 *bytes_sent)
     if (bytes_sent) *bytes_sent = 0;
     if (nq == 0) return;
     SG_CHECK(nq < 0xFFFFFFFFull, "too many queries for one batch");
-    const char *fake_env = getenv("SAGE2GPU_FAKE_TAG_COLLISIONS");
-    const u64 fake_mask = fake_env ? strtoull(fake_env, nullptr, 0) : 0ull;
     // one fused launch per source: answers land in the source's mailbox while the kernel runs ("combine")
-    const ShardView T = shard_view(c, fake_mask);
+    const ShardView T = shard_view(c);
     DevBuf<unsigned long long> d_cur(world, st);
     SG_CUDA(cudaMemsetAsync(d_cur.p, 0, world * sizeof(unsigned long long), st));
     c.an_entries.alloc((u64)world * m.ecap, st);

@@ -79,18 +79,6 @@ def test_small_pieces_reach_every_context(name, tmp_path):
         assert f"Number of unique reads: {GOLD[name]['unique_reads']}" in log
 
 
-def test_sharded_layout_takes_the_verified_pass(tmp_path):
-    """Fake 24-bit tag collisions (test knob of csrc/shard.cu): the reads that met one are routed once more with exact keys."""
-    reads, k = _get("varlen_err")
-    fq = tmp_path / "in.fastq"
-    synth.write_fastq(str(fq), reads)
-    for devs in DEVICES:
-        r, g, log = _run(["-f", str(fq), "-k", str(k)], tmp_path / devs.replace(",", "_"), devs, "sharded",
-                         SAGE2GPU_FAKE_TAG_COLLISIONS="0x3f00000000")
-        assert (r, g) == _gold("varlen_err"), devs
-        assert int(re.search(r"reads of the verified redo pass \(max over the contexts\): (\d+)", log).group(1)) > 0
-
-
 def test_sharded_layout_grows_the_mailboxes_for_the_phase_c_list(tmp_path):
     """An error-rich set sends many reads to phase C; with routed batches of 64 reads the list batch is far larger than the
     mailboxes, which must grow for it."""

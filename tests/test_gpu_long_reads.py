@@ -208,18 +208,6 @@ def test_sharded_table_equals_oracle(name, world, p2p):
         np.testing.assert_array_equal(g.extensions()["explored"], o.explored_b[1:])
 
 
-def test_sharded_tag_collisions_at_the_widest_stride(monkeypatch):
-    """Fake tag collisions send probes through the verified pass of the routed kernel, which runs one resident block at
-    SW > 8."""
-    monkeypatch.setenv("SAGE2GPU_FAKE_TAG_COLLISIONS", "0x3f00000000")
-    o, gpus = _sharded("v505", 2)
-    assert sum(g.counters()["probe_restarts"] for g in gpus) > 0
-    assert sum(g.counters()["compare_calls"] for g in gpus) == o.compare_calls
-    for g in gpus:
-        _same_edges(g, o)
-        np.testing.assert_array_equal(g.extensions()["explored"], o.explored_b[1:])
-
-
 # ---- f. the streamed upload -------------------------------------------------------------------------------------------
 
 def test_streamed_upload_equals_one_shot():

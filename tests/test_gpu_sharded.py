@@ -55,17 +55,6 @@ def test_sharded_table_over_mailboxes_equals_oracle(name, world):
         np.testing.assert_array_equal(g.extensions()["explored"], o.explored_b[1:])
 
 
-def test_mailbox_tag_collisions(monkeypatch):
-    monkeypatch.setenv("SAGE2GPU_FAKE_TAG_COLLISIONS", "0x3f00000000")
-    o, gpus = _sharded("varlen_err", 2, p2p=True)
-    assert sum(g.counters()["probe_restarts"] for g in gpus) > 0
-    for g in gpus:
-        e = g.edges()
-        assert len(e) == o.n_edges
-        for f in ("from", "to", "type", "delta", "delta_twin"):
-            np.testing.assert_array_equal(e[f], o.edges[f])
-
-
 @pytest.mark.parametrize("name,world", [("clean", 1), ("rep", 2), ("k70", 3), ("hicopy", 2), ("deep", 2), ("varlen_err", 3),
                                         ("deep_varlen", 2), ("tandem", 2), ("mixed", 4), ("err", 8), ("k31", 2),
                                         ("empty", 2), ("allbad", 2), ("single", 3)])
@@ -91,20 +80,6 @@ def test_small_batches_and_uneven_slices():
         assert len(e) == o.n_edges
         for f in ("from", "to", "type", "delta", "delta_twin"):
             np.testing.assert_array_equal(e[f], o.edges[f])
-
-
-def test_tag_collisions_take_the_verified_pass(monkeypatch):
-    # test knob of csrc/shard.cu: tag probes whose key hash has none of the mask bits behave like a tag collision
-    monkeypatch.setenv("SAGE2GPU_FAKE_TAG_COLLISIONS", "0x3f00000000")
-    o, gpus = _sharded("varlen_err", 2)
-    assert sum(g.counters()["probe_restarts"] for g in gpus) > 0
-    assert sum(g.counters()["compare_calls"] for g in gpus) == o.compare_calls
-    for g in gpus:
-        e = g.edges()
-        assert len(e) == o.n_edges
-        for f in ("from", "to", "type", "delta", "delta_twin"):
-            np.testing.assert_array_equal(e[f], o.edges[f])
-        np.testing.assert_array_equal(g.extensions()["explored"], o.explored_b[1:])
 
 
 def test_sharded_context_refuses_the_local_search():
