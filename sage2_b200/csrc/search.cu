@@ -26,7 +26,7 @@
 namespace sg {
 
 // search_fast.cu
-bool launch_phase_a_fast(Context &c, const SearchParams &P, unsigned long long *d_counters, u32 *redo_ids, unsigned *redo_count);
+bool launch_phase_a_fast(Context &c, const SearchParams &P, unsigned long long *d_counters, DevBuf<u32> &redo_ids, DevBuf<unsigned> &redo_n);
 
 // FAST-mode scan state of one read (warp-uniform): first right hit, last left hit, last hit of each side
 struct FastState {
@@ -109,10 +109,11 @@ __device__ __forceinline__ u64 make_item(int jj, bool first, bool inl, u64 paylo
 // ------------------------------------------------------------------------------------------------
 // K4: phase A
 // ------------------------------------------------------------------------------------------------
-// ORDERED: the batch is processed in the order of the id list P.ids instead of id order (the reads the superstring scan
-// left, or the minimizer order that keeps overlapping reads together in time, DESIGN.md section 3); results do not depend on it.
-template <int SW, int MINB, bool ROUTED, bool ORDERED = false>
-__global__ void __launch_bounds__(SearchCfg<SW>::WARPS * 32, MINB)
+// With an id list P.ids the batch is processed in its order instead of id order (the reads the superstring scan left, or
+// the minimizer order that keeps overlapping reads together in time, DESIGN.md section 3); results do not depend on it.
+// Registers are cut for 4 resident blocks per SM up to 8 words (3 and 5 were measured slower, DESIGN.md section 3), 1 above.
+template <int SW, bool ROUTED>
+__global__ void __launch_bounds__(SearchCfg<SW>::WARPS * 32, SW <= 8 ? 4 : 1)
 phase_a_kernel(SearchParams P, u64 *__restrict__ extR, u64 *__restrict__ extL, uint8_t *__restrict__ flag5,
                u32 *__restrict__ cont_max, unsigned long long *__restrict__ counters)
 {
@@ -132,9 +133,9 @@ phase_a_kernel(SearchParams P, u64 *__restrict__ extR, u64 *__restrict__ extL, u
     unsigned calls = 0, probes = 0, n_exact = 0, n_restart = 0;      // per warp: far below 2^32
     if (lane == 0) { Xf[SW] = 0; Xr[SW] = 0; prevR[SW] = 0; prevL[SW] = 0; }
 
-    const u64 n_batch = ROUTED ? P.n : ((ORDERED && P.n_dev) ? (u64)*P.n_dev : P.hi - P.lo);
+    const u64 n_batch = ROUTED ? P.n : (P.n_dev ? (u64)*P.n_dev : P.hi - P.lo);
     for (u64 sb = (u64)blockIdx.x * WARPS + warp; sb < n_batch; sb += nwarps) {
-        const u64 i = ((ROUTED || ORDERED) && P.ids) ? (u64)P.ids[sb] : P.lo + sb;
+        const u64 i = P.ids ? (u64)P.ids[sb] : P.lo + sb;
         if (lane < SW) { Xf[lane] = P.F[i * SWS + lane]; Xr[lane] = P.RC[i * SWS + lane]; }
         __syncwarp();
         const int len1 = (int)(Xf[SW - 1] & 0xFFFF);
@@ -488,55 +489,14 @@ phase_c_kernel(SearchParams P, const u32 *__restrict__ s_ids, u64 nS, const uint
 // ------------------------------------------------------------------------------------------------
 // host side
 // ------------------------------------------------------------------------------------------------
-static unsigned search_grid(u64 n_reads, int warps, int blocks_per_sm)
-{
-    u64 g = (n_reads + warps - 1) / warps;
-    const u64 cap = (u64)kSMs * blocks_per_sm;
-    if (g > cap) g = cap;
-    if (g == 0) g = 1;
-    return (unsigned)g;
-}
-
-template <int SW, int MINB, bool ROUTED>
-static void launch_phase_a_v(Context &c, const SearchParams &P, unsigned long long *d_counters)
-{
-    constexpr int WARPS = SearchCfg<SW>::WARPS;
-    static int blocks_per_sm = 0;
-    if (blocks_per_sm == 0) {
-        SG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, phase_a_kernel<SW, MINB, ROUTED>, WARPS * 32, 0));
-        if (blocks_per_sm < 1) blocks_per_sm = 1;
-    }
-    const u64 n = ROUTED ? P.n : P.hi - P.lo;
-    phase_a_kernel<SW, MINB, ROUTED><<<search_grid(n, WARPS, blocks_per_sm), WARPS * 32, 0, c.stream>>>(P, c.extR.p, c.extL.p, c.flag5.p, c.cont_max.p, d_counters);
-}
-
-// MINB = resident blocks per SM the register budget is cut for (occupancy against spills).
-template <int SW>
+// the local search of a slice and its redo pass after the scan, or (ROUTED) one routed batch; the grid covers the whole
+// slice or batch even when only the device knows how many ids a list holds
+template <int SW, bool ROUTED>
 static void launch_phase_a(Context &c, const SearchParams &P, unsigned long long *d_counters)
 {
-    if constexpr (SW <= 8) {
-        static const int minb = [] { const char *e = getenv("SAGE2GPU_PA_MINB"); return e ? atoi(e) : 4; }();
-        if (minb <= 2) launch_phase_a_v<SW, 2, false>(c, P, d_counters);
-        else if (minb == 3) launch_phase_a_v<SW, 3, false>(c, P, d_counters);
-        else if (minb == 4) launch_phase_a_v<SW, 4, false>(c, P, d_counters);
-        else launch_phase_a_v<SW, 5, false>(c, P, d_counters);
-    } else {
-        launch_phase_a_v<SW, 1, false>(c, P, d_counters);
-    }
-}
-
-template <int SW>
-static void launch_phase_a_ordered(Context &c, const SearchParams &P, unsigned long long *d_counters)
-{
     constexpr int WARPS = SearchCfg<SW>::WARPS;
-    constexpr int MINB = SW <= 8 ? 4 : 1;
-    static int blocks_per_sm = 0;
-    if (blocks_per_sm == 0) {
-        SG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, phase_a_kernel<SW, MINB, false, true>, WARPS * 32, 0));
-        if (blocks_per_sm < 1) blocks_per_sm = 1;
-    }
-    phase_a_kernel<SW, MINB, false, true><<<search_grid(P.hi - P.lo, WARPS, blocks_per_sm), WARPS * 32, 0, c.stream>>>(P, c.extR.p, c.extL.p, c.flag5.p,
-                                                                                                                   c.cont_max.p, d_counters);
+    const unsigned g = persistent_grid<phase_a_kernel<SW, ROUTED>>(ROUTED ? P.n : P.hi - P.lo, WARPS);
+    phase_a_kernel<SW, ROUTED><<<g, WARPS * 32, 0, c.stream>>>(P, c.extR.p, c.extL.p, c.flag5.p, c.cont_max.p, d_counters);
 }
 
 #define SG_DISPATCH_SW(SWV, CALL)                                                       \
@@ -626,13 +586,6 @@ static const u32 *minimizer_order(Context &c, u64 lo, u64 hi, DevBuf<u64> &ka, D
 }
 
 template <int SW>
-static void launch_phase_a_routed(Context &c, const SearchParams &P, unsigned long long *d_counters)
-{
-    if constexpr (SW <= 8) launch_phase_a_v<SW, 4, true>(c, P, d_counters);
-    else launch_phase_a_v<SW, 1, true>(c, P, d_counters);
-}
-
-template <int SW>
 static void launch_phase_c(Context &c, const SearchParams &P, const u32 *s_ids, u64 nS, u32 *counts, const u32 *offsets, u64 *cand, bool fill)
 {
     constexpr int WARPS = SearchCfg<SW>::WARPS;
@@ -675,67 +628,84 @@ static void use_routed_batch(const Context &c, SearchParams &P)
     P.trusted = c.rt_exact ? 1 : 0;
 }
 
+// Rank `rank`'s slice [lo, hi) of the reads cut into `world` equal chunks, and the phase-A arrays of all chunks (the
+// exchange moves whole chunks); cont_max and the counters start at 0.
+static void begin_phase_a(Context &c, int rank, int world, u64 &lo, u64 &hi)
+{
+    cudaStream_t st = c.stream;
+    SG_CHECK(world >= 1 && rank >= 0 && rank < world, "bad rank / world");
+    const u64 U = c.cnt.unique_reads;
+    const u64 chunk = partition_chunk(U, world), padded = chunk * (u64)world;
+    c.pa_chunk = chunk; c.pa_world = world;
+    lo = (u64)rank * chunk < U ? (u64)rank * chunk : U;
+    hi = lo + chunk < U ? lo + chunk : U;
+    c.have_phase_a = false; c.have_phase_b = false; c.have_graph = false;
+    c.extR.alloc(padded, st); c.extL.alloc(padded, st); c.flag5.alloc(padded, st); c.cont_max.alloc(padded, st);
+    c.cnt.compare_calls = 0; c.cnt.window_probes = 0; c.cnt.slow_path_reads = 0; c.cnt.probe_restarts = 0;
+    if (U > 0) SG_CUDA(cudaMemsetAsync(c.cont_max.p, 0, padded * sizeof(u32), st));
+}
+
+// The phase-A kernels' counters (compare calls, window probes, slow-path reads, probe restarts), zeroed, and the time of
+// the launches between construction and finish().
+struct PhaseARun {
+    cudaStream_t st;
+    DevBuf<unsigned long long> counters;
+    cudaEvent_t e0 = nullptr, e1 = nullptr;
+    explicit PhaseARun(cudaStream_t s) : st(s), counters(4, s)
+    {
+        SG_CUDA(cudaMemsetAsync(counters.p, 0, 4 * sizeof(unsigned long long), st));
+        SG_CUDA(cudaEventCreate(&e0)); SG_CUDA(cudaEventCreate(&e1));
+        SG_CUDA(cudaEventRecord(e0, st));
+    }
+    ~PhaseARun() { cudaEventDestroy(e0); cudaEventDestroy(e1); }
+    // waits for the launches; h = the counters, returns their time in ms
+    float finish(unsigned long long (&h)[4])
+    {
+        SG_CUDA(cudaEventRecord(e1, st));
+        SG_CUDA(cudaMemcpyAsync(h, counters.p, sizeof(h), cudaMemcpyDeviceToHost, st));
+        SG_CUDA(cudaStreamSynchronize(st));
+        float ms = 0;
+        cudaEventElapsedTime(&ms, e0, e1);
+        return ms;
+    }
+};
+
 void stage_phase_a(Context &c, int rank, int world)
 {
     cudaStream_t st = c.stream;
     ArenaScope arena_scope(c.arena, st);
     SG_CHECK(c.have_table, "build_hash_table must run before the overlap search");
     SG_CHECK(c.tb_world == 1, "this context holds one shard of the table: use the routed search (sage2gpu_route_*)");
-    SG_CHECK(world >= 1 && rank >= 0 && rank < world, "bad rank / world");
-    const u64 U = c.cnt.unique_reads;
-    const u64 chunk = partition_chunk(U, world), padded = chunk * (u64)world;
-    c.pa_chunk = chunk; c.pa_world = world;
-    c.have_phase_a = false; c.have_phase_b = false; c.have_graph = false;
-    c.extR.alloc(padded, st); c.extL.alloc(padded, st); c.flag5.alloc(padded, st); c.cont_max.alloc(padded, st);
-    c.cnt.compare_calls = 0; c.cnt.window_probes = 0; c.cnt.slow_path_reads = 0; c.cnt.probe_restarts = 0;
-    if (U == 0) { c.have_phase_a = true; return; }
+    SearchParams P = make_params(c);
+    begin_phase_a(c, rank, world, P.lo, P.hi);
+    if (c.cnt.unique_reads == 0) { c.have_phase_a = true; return; }
     if (world > 1) {      // slices of other ranks (and the padding) are defined before the exchange overwrites them
+        const u64 padded = c.pa_chunk * (u64)world;
         SG_CUDA(cudaMemsetAsync(c.extR.p, 0, padded * sizeof(u64), st));
         SG_CUDA(cudaMemsetAsync(c.extL.p, 0, padded * sizeof(u64), st));
         SG_CUDA(cudaMemsetAsync(c.flag5.p, 0, padded, st));
     }
-    SG_CUDA(cudaMemsetAsync(c.cont_max.p, 0, padded * sizeof(u32), st));
-    DevBuf<unsigned long long> d_counters(4, st);
-    SG_CUDA(cudaMemsetAsync(d_counters.p, 0, 4 * sizeof(unsigned long long), st));
-    SearchParams P = make_params(c);
-    P.lo = (u64)rank * chunk < U ? (u64)rank * chunk : U;
-    P.hi = P.lo + chunk < U ? P.lo + chunk : U;
-    cudaEvent_t e0, e1;
-    SG_CUDA(cudaEventCreate(&e0)); SG_CUDA(cudaEventCreate(&e1));
-    SG_CUDA(cudaEventRecord(e0, st));
     // SAGE2GPU_READ_ORDER=id|minimizer ("minhash" is read as minimizer); unset: by footprint
     static const int env_order = [] { const char *e = getenv("SAGE2GPU_READ_ORDER"); return !e ? -1 : (e[0] == 'm' ? 1 : 0); }();
     static const bool env_fast = [] { const char *e = getenv("SAGE2GPU_PA_FAST"); return !(e && e[0] == '0'); }();
     const int order = c.opt_read_order >= 0 ? c.opt_read_order : env_order;
     const bool by_minimizer = order >= 0 ? order == 1 : read_order_pays(c);
-    const bool fast = (c.opt_fast_scan < 0 ? env_fast : c.opt_fast_scan == 1) && c.SW <= 8;
+    const bool fast = c.opt_fast_scan < 0 ? env_fast : c.opt_fast_scan == 1;
     DevBuf<u64> oka, okb;
     DevBuf<u32> ova, ovb, redo_ids;
     DevBuf<unsigned> redo_n;
-    if (P.hi > P.lo && by_minimizer) {      // schedule that keeps overlapping reads together in time (DESIGN.md section 3)
-        P.ids = minimizer_order(c, P.lo, P.hi, oka, okb, ova, ovb);
-        SG_CUDA(cudaEventRecord(e0, st));    // the ordering is not part of the search kernel's time (it is part of the stage's)
-    }
-    if (P.hi > P.lo && fast) {
+    // schedule that keeps overlapping reads together in time (DESIGN.md section 3); the ordering is part of the stage's
+    // time, not of the search kernel's
+    if (P.hi > P.lo && by_minimizer) P.ids = minimizer_order(c, P.lo, P.hi, oka, okb, ova, ovb);
+    PhaseARun run(st);
+    if (P.hi > P.lo) {
         // the superstring scan first (search_fast.cu); the general kernel then takes the reads it could not certify
-        redo_ids.alloc(P.hi - P.lo, st); redo_n.alloc(1, st);
-        SG_CUDA(cudaMemsetAsync(redo_n.p, 0, sizeof(unsigned), st));
-        launch_phase_a_fast(c, P, d_counters.p, redo_ids.p, redo_n.p);
-        SearchParams P2 = P;
-        P2.ids = redo_ids.p; P2.n_dev = redo_n.p;
-        SG_DISPATCH_SW(c.SW, launch_phase_a_ordered<SWC>(c, P2, d_counters.p));
-        SG_LAUNCHED();
-    } else if (P.hi > P.lo && by_minimizer) {
-        SG_DISPATCH_SW(c.SW, launch_phase_a_ordered<SWC>(c, P, d_counters.p));
-        SG_LAUNCHED();
-    } else if (P.hi > P.lo) {
-        SG_DISPATCH_SW(c.SW, launch_phase_a<SWC>(c, P, d_counters.p));
+        if (fast && launch_phase_a_fast(c, P, run.counters.p, redo_ids, redo_n)) { P.ids = redo_ids.p; P.n_dev = redo_n.p; }
+        SG_DISPATCH_SW(c.SW, (launch_phase_a<SWC, false>(c, P, run.counters.p)));
         SG_LAUNCHED();
     }
-    SG_CUDA(cudaEventRecord(e1, st));
     unsigned long long h[4];
-    SG_CUDA(cudaMemcpyAsync(h, d_counters.p, sizeof(h), cudaMemcpyDeviceToHost, st));
-    SG_CUDA(cudaStreamSynchronize(st));
+    c.tm.phase_a_kernel = run.finish(h);
     c.cnt.compare_calls = h[0];
     c.cnt.window_probes = h[1];
     c.cnt.slow_path_reads = h[2];
@@ -747,8 +717,6 @@ void stage_phase_a(Context &c, int rank, int world)
         SG_CUDA(cudaStreamSynchronize(st));
         c.cnt.fast_path_reads = (P.hi - P.lo) - nr;
     }
-    cudaEventElapsedTime(&c.tm.phase_a_kernel, e0, e1);
-    cudaEventDestroy(e0); cudaEventDestroy(e1);
     c.have_phase_a = true;
 }
 
@@ -784,23 +752,15 @@ void stage_phase_a_sharded_begin(Context &c, int rank, int world)
 {
     cudaStream_t st = c.stream;
     SG_CHECK(c.have_table, "build_hash_table[_shard] must run before the overlap search");
-    SG_CHECK(world >= 1 && rank >= 0 && rank < world, "bad rank / world");
-    const u64 U = c.cnt.unique_reads;
-    const u64 chunk = partition_chunk(U, world), padded = chunk * (u64)world;
-    c.pa_chunk = chunk; c.pa_world = world;
-    c.pa_lo = (u64)rank * chunk < U ? (u64)rank * chunk : U;
-    c.pa_hi = c.pa_lo + chunk < U ? c.pa_lo + chunk : U;
-    c.have_phase_a = false; c.have_phase_b = false; c.have_graph = false;
-    c.extR.alloc(padded, st); c.extL.alloc(padded, st); c.flag5.alloc(padded, st); c.cont_max.alloc(padded, st);
-    c.rt_redo.alloc(chunk, st);
-    c.cnt.compare_calls = 0; c.cnt.window_probes = 0; c.cnt.slow_path_reads = 0; c.cnt.probe_restarts = 0;
+    begin_phase_a(c, rank, world, c.pa_lo, c.pa_hi);
+    c.rt_redo.alloc(c.pa_chunk, st);
     c.tm.phase_a_kernel = 0;
-    if (U == 0) return;
+    if (c.cnt.unique_reads == 0) return;
+    const u64 padded = c.pa_chunk * (u64)world;
     SG_CUDA(cudaMemsetAsync(c.extR.p, 0, padded * sizeof(u64), st));
     SG_CUDA(cudaMemsetAsync(c.extL.p, 0, padded * sizeof(u64), st));
     SG_CUDA(cudaMemsetAsync(c.flag5.p, 0, padded, st));
-    SG_CUDA(cudaMemsetAsync(c.cont_max.p, 0, padded * sizeof(u32), st));
-    SG_CUDA(cudaMemsetAsync(c.rt_redo.p, 0, chunk, st));
+    SG_CUDA(cudaMemsetAsync(c.rt_redo.p, 0, c.pa_chunk, st));
 }
 
 // K4 on the routed batch (route_begin .. route_finish); returns the reads of the batch flagged for the redo pass
@@ -818,26 +778,17 @@ u64 stage_phase_a_routed(Context &c)
     DevBuf<uint8_t> redo2;
     if (c.rt_is_list) { redo2.alloc(c.rt_n, st); SG_CUDA(cudaMemsetAsync(redo2.p, 0, c.rt_n, st)); P.redo = redo2.p; }
     else P.redo = c.rt_redo.p + (c.rt_first - c.pa_lo);
-    DevBuf<unsigned long long> d_counters(4, st);
-    SG_CUDA(cudaMemsetAsync(d_counters.p, 0, 4 * sizeof(unsigned long long), st));
-    cudaEvent_t e0, e1;
-    SG_CUDA(cudaEventCreate(&e0)); SG_CUDA(cudaEventCreate(&e1));
-    SG_CUDA(cudaEventRecord(e0, st));
-    SG_DISPATCH_SW(c.SW, launch_phase_a_routed<SWC>(c, P, d_counters.p));
+    PhaseARun run(st);
+    SG_DISPATCH_SW(c.SW, (launch_phase_a<SWC, true>(c, P, run.counters.p)));
     SG_LAUNCHED();
-    SG_CUDA(cudaEventRecord(e1, st));
     unsigned long long h[4];
-    SG_CUDA(cudaMemcpyAsync(h, d_counters.p, sizeof(h), cudaMemcpyDeviceToHost, st));
-    SG_CUDA(cudaStreamSynchronize(st));
+    const float ms = run.finish(h);
     c.cnt.compare_calls += h[0];
     c.cnt.window_probes += h[1];
     c.cnt.slow_path_reads += h[2];
     if (!c.rt_exact) c.cnt.probe_restarts += h[3];
     else SG_CHECK(h[3] == 0, "a verified answer failed its proof in the search kernel");
-    float ms = 0;
-    cudaEventElapsedTime(&ms, e0, e1);
     c.tm.phase_a_kernel += ms;
-    cudaEventDestroy(e0); cudaEventDestroy(e1);
     return h[3];
 }
 

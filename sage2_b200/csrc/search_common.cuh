@@ -24,7 +24,8 @@ struct SearchParams {
     u64 n;
     u32 wstride;
     int trusted;
-    // phase_a_kernel<.., ORDERED>: number of ids when it is only known on the device (the redo list of search_fast.cu)
+    // phase_a_kernel (not ROUTED): number of ids when it is only known on the device (the redo list of search_fast.cu);
+    // nullptr: ids[0..hi-lo), or [lo, hi) in id order when ids is nullptr too
     const unsigned *n_dev;
 };
 
@@ -51,6 +52,30 @@ struct SearchCfg {
     static constexpr int LPI = SWS / 4;          // lanes that fetch one partner record together (one sector each)
     static constexpr int SWP = SWS + 1;          // odd record stride in shared memory (bank spread) + the word read past
 };
+
+// Grid of a warp-per-read kernel with a grid-stride loop: one warp per read, at most blocks_per_sm blocks per SM, at least
+// one block.
+inline unsigned search_grid(u64 n_reads, int warps, int blocks_per_sm)
+{
+    u64 g = (n_reads + warps - 1) / warps;
+    const u64 cap = (u64)kSMs * blocks_per_sm;
+    if (g > cap) g = cap;
+    if (g == 0) g = 1;
+    return (unsigned)g;
+}
+
+// search_grid for a persistent launch of KERNEL: as many blocks per SM as can be resident at once (occupancy API, asked
+// once per kernel).
+template <auto KERNEL>
+unsigned persistent_grid(u64 n_reads, int warps)
+{
+    static int blocks_per_sm = 0;
+    if (blocks_per_sm == 0) {
+        SG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, KERNEL, warps * 32, 0));
+        if (blocks_per_sm < 1) blocks_per_sm = 1;
+    }
+    return search_grid(n_reads, warps, blocks_per_sm);
+}
 
 template <int SW>
 __device__ __forceinline__ u64 t_window32(const u64 *X, int s)

@@ -347,30 +347,25 @@ phase_a_fast_kernel(SearchParams P, u64 *__restrict__ extR, u64 *__restrict__ ex
 }
 
 template <int SW, int MINB>
-static void launch_fast_v(Context &c, const SearchParams &P, unsigned long long *d_counters, u32 *redo_ids, unsigned *redo_count)
+static void launch_fast_v(Context &c, const SearchParams &P, unsigned long long *d_counters, DevBuf<u32> &redo_ids, DevBuf<unsigned> &redo_n)
 {
     constexpr int WARPS = SearchCfg<SW>::WARPS;
-    static int blocks_per_sm = 0;
-    if (blocks_per_sm == 0) {
-        SG_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks_per_sm, phase_a_fast_kernel<SW, MINB>, WARPS * 32, 0));
-        if (blocks_per_sm < 1) blocks_per_sm = 1;
-    }
-    u64 g = (P.hi - P.lo + WARPS - 1) / WARPS;
-    if (g > (u64)kSMs * blocks_per_sm) g = (u64)kSMs * blocks_per_sm;
-    if (g == 0) g = 1;
-    phase_a_fast_kernel<SW, MINB><<<(unsigned)g, WARPS * 32, 0, c.stream>>>(P, c.extR.p, c.extL.p, c.flag5.p, c.cont_max.p, d_counters, redo_ids,
-                                                                            redo_count);
+    redo_ids.alloc(P.hi - P.lo, c.stream); redo_n.alloc(1, c.stream);
+    SG_CUDA(cudaMemsetAsync(redo_n.p, 0, sizeof(unsigned), c.stream));
+    const unsigned g = persistent_grid<phase_a_fast_kernel<SW, MINB>>(P.hi - P.lo, WARPS);
+    phase_a_fast_kernel<SW, MINB><<<g, WARPS * 32, 0, c.stream>>>(P, c.extR.p, c.extL.p, c.flag5.p, c.cont_max.p, d_counters, redo_ids.p, redo_n.p);
 }
 
 // The superstring scan of reads [P.lo, P.hi) (in the order of P.ids when given); the reads it could not certify are
-// appended to redo_ids (*redo_count of them).  false: no instantiation for this record stride (long reads).
-bool launch_phase_a_fast(Context &c, const SearchParams &P, unsigned long long *d_counters, u32 *redo_ids, unsigned *redo_count)
+// listed in redo_ids (*redo_n of them; both allocated here).  false: no instantiation for this record stride (long
+// reads), nothing launched.
+bool launch_phase_a_fast(Context &c, const SearchParams &P, unsigned long long *d_counters, DevBuf<u32> &redo_ids, DevBuf<unsigned> &redo_n)
 {
     switch (c.SW) {
         // 4 resident blocks per SM (64 registers): 3 blocks (79 registers) and 5 blocks (48 registers, spills) were measured
         // slower, 12.3 / 11.8 ms against 10.1 ms at cfg2; requesting the home sectors of several window chunks before the
         // first is used was slower too (10.9 / 11.6 / 13.1 ms for 1 / 2 / 3 chunks ahead): the kernel is not short of loads in flight
-#define SG_FAST_CASE(SWV) case SWV: launch_fast_v<SWV, 4>(c, P, d_counters, redo_ids, redo_count); break;
+#define SG_FAST_CASE(SWV) case SWV: launch_fast_v<SWV, 4>(c, P, d_counters, redo_ids, redo_n); break;
         SG_FAST_CASE(2) SG_FAST_CASE(3) SG_FAST_CASE(4) SG_FAST_CASE(5) SG_FAST_CASE(6) SG_FAST_CASE(8)
 #undef SG_FAST_CASE
         default: return false;
