@@ -4,9 +4,11 @@
 // kernel could not certify (a list built on the device; 0 of 2.24 M reads at cfg2, 4,008 of 27.9 M at cfg4).
 //
 // One warp per read.
-//   1. PROBE    all windows of the read first: lane l derives the key of window base+l by funnel shifts, reads ONE
-//               32-byte sector of the slot index and picks its slot without branches; the (window, bucket entry) items
-//               are written to shared memory in the reference's order (window ascending, bucket order).
+//   1. PROBE    all windows of the read first: the lanes derive the windows' keys by funnel shifts and hash them into
+//               shared memory; the sector loads then run as one warp-wide queue (a lane takes the next window as soon as
+//               its walk over 32-byte sectors ends, so no lane waits for another's walk) and a sector's slot is picked
+//               without branches; one walk over the buckets of all windows writes the (window, bucket entry) items to
+//               shared memory in the reference's order (window ascending, bucket order).
 //   2. COMPARE  32 items per round, one partner record per lane (fetched by lane groups, one 256-bit load per sector).
 //               Per side the warp keeps a superstring S in shared memory: read i (right hits) or its reverse complement
 //               (left hits) followed by the bases the hits seen so far agree on beyond its end.  An item is compared
@@ -29,31 +31,18 @@ namespace sg {
 constexpr int kFastCap = 192;        // items (window, bucket entry) of one read held in shared memory
 constexpr int kFastWindows = 128;    // windows of one read (the window travels in 7 bits)
 
-// hashTableSearch (hashTable.cpp:193-231) on the sector index with a branch-free sector test: the slots of a sector fill
-// in order, so empty slots are a suffix and "no tag match + an empty slot" means absent.  A tag match counts as found
-// (proven by the compare of the bucket's first entry).  Returns false for a masked key (>= 100 entries), which
-// probe_window confirms through its representative read.
-__device__ __forceinline__ bool probe_sectors(const SearchParams &P, u64 hsh, u64 &payload, u32 &cnt)
+constexpr uint8_t kFastMasked = 0xFF; // window count of a masked-key candidate until probe_window has settled it
+
+// One step of hashTableSearch (hashTable.cpp:193-231) on the sector index, with a branch-free sector test: the slots of a
+// sector fill in order, so empty slots are a suffix and "no tag match + an empty slot" means absent.  Returns the first
+// slot whose tag matches (0: none); `more`: no match and the sector is full, the key may sit in the next one.
+__device__ __forceinline__ u64 sector_match(const u64 (&s)[4], u64 tag, bool &more)
 {
-    const u64 tag = slot_tag(hsh);
-    const u64 *shard = P.slots + kSlotsPerSector * shard_base_sector(hsh, P.nsec, P.shards);
-    u64 sec = home_sector(hsh, P.nsec);
-    payload = 0; cnt = 0;
-    for (;;) {
-        u64 s[4];
-        ldg256_keep(shard + kSlotsPerSector * sec, s);
-        const bool m0 = (s[0] >> 40) == tag && s[0] != 0, m1 = (s[1] >> 40) == tag && s[1] != 0;
-        const bool m2 = (s[2] >> 40) == tag && s[2] != 0, m3 = (s[3] >> 40) == tag && s[3] != 0;
-        const u64 cand = m0 ? s[0] : (m1 ? s[1] : (m2 ? s[2] : (m3 ? s[3] : 0ull)));
-        if (cand != 0) {
-            const u32 c = slot_get_count(cand);
-            if (c >= (u32)kHashThreshold) return false;
-            payload = slot_get_payload(cand); cnt = c;
-            return true;
-        }
-        if (s[3] == 0) return true;                  // room left in this sector: the key is absent
-        sec = (sec + 1 == P.nsec) ? 0 : sec + 1;
-    }
+    const bool m0 = (s[0] >> 40) == tag && s[0] != 0, m1 = (s[1] >> 40) == tag && s[1] != 0;
+    const bool m2 = (s[2] >> 40) == tag && s[2] != 0, m3 = (s[3] >> 40) == tag && s[3] != 0;
+    const u64 cand = m0 ? s[0] : (m1 ? s[1] : (m2 ? s[2] : (m3 ? s[3] : 0ull)));
+    more = cand == 0 && s[3] != 0;
+    return cand;
 }
 
 // Position of the first base t in [0, ov) with S[s + t] != Y[t]; 0x7fffffff when there is none.
@@ -141,6 +130,8 @@ phase_a_fast_kernel(SearchParams P, u64 *__restrict__ extR, u64 *__restrict__ ex
     __shared__ u64 sQ[WARPS][32 * SWP];
     __shared__ u32 sEnt[WARPS][kFastCap];
     __shared__ uint8_t sWin[WARPS][kFastCap];
+    __shared__ u64 sH[WARPS][kFastWindows];
+    __shared__ u32 sC[WARPS][kFastWindows / 4];
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     u64 *SR = sS[warp][0], *SL = sS[warp][1], *Qs = sQ[warp];
     u32 *ents = sEnt[warp];
@@ -172,24 +163,68 @@ phase_a_fast_kernel(SearchParams P, u64 *__restrict__ extR, u64 *__restrict__ ex
         // unless they are the first of their bucket, which proves the bucket's key.
         int Tr = 0, Tl = 0;
         unsigned my_probes = 0;
-        for (int base = 0; base < W && !punt; base += 32) {
-            const int j = base + lane;
-            u64 payload = 0;
-            u32 cnt = 0;
-            if (j < W) {
+        u64 *H = sH[warp];                                          // window j: its key hash, then its bucket's payload
+        uint8_t *C = reinterpret_cast<uint8_t *>(sC[warp]);         // window j: its bucket size
+        if (!punt) {
+            for (int j = lane; j < W; j += 32) {
                 u64 v0, v1;
                 row_extract_key(SR, j, P.h, v0, v1);
-                if (!probe_sectors(P, hash_key(v0, v1), payload, cnt)) probe_window<SW>(P, v0, v1, false, payload, cnt);
+                H[j] = hash_key(v0, v1);
                 my_probes++;
             }
-            // The chunk's bucket sizes are scanned once; the warp then walks the chunk's entries 32 at a time, one per
-            // lane (a bucket's entries are contiguous, so the loads are near-coalesced).  A lane finds its window by a
-            // binary search over the scan, and the kept entries are compacted by ballot: both lists stay in window
-            // order, then bucket order.
-            u32 incl = cnt;
+            __syncwarp();
+            // The sector loads as one warp-wide queue: a lane holds one probe and takes the next window nobody has taken
+            // as soon as its probe ends.  Probes of full sectors walk on without holding up the other lanes' windows, so
+            // the warp spends one round per sector load of its busiest lane, not of every 32-window chunk's slowest.
+            int next = 0, qj = -1;                                  // next window not taken (warp-uniform); mine, -1: idle
+            u64 qh = 0, qbase = 0, qsec = 0;
+            for (;;) {
+                const unsigned idle = __ballot_sync(FULL, qj < 0);
+                if (qj < 0) {
+                    const int jn = next + __popc(idle & lt_mask);
+                    if (jn < W) {
+                        qj = jn; qh = H[jn];
+                        qbase = shard_base_sector(qh, P.nsec, P.shards); qsec = home_sector(qh, P.nsec);
+                    }
+                }
+                next += __popc(idle);
+                if (qj >= 0) {
+                    u64 s[4];
+                    ldg256_keep(P.slots + kSlotsPerSector * (qbase + qsec), s);
+                    bool more;
+                    const u64 cand = sector_match(s, slot_tag(qh), more);
+                    if (more) qsec = (qsec + 1 == P.nsec) ? 0 : qsec + 1;
+                    else {                  // a tag match counts as found (proven by the compare of the bucket's first entry)
+                        const u32 c = slot_get_count(cand);
+                        C[qj] = c >= (u32)kHashThreshold ? kFastMasked : (uint8_t)c;
+                        H[qj] = slot_get_payload(cand);
+                        qj = -1;
+                    }
+                }
+                if (next >= W && !__any_sync(FULL, qj >= 0)) break;
+            }
+            __syncwarp();
+            // a tag match on a masked key (>= 100 entries) is confirmed through its representative read
+            for (int j = lane; j < W; j += 32)
+                if (C[j] == kFastMasked) {
+                    u64 v0, v1, payload;
+                    u32 cnt;
+                    row_extract_key(SR, j, P.h, v0, v1);
+                    probe_window<SW>(P, v0, v1, false, payload, cnt);
+                    H[j] = payload; C[j] = (uint8_t)cnt;
+                }
+            __syncwarp();
+            // The bucket sizes are scanned once, four windows per lane; the warp then walks the entries of all windows 32
+            // at a time, one per lane (a bucket's entries are contiguous, so the loads are near-coalesced).  A lane finds
+            // its four windows by a binary search over the scan and its window among them from their sizes, and the kept
+            // entries are compacted by ballot: both lists stay in window order, then bucket order.
+            const int nw = min(max(W - 4 * lane, 0), 4);
+            const u32 cw = sC[warp][lane] & (nw == 4 ? ~0u : (1u << (8 * nw)) - 1u);
+            const u32 sum = __dp4a(cw, 0x01010101u, 0u);
+            u32 incl = sum;
 #pragma unroll
             for (int o = 1; o < 32; o <<= 1) { const u32 y = __shfl_up_sync(FULL, incl, o); if (lane >= o) incl += y; }
-            const u32 excl = incl - cnt;
+            const u32 excl = incl - sum;
             const u32 tot = __shfl_sync(FULL, incl, 31);
             for (u32 t0 = 0; t0 < tot; t0 += 32) {
                 const u32 t = t0 + lane;
@@ -199,12 +234,16 @@ phase_a_fast_kernel(SearchParams P, u64 *__restrict__ extR, u64 *__restrict__ ex
                     const u32 pm = __shfl_sync(FULL, incl, lo + step - 1);
                     if (pm <= t) lo += step;
                 }
-                const u32 e = t - __shfl_sync(FULL, excl, lo), c = __shfl_sync(FULL, cnt, lo);
-                const u64 pay = __shfl_sync(FULL, payload, lo);
-                const int jw = base + lo;
+                u32 e = t - __shfl_sync(FULL, excl, lo);
+                const u32 cl = __shfl_sync(FULL, cw, lo);
+                int sub = 0;
+#pragma unroll
+                for (int q = 0; q < 3; ++q) { const u32 c = (cl >> (8 * sub)) & 0xFF; if (e >= c) { e -= c; ++sub; } }
+                const u32 c = (cl >> (8 * sub)) & 0xFF;
+                const int jw = 4 * lo + sub;
                 const bool valid = t < tot;
                 u32 ent = 0;
-                if (valid) ent = c == 1 ? (u32)pay : __ldg(&P.entries[pay + e]);
+                if (valid) ent = c == 1 ? (u32)H[jw] : __ldg(&P.entries[H[jw] + e]);
                 const bool right = !(ent & 1u);
                 const bool keep = valid && (e == 0 || ((ent >> 2) != (u32)i && (right ? gate_right(jw, len1, P.k) : gate_left(jw, P.k, P.h))));
                 const unsigned kR = __ballot_sync(FULL, keep && right), kL = __ballot_sync(FULL, keep && !right);
