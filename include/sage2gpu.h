@@ -25,7 +25,8 @@ extern "C" {
 typedef struct sage2gpu_ctx sage2gpu_ctx;
 
 enum { SAGE2GPU_OK = 0, SAGE2GPU_ERR_CUDA = 1, SAGE2GPU_ERR_ARG = 2, SAGE2GPU_ERR_STATE = 3, SAGE2GPU_ERR_IO = 4,
-       SAGE2GPU_ERR_FORMAT = 5 /* sage2gpu_load_append_text: not the regular 4-line FASTQ / 2-line FASTA layout;
+       SAGE2GPU_ERR_FORMAT = 5 /* sage2gpu_load_append_text / _bgzf: not the regular 4-line FASTQ / 2-line FASTA layout;
+                                  sage2gpu_*bgzf: a BGZF member fails a check;
                                   sage2gpu_*saved_reads*: the file breaks the grammar of a saved .reads file */ };
 
 /* Log counters of the reference (readLoader.cpp:164-169,257; hashTable.cpp:86,124;
@@ -95,6 +96,24 @@ int sage2gpu_load_finish(sage2gpu_ctx *ctx);
  * parses that text sequentially and uses sage2gpu_load_append.  The buffer may be reused on return. */
 int sage2gpu_load_append_text(sage2gpu_ctx *ctx, const uint8_t *text, uint64_t n_bytes, int is_final, int *marker,
                               uint64_t max_records, uint64_t *consumed, uint64_t *n_records);
+/* The same for a piece of a BGZF-compressed file (htslib's bgzip: gzip members of at most 64 KiB of text, each with a `BC`
+ * extra subfield holding BSIZE), inflated on the device (replaces FastAQReader::getNextRead, fastAQReader.cpp:16-45, over
+ * kseq + gzread).  bgzf[0, n_bytes) holds whole members; their text follows prefix[0, prefix_bytes) (host text: what the
+ * previous piece did not consume, which may have gone to another context), and that text is split exactly as
+ * sage2gpu_load_append_text splits it, with the same is_final, *marker, max_records, *n_records and *consumed (bytes of that
+ * text, prefix included).  *rest_bytes = the text not consumed; its first min(*rest_bytes, rest_capacity) bytes are copied to
+ * `rest` -- the prefix of the next piece.  Every member's CRC32 and ISIZE are checked.  Returns SAGE2GPU_ERR_FORMAT with
+ * nothing appended when a member fails a check (*bad_member = its index in the piece, sage2gpu_last_error names it and the
+ * rule; the context stays usable) or when the text is irregular (*bad_member = -1: parse it sequentially, as with
+ * _append_text).  The buffers may be reused on return. */
+int sage2gpu_load_append_bgzf(sage2gpu_ctx *ctx, const uint8_t *prefix, uint64_t prefix_bytes, const uint8_t *bgzf, uint64_t n_bytes,
+                              int is_final, int *marker, uint64_t max_records, uint64_t *consumed, uint64_t *n_records, uint8_t *rest,
+                              uint64_t rest_capacity, uint64_t *rest_bytes, int64_t *bad_member);
+/* The BGZF members of bgzf[0, n_bytes) inflated on the device into text[0, *text_bytes) (host buffers; *text_bytes = the sum of
+ * their ISIZEs, set even when text_capacity is too small, which fails with SAGE2GPU_ERR_STATE).  Checks and *bad_member as
+ * above.  *kernel_ms (may be NULL) = the inflate kernel alone. */
+int sage2gpu_inflate_bgzf(sage2gpu_ctx *ctx, const uint8_t *bgzf, uint64_t n_bytes, uint8_t *text, uint64_t text_capacity, uint64_t *text_bytes,
+                          int64_t *bad_member, float *kernel_ms);
 /* Reads appended since sage2gpu_load_begin; removal of the appended reads [first, first + count) (the reference
  * stops a two-file data set when the shorter mate file ends, inputReader.cpp:26-49). */
 int sage2gpu_load_count(sage2gpu_ctx *ctx, uint64_t *n_reads);

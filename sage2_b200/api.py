@@ -19,9 +19,11 @@ LIB_PATH = os.path.join(HERE, "libsage2gpu.so")
 
 
 class Sage2GpuError(RuntimeError):
-    """`code` = the library's return code (include/sage2gpu.h: 5 = SAGE2GPU_ERR_FORMAT), `bad_line` = the line a format error names."""
+    """`code` = the library's return code (include/sage2gpu.h: 5 = SAGE2GPU_ERR_FORMAT), `bad_line` = the line a format error names,
+    `bad_member` = the index of the BGZF member that failed a check (-1: none)."""
     code = 0
     bad_line = 0
+    bad_member = -1
 
 
 ERR_FORMAT = 5
@@ -64,7 +66,7 @@ EXPORTS = ["sage2gpu_create", "sage2gpu_destroy", "sage2gpu_last_error", "sage2g
            "sage2gpu_synth_reads", "sage2gpu_build_hash_table_part", "sage2gpu_load_finish_packed", "sage2gpu_peer_copy",
            "sage2gpu_phase_a_import", "sage2gpu_load_max_length", "sage2gpu_load_finish_slice", "sage2gpu_table_bytes",
            "sage2gpu_load_saved_reads", "sage2gpu_saved_reads_info", "sage2gpu_saved_reads_slice", "sage2gpu_saved_reads_pack",
-           "sage2gpu_saved_reads_finish", "sage2gpu_table_view"]
+           "sage2gpu_saved_reads_finish", "sage2gpu_table_view", "sage2gpu_load_append_bgzf", "sage2gpu_inflate_bgzf"]
 
 _lib = None
 
@@ -95,6 +97,9 @@ def load_library():
         lib.sage2gpu_load_begin.argtypes = [vp, C.c_int]
         lib.sage2gpu_load_append.argtypes = [vp, vp, vp, i64]
         lib.sage2gpu_load_append_text.argtypes = [vp, vp, C.c_uint64, C.c_int, C.POINTER(C.c_int), C.c_uint64, u64p, u64p]
+        lib.sage2gpu_load_append_bgzf.argtypes = [vp, vp, C.c_uint64, vp, C.c_uint64, C.c_int, C.POINTER(C.c_int), C.c_uint64, u64p, u64p,
+                                                  vp, C.c_uint64, u64p, C.POINTER(i64)]
+        lib.sage2gpu_inflate_bgzf.argtypes = [vp, vp, C.c_uint64, vp, C.c_uint64, u64p, C.POINTER(i64), C.POINTER(C.c_float)]
         lib.sage2gpu_load_count.argtypes = [vp, u64p]
         lib.sage2gpu_load_remove.argtypes = [vp, C.c_uint64, C.c_uint64]
         lib.sage2gpu_load_finish.argtypes = [vp]
@@ -226,6 +231,47 @@ class Sage2Gpu:
 
     def load_begin(self, min_overlap: int):
         self._check(self._lib.sage2gpu_load_begin(self._h, int(min_overlap)), "load_begin")
+
+    def inflate_bgzf(self, data: bytes, text_capacity: int = -1):
+        """The BGZF members of `data` inflated on the device: (text bytes, kernel ms).  A member that fails a check raises
+        Sage2GpuError with code ERR_FORMAT and `bad_member` = its index."""
+        src = np.frombuffer(bytes(data), np.uint8)
+        n_out, bad, ms = C.c_uint64(), C.c_int64(-1), C.c_float()
+        if text_capacity < 0:       # sizing: ISIZE sums come from the headers, nothing is inflated for a 0-byte buffer
+            self._lib.sage2gpu_inflate_bgzf(self._h, src.ctypes.data, len(src), None, 0, C.byref(n_out), C.byref(bad), None)
+            text_capacity = n_out.value
+        out = np.empty(max(1, text_capacity), np.uint8)
+        rc = self._lib.sage2gpu_inflate_bgzf(self._h, src.ctypes.data, len(src), out.ctypes.data, text_capacity, C.byref(n_out),
+                                             C.byref(bad), C.byref(ms))
+        self._check_bgzf(rc, "inflate_bgzf", bad.value)
+        return out[:n_out.value].tobytes(), float(ms.value)
+
+    def load_append_bgzf(self, prefix: bytes, data: bytes, is_final: bool, marker: int = 0, max_records: int = (1 << 64) - 1,
+                         rest_capacity: int = 1 << 26):
+        """One piece of whole BGZF members after the host text `prefix` (sage2gpu_load_append_bgzf).  Returns a dict with
+        marker, consumed, n_records and rest (the text the next piece takes as its prefix)."""
+        pre = np.frombuffer(bytes(prefix) or b"\0", np.uint8)
+        src = np.frombuffer(bytes(data) or b"\0", np.uint8)
+        rest = np.empty(max(1, rest_capacity), np.uint8)
+        mk, used, nrec, nrest, bad = C.c_int(marker), C.c_uint64(), C.c_uint64(), C.c_uint64(), C.c_int64(-1)
+        rc = self._lib.sage2gpu_load_append_bgzf(self._h, pre.ctypes.data, len(prefix), src.ctypes.data, len(data), int(bool(is_final)),
+                                                 C.byref(mk), max_records, C.byref(used), C.byref(nrec), rest.ctypes.data, rest_capacity,
+                                                 C.byref(nrest), C.byref(bad))
+        self._check_bgzf(rc, "load_append_bgzf", bad.value)
+        return {"marker": mk.value, "consumed": used.value, "n_records": nrec.value,
+                "rest": rest[:min(nrest.value, rest_capacity)].tobytes()}
+
+    def _check_bgzf(self, rc: int, what: str, bad_member: int):
+        try:
+            self._check(rc, what)
+        except Sage2GpuError as e:
+            e.bad_member = int(bad_member)
+            raise
+
+    def load_count(self) -> int:
+        n = C.c_uint64()
+        self._check(self._lib.sage2gpu_load_count(self._h, C.byref(n)), "load_count")
+        return n.value
 
     def load_append(self, bases: np.ndarray, offsets: np.ndarray):
         """One chunk of a streamed upload: read r = bases[offsets[r], offsets[r+1]).  The buffers are kept alive until the

@@ -48,6 +48,9 @@ int guarded(sage2gpu_ctx *ctx, Fn fn)
     } catch (const sg::FormatError &e) {
         ctx->c.last_error = e.what();
         return SAGE2GPU_ERR_FORMAT;
+    } catch (const sg::BgzfError &e) {
+        ctx->c.last_error = e.what();
+        return SAGE2GPU_ERR_FORMAT;
     } catch (const sg::IoError &e) {
         ctx->c.last_error = e.what();
         return SAGE2GPU_ERR_IO;
@@ -430,6 +433,76 @@ int sage2gpu_load_append_text(sage2gpu_ctx *ctx, const uint8_t *text, uint64_t n
         *consumed = used; *n_records = nrec;
     });
     if (rc == 0 && !regular) { ctx->c.last_error = "text is not in the regular 4-line FASTQ / 2-line FASTA layout"; return SAGE2GPU_ERR_FORMAT; }
+    return rc;
+}
+
+int sage2gpu_load_append_bgzf(sage2gpu_ctx *ctx, const uint8_t *prefix, uint64_t prefix_bytes, const uint8_t *bgzf, uint64_t n_bytes, int is_final,
+                              int *marker, uint64_t max_records, uint64_t *consumed, uint64_t *n_records, uint8_t *rest, uint64_t rest_capacity,
+                              uint64_t *rest_bytes, int64_t *bad_member)
+{
+    bool regular = true;
+    if (bad_member) *bad_member = -1;
+    int rc = guarded(ctx, [&](sg::Context &c) {
+        SG_CHECK(c.up_open, "sage2gpu_load_begin must be called first");
+        SG_CHECK(marker && consumed && n_records && rest_bytes && (prefix_bytes == 0 || prefix) && (n_bytes == 0 || bgzf) &&
+                 (rest_capacity == 0 || rest), "null argument");
+        SG_CUDA(cudaEventSynchronize(c.up_event));
+        *consumed = *n_records = *rest_bytes = 0;
+        cudaStream_t st = c.stream;
+        sg::ArenaScope arena_scope(c.arena, st);
+        std::vector<sg::BgzfMember> mem;
+        sg::u64 text_bytes = 0;
+        try {
+            sg::bgzf_scan_members(bgzf, n_bytes, prefix_bytes, mem, text_bytes);
+            // the text of the piece: the prefix, then every member's text; one byte more for a final '\n'
+            sg::DevBuf<uint8_t> d_text(text_bytes + 1, st), d_in(n_bytes, st);
+            if (prefix_bytes) SG_CUDA(cudaMemcpyAsync(d_text.p, prefix, prefix_bytes, cudaMemcpyHostToDevice, st));
+            if (n_bytes) SG_CUDA(cudaMemcpyAsync(d_in.p, bgzf, n_bytes, cudaMemcpyHostToDevice, st));
+            sg::stage_inflate_members(c, d_in.p, mem.data(), mem.size(), d_text.p);
+            sg::u64 used = 0, nrec = 0;
+            regular = sg::stage_parse_device_text(c, d_text.p, text_bytes, is_final != 0, *marker, max_records, used, nrec);
+            if (!regular) return;
+            *consumed = used; *n_records = nrec;
+            *rest_bytes = text_bytes - used;
+            const sg::u64 back = std::min<sg::u64>(*rest_bytes, rest_capacity);
+            if (back) {
+                SG_CUDA(cudaMemcpyAsync(rest, d_text.p + used, back, cudaMemcpyDeviceToHost, st));
+                SG_CUDA(cudaStreamSynchronize(st));
+            }
+        } catch (const sg::BgzfError &e) {
+            if (bad_member) *bad_member = (int64_t)e.member;
+            throw;
+        }
+    });
+    if (rc == 0 && !regular) { ctx->c.last_error = "text is not in the regular 4-line FASTQ / 2-line FASTA layout"; return SAGE2GPU_ERR_FORMAT; }
+    return rc;
+}
+
+int sage2gpu_inflate_bgzf(sage2gpu_ctx *ctx, const uint8_t *bgzf, uint64_t n_bytes, uint8_t *text, uint64_t text_capacity, uint64_t *text_bytes,
+                          int64_t *bad_member, float *kernel_ms)
+{
+    if (bad_member) *bad_member = -1;
+    int rc = guarded(ctx, [&](sg::Context &c) {
+        SG_CHECK(text_bytes && (n_bytes == 0 || bgzf), "null argument");
+        cudaStream_t st = c.stream;
+        sg::ArenaScope arena_scope(c.arena, st);
+        std::vector<sg::BgzfMember> mem;
+        sg::u64 out = 0;
+        try {
+            sg::bgzf_scan_members(bgzf, n_bytes, 0, mem, out);
+            *text_bytes = out;
+            SG_CHECK(out <= text_capacity && (out == 0 || text), "the text buffer is smaller than the sum of the members' ISIZE");
+            sg::DevBuf<uint8_t> d_in(n_bytes, st), d_out(out, st);
+            if (n_bytes) SG_CUDA(cudaMemcpyAsync(d_in.p, bgzf, n_bytes, cudaMemcpyHostToDevice, st));
+            const float ms = sg::stage_inflate_members(c, d_in.p, mem.data(), mem.size(), d_out.p);
+            if (kernel_ms) *kernel_ms = ms;
+            if (out) SG_CUDA(cudaMemcpyAsync(text, d_out.p, out, cudaMemcpyDeviceToHost, st));
+            SG_CUDA(cudaStreamSynchronize(st));
+        } catch (const sg::BgzfError &e) {
+            if (bad_member) *bad_member = (int64_t)e.member;
+            throw;
+        }
+    });
     return rc;
 }
 

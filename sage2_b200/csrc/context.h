@@ -150,6 +150,27 @@ struct IoError : public std::runtime_error {
     explicit IoError(const std::string &m) : std::runtime_error(m) {}
 };
 
+// inflate.cu: one BGZF member of a batch, as the host reads it from the member's header and trailer
+struct BgzfMember {
+    u64 in_off;         // byte offset of the member in the batch's compressed bytes
+    u64 out_off;        // byte offset of its text in the output buffer (prefix sum of the ISIZEs)
+    u32 in_bytes;       // BSIZE + 1: the whole member, header and trailer included
+    u32 header_bytes;   // gzip header; the DEFLATE data is [header_bytes, in_bytes - 8)
+    u32 crc, out_bytes; // CRC32 and ISIZE of the trailer
+};
+enum BgzfCode : u32 { BGZF_HEADER = 1, BGZF_BSIZE, BGZF_ISIZE_LIMIT, BGZF_BLOCK_TYPE, BGZF_STORED_LEN, BGZF_BAD_CODE_LENGTHS, BGZF_BAD_CODE,
+                      BGZF_DISTANCE, BGZF_OUTPUT_OVERFLOW, BGZF_TRUNCATED, BGZF_TRAILING, BGZF_ISIZE, BGZF_CRC };
+const char *bgzf_error_text(u32 code);
+
+// A BGZF member that fails a check: its index in the batch, its byte offset there and the rule (BgzfCode)
+struct BgzfError : public std::runtime_error {
+    u64 member, offset;
+    u32 code;
+    BgzfError(u64 m, u64 off, u32 c)
+        : std::runtime_error("BGZF member " + std::to_string(m) + " (byte " + std::to_string(off) + " of the compressed data): " + bgzf_error_text(c)),
+          member(m), offset(off), code(c) {}
+};
+
 // stages (each throws sg::CudaError)
 void stage_ingest_ascii(Context &c, const uint8_t *bases, const int64_t *offsets, int64_t n_reads, bool device_resident, int forced_max_len = 0);
 void stage_raw_gather_layout(Context &c, int rank, int world, const u64 *counts, void **raw, u64 *first, u64 *total);
@@ -160,6 +181,13 @@ void stage_upload_chunk(Context &c, const uint8_t *bases, const int64_t *offsets
 int stage_uploaded_max_len(Context &c);     // longest read of the streamed upload so far
 // parse.cu: record splitting of raw FASTA/FASTQ text on the device; false = irregular layout, nothing appended
 bool stage_parse_text_chunk(Context &c, const uint8_t *text, u64 n_bytes, bool final, int &marker, u64 max_records, u64 &consumed, u64 &n_records);
+// the same on text already in device memory: d_text holds n_bytes of text and room for one more byte (a final '\n')
+bool stage_parse_device_text(Context &c, uint8_t *d_text, u64 n_bytes, bool final, int &marker, u64 max_records, u64 &consumed, u64 &n_records);
+// inflate.cu: the members of buf[0, n) (whole members) read from their headers, texts placed from out_base on; throws BgzfError
+void bgzf_scan_members(const uint8_t *buf, u64 n, u64 out_base, std::vector<BgzfMember> &members, u64 &out_end);
+// the members inflated from d_in into d_out on the device, CRC32 and ISIZE checked; returns the kernel's milliseconds, throws
+// BgzfError naming the first bad member
+float stage_inflate_members(Context &c, const uint8_t *d_in, const BgzfMember *h_members, u64 n_members, uint8_t *d_out);
 void stage_remove_uploaded(Context &c, u64 first, u64 count);
 // parse.cu: a saved .reads file (ReadLoader::loadReadsFromFile, readLoader.cpp:289).  Header: the declared number of reads and the
 // byte offset of the body.  Slice: the lines whose first byte lies in [begin, end) of the body, parsed and checked on the device into

@@ -85,25 +85,22 @@ static unsigned pgrid(u64 n, unsigned per_thread = 4)
     return g > kSMs * 16u ? kSMs * 16u : g;
 }
 
-bool stage_parse_text_chunk(Context &c, const uint8_t *text, u64 n_bytes, bool final, int &marker, u64 max_records, u64 &consumed, u64 &n_records)
+// The record splitter of both entries below: d_text[0, n_bytes) on the device, with room for one more byte; first / last = its
+// first and last byte (the host knows them without a copy when the text came from the host)
+static bool split_device_text(Context &c, uint8_t *d_text, u64 n_bytes, uint8_t first, uint8_t last, bool final, int &marker, u64 max_records,
+                              u64 &consumed, u64 &n_records)
 {
     cudaStream_t st = c.stream;
-    ArenaScope arena_scope(c.arena, st);
-    consumed = 0; n_records = 0;
-    if (n_bytes == 0 || max_records == 0) return true;
-    SG_CHECK(n_bytes < 0x7FFFFFF0ull, "text chunks must be smaller than 2 GiB");
     if (marker == 0) {
-        if (text[0] != '@' && text[0] != '>') return false;
-        marker = text[0];
+        if (first != '@' && first != '>') return false;
+        marker = first;
     }
     const int lpr = marker == '@' ? 4 : 2;
-    const bool add_nl = final && text[n_bytes - 1] != '\n';
+    const bool add_nl = final && last != '\n';
     const u64 n = n_bytes + (add_nl ? 1 : 0);
-    DevBuf<uint8_t> d_text(n, st);
-    SG_CUDA(cudaMemcpyAsync(d_text.p, text, n_bytes, cudaMemcpyHostToDevice, st));
-    if (add_nl) SG_CUDA(cudaMemsetAsync(d_text.p + n_bytes, '\n', 1, st));
+    if (add_nl) SG_CUDA(cudaMemsetAsync(d_text + n_bytes, '\n', 1, st));
     DevBuf<u32> flag(n, st), idx(n, st), d_lines(1, st);
-    nl_flag_kernel<<<pgrid(n), 256, 0, st>>>(d_text.p, n, flag.p);
+    nl_flag_kernel<<<pgrid(n), 256, 0, st>>>(d_text, n, flag.p);
     SG_LAUNCHED();
     exclusive_scan_u32(flag.p, idx.p, n, d_lines.p, st);
     u32 L = 0;
@@ -113,11 +110,11 @@ bool stage_parse_text_chunk(Context &c, const uint8_t *text, u64 n_bytes, bool f
     if (R > max_records) R = max_records;
     if (R == 0) return !final;                       // no complete record in this chunk (a final stub is irregular)
     DevBuf<u32> ls((size_t)L + 1, st);
-    line_start_kernel<<<pgrid(n), 256, 0, st>>>(d_text.p, n, idx.p, ls.p);
+    line_start_kernel<<<pgrid(n), 256, 0, st>>>(d_text, n, idx.p, ls.p);
     SG_LAUNCHED();
     DevBuf<u32> seq_len(R, st), seq_off(R, st), d_out(3, st);
     SG_CUDA(cudaMemsetAsync(d_out.p, 0, 3 * sizeof(u32), st));
-    record_check_kernel<<<pgrid(R, 1), 256, 0, st>>>(d_text.p, ls.p, R, lpr, marker, seq_len.p, d_out.p);
+    record_check_kernel<<<pgrid(R, 1), 256, 0, st>>>(d_text, ls.p, R, lpr, marker, seq_len.p, d_out.p);
     SG_LAUNCHED();
     exclusive_scan_u32(seq_len.p, seq_off.p, R, d_out.p + 2, st);
     u32 h_out[3];
@@ -131,7 +128,7 @@ bool stage_parse_text_chunk(Context &c, const uint8_t *text, u64 n_bytes, bool f
     grow_persistent(c.up_d_offsets, (size_t)(c.up_reads ? c.up_reads + 1 : 0), (size_t)(c.up_reads + R + 1), st);
     unsigned g = grid_for(R, 8, 1);
     if (g > kSMs * 16u) g = kSMs * 16u;
-    record_copy_kernel<<<g, 256, 0, st>>>(d_text.p, ls.p, seq_len.p, seq_off.p, R, lpr, c.up_bases, c.up_d_bases.p, c.up_d_offsets.p + c.up_reads);
+    record_copy_kernel<<<g, 256, 0, st>>>(d_text, ls.p, seq_len.p, seq_off.p, R, lpr, c.up_bases, c.up_d_bases.p, c.up_d_offsets.p + c.up_reads);
     SG_LAUNCHED();
     SG_CUDA(cudaStreamSynchronize(st));              // the caller may overwrite `text` now
     c.up_reads += R;
@@ -139,6 +136,32 @@ bool stage_parse_text_chunk(Context &c, const uint8_t *text, u64 n_bytes, bool f
     consumed = used > n_bytes ? n_bytes : used;
     n_records = R;
     return true;
+}
+
+bool stage_parse_text_chunk(Context &c, const uint8_t *text, u64 n_bytes, bool final, int &marker, u64 max_records, u64 &consumed, u64 &n_records)
+{
+    cudaStream_t st = c.stream;
+    ArenaScope arena_scope(c.arena, st);
+    consumed = 0; n_records = 0;
+    if (n_bytes == 0 || max_records == 0) return true;
+    SG_CHECK(n_bytes < 0x7FFFFFF0ull, "text chunks must be smaller than 2 GiB");
+    DevBuf<uint8_t> d_text(n_bytes + 1, st);
+    SG_CUDA(cudaMemcpyAsync(d_text.p, text, n_bytes, cudaMemcpyHostToDevice, st));
+    return split_device_text(c, d_text.p, n_bytes, text[0], text[n_bytes - 1], final, marker, max_records, consumed, n_records);
+}
+
+bool stage_parse_device_text(Context &c, uint8_t *d_text, u64 n_bytes, bool final, int &marker, u64 max_records, u64 &consumed, u64 &n_records)
+{
+    cudaStream_t st = c.stream;
+    ArenaScope arena_scope(c.arena, st);
+    consumed = 0; n_records = 0;
+    if (n_bytes == 0 || max_records == 0) return true;
+    SG_CHECK(n_bytes < 0x7FFFFFF0ull, "text chunks must be smaller than 2 GiB");
+    uint8_t ends[2];
+    SG_CUDA(cudaMemcpyAsync(&ends[0], d_text, 1, cudaMemcpyDeviceToHost, st));
+    SG_CUDA(cudaMemcpyAsync(&ends[1], d_text + n_bytes - 1, 1, cudaMemcpyDeviceToHost, st));
+    SG_CUDA(cudaStreamSynchronize(st));
+    return split_device_text(c, d_text, n_bytes, ends[0], ends[1], final, marker, max_records, consumed, n_records);
 }
 
 // drop the uploaded reads [first, first + count)

@@ -14,6 +14,11 @@
 // beside the later stages on every GPU, otherwise sharded by key hash with the window probes routed through peer-memory
 // mailboxes (low-memory mode); SAGE2GPU_TABLE_LAYOUT=replicated|sharded forces the choice, the log states it.
 //
+// Input: plain FASTA / FASTQ text goes to the GPU in pieces and its records are split there.  BGZF files (htslib's bgzip: gzip
+// members with a BC field) are inflated on the GPU as well, piece by piece of whole members; other gzip files are inflated by
+// host zlib.  A BGZF member that fails a check (CRC32, ISIZE, DEFLATE rules) stops the program with a FORMAT error naming its
+// compressed offset.
+//
 // Restarts: -m 2 and -m 3 load <outputDir><inputPrefix>.reads (ReadLoader::loadReadsFromFile, readLoader.cpp:289) -- parsed
 // and checked on the device, spread over the contexts with --devices -- and do not open the -f / -l inputs in steps 1-3 (the
 // flags stay required, as in the reference's checkRequired).  When that file does not exist, step 1 runs from the input files.
@@ -86,7 +91,7 @@ void printUsage()
 void printListOfArgs()
 {
     std::cout << "OPTIONS (those of SAGE2):\n"
-                 "\t-f|--fileInput <file>   interleaved FASTA/FASTQ file (plain or gzip)\n"
+                 "\t-f|--fileInput <file>   interleaved FASTA/FASTQ file (plain or gzip; BGZF is inflated on the GPU)\n"
                  "\t-l|--listInput <file>   list of input files (f1=/f2= pairs or f= interleaved)\n"
                  "\t-k|--minOverlap <int>   minimum overlap length\n"
                  "\t-o|--outputDir <dir>    output directory\n"
@@ -280,6 +285,17 @@ public:
         if (rc == 0 && nrec) appended(r, nrec);
         return rc;
     }
+    // inflate + record splitting of one piece of BGZF members on context next(); see sage2gpu_load_append_bgzf
+    int appendBgzf(const uint8_t *prefix, size_t np, const uint8_t *bgzf, size_t n, bool final, int *marker, uint64_t max_records,
+                   uint64_t &consumed, uint64_t &nrec, uint8_t *rest, size_t rest_cap, uint64_t &rest_bytes, int64_t &bad_member)
+    {
+        const int r = next_;
+        const int rc = sage2gpu_load_append_bgzf(ctx_[r], prefix, np, bgzf, n, final ? 1 : 0, marker, max_records, &consumed, &nrec, rest,
+                                                 rest_cap, &rest_bytes, &bad_member);
+        touch(r);
+        if (rc == 0 && nrec) appended(r, nrec);
+        return rc;
+    }
     // pinned buffer for raw file text (device-side record splitting)
     uint8_t *text(size_t &cap)
     {
@@ -389,11 +405,128 @@ uint64_t parseSequential(Uploader &up, sg_host::FastAQStream &in, uint64_t max_r
     return n;
 }
 
+uint32_t le32(const uint8_t *p) { return (uint32_t)p[0] | (uint32_t)p[1] << 8 | (uint32_t)p[2] << 16 | (uint32_t)p[3] << 24; }
+
+// The gzip member header at p[0, n): its size (BSIZE + 1) when it is a BGZF member (gzip magic, FEXTRA, a `BC` subfield with
+// SLEN 2); 0 when it is not; -1 when n is too short to tell
+long bgzfMemberBytes(const uint8_t *p, size_t n)
+{
+    if (n < 12) return -1;
+    if (p[0] != 0x1f || p[1] != 0x8b || p[2] != 8 || !(p[3] & 4)) return 0;
+    const size_t xlen = (size_t)p[10] | (size_t)p[11] << 8;
+    if (n < 12 + xlen) return -1;
+    for (size_t i = 12; i + 4 <= 12 + xlen;) {
+        const size_t slen = (size_t)p[i + 2] | (size_t)p[i + 3] << 8;
+        if (i + 4 + slen > 12 + xlen) break;
+        if (p[i] == 'B' && p[i + 1] == 'C' && slen == 2) return 1 + (long)((size_t)p[i + 4] | (size_t)p[i + 5] << 8);
+        i += 4 + slen;
+    }
+    return 0;
+}
+
+// the sequential parser from compressed offset `off` of the file on (a member boundary, so zlib starts a fresh stream) after the
+// host text pending[0, n)
+uint64_t parseRestSequential(Uploader &up, int fd, off_t off, const uint8_t *pending, size_t n, uint64_t max_records, const std::string &path)
+{
+    if (lseek(fd, off, SEEK_SET) != off) { close(fd); throw std::runtime_error("cannot read " + path); }
+    gzFile gz = gzdopen(fd, "r");
+    if (!gz) { close(fd); throw std::runtime_error("cannot read " + path); }
+    gzbuffer(gz, 1 << 20);
+    sg_host::FastAQStream in(gz, pending, n);           // takes the handle
+    const uint64_t got = parseSequential(up, in, max_records);
+    up.sync();
+    return got;
+}
+
+// A BGZF file: the compressed bytes are read with read(2) into pinned memory, cut into pieces of whole members whose texts
+// add up to at most pieceBytes() (at least one member), and every piece is inflated and split on the device.  The text a
+// piece leaves over (at most one record) comes back to the host and goes in front of the next piece, which may go to
+// another context.  Irregular text, and members without a `BC` field, continue on the sequential parser.
+uint64_t readBgzf(Uploader &up, int fd, const std::string &path, uint64_t max_records, bool &used_device_parser)
+{
+    const size_t piece = pieceBytes(), ccap = piece + ((size_t)1 << 20), rcap = 2 * piece + ((size_t)1 << 17);
+    uint8_t *cbuf = (uint8_t *)sage2gpu_host_alloc(ccap), *pre = (uint8_t *)sage2gpu_host_alloc(rcap),
+            *rest = (uint8_t *)sage2gpu_host_alloc(rcap);
+    if (!cbuf || !pre || !rest) printError("MEM_ALLOC", "pinned BGZF buffers");
+    struct Free { uint8_t *a, *b, *c; ~Free() { sage2gpu_host_free(a); sage2gpu_host_free(b); sage2gpu_host_free(c); } } release{ cbuf, pre, rest };
+    size_t have = 0, np = 0;               // compressed bytes in cbuf (from file offset base on); host text in front of the next piece
+    off_t base = 0;
+    bool eof = false;
+    int marker = 0;
+    uint64_t total = 0;
+    auto fill = [&] {
+        while (have < ccap && !eof) {
+            const ssize_t n = read(fd, cbuf + have, ccap - have);
+            if (n < 0) { close(fd); throw std::runtime_error("cannot read " + path); }
+            if (n == 0) eof = true; else have += (size_t)n;
+        }
+    };
+    auto fallback = [&](off_t off, const char *why) {
+        logStream << "\tBGZF file " << path << ": " << why << " at compressed offset " << off
+                  << "; the rest of the file continues on the sequential parser (host zlib).\n";
+        return total + parseRestSequential(up, fd, off, pre, np, max_records - total, path);
+    };
+    up.sync();
+    for (;;) {
+        fill();
+        // whole members from the front of cbuf
+        size_t end = 0;
+        uint64_t text = 0;
+        bool plain = false;                // the next member has no BC field
+        for (;;) {
+            if (end == have) break;
+            const long mb = bgzfMemberBytes(cbuf + end, have - end);
+            if (mb == 0) { plain = true; break; }
+            if (mb < 0 || end + (size_t)mb > have) {
+                if (end > 0 || !eof) break;     // the rest of the member comes with the next fill
+                printError("FORMAT", path + ": BGZF member at compressed offset " + std::to_string(base + (off_t)end) +
+                                         (mb < 0 ? ": truncated header" : ": BSIZE reaches past the end of the file"));
+            }
+            if ((size_t)mb < 26) printError("FORMAT", path + ": BGZF member at compressed offset " + std::to_string(base + (off_t)end) + ": BSIZE too small");
+            const uint32_t isize = le32(cbuf + end + mb - 4);
+            if (end > 0 && text + isize > piece) break;
+            end += (size_t)mb;
+            text += isize;
+        }
+        if (end == 0 && plain) return fallback(base, "a gzip member without a BC field");
+        const bool final = end == have && eof;
+        uint64_t consumed = 0, nrec = 0, nrest = 0;
+        int64_t bad = -1;
+        const int r = up.next();
+        const int rc = up.appendBgzf(pre, np, cbuf, end, final, &marker, max_records - total, consumed, nrec, rest, rcap, nrest, bad);
+        if (rc == SAGE2GPU_ERR_FORMAT && bad >= 0) {
+            // the member's offset: walk the piece's members once more
+            size_t off = 0;
+            for (int64_t i = 0; i < bad; ++i) off += (size_t)bgzfMemberBytes(cbuf + off, end - off);
+            std::string e = sage2gpu_last_error(up.ctx(r));
+            const size_t colon = e.find("): ");
+            printError("FORMAT", path + ": BGZF member at compressed offset " + std::to_string(base + (off_t)off) + ": " +
+                                     (colon == std::string::npos ? e : e.substr(colon + 3)));
+        }
+        if (rc == SAGE2GPU_ERR_FORMAT) return fallback(base, "text not in the regular 4-line FASTQ / 2-line FASTA layout");
+        if (rc != 0) up.fail(r);
+        used_device_parser = true;
+        total += nrec;
+        if (nrest > rcap) printError("MEM_ALLOC", "a record longer than the BGZF rest buffer");
+        std::swap(pre, rest);
+        np = (size_t)nrest;
+        memmove(cbuf, cbuf + end, have - end);
+        have -= end;
+        base += (off_t)end;
+        if (total >= max_records || final) break;
+        if (consumed == 0) return fallback(base, "a record longer than a piece");
+    }
+    up.sync();
+    close(fd);
+    return total;
+}
+
 // One file: raw text goes to the device in 32 MB pieces and the records are split there
 // (sage2gpu_load_append_text); text that is not in the regular layout is parsed sequentially from that point on.
-uint64_t readFile(Uploader &up, const std::string &path, uint64_t max_records, bool &used_device_parser)
+// BGZF files are inflated on the device too (readBgzf).
+uint64_t readFile(Uploader &up, const std::string &path, uint64_t max_records, bool &used_device_parser, bool &inflated_on_device)
 {
-    used_device_parser = false;
+    used_device_parser = inflated_on_device = false;
     if (!up.active()) {                    // --parse-only
         sg_host::FastAQStream in(path);
         return parseSequential(up, in, max_records);
@@ -401,8 +534,14 @@ uint64_t readFile(Uploader &up, const std::string &path, uint64_t max_records, b
     // plain files are read with read(2) straight into the pinned buffer; gzip goes through zlib
     const int fd = open(path.c_str(), O_RDONLY);
     if (fd < 0) throw std::runtime_error("cannot open " + path);
-    unsigned char magic[2] = { 0, 0 };
-    const bool is_gz = pread(fd, magic, 2, 0) == 2 && magic[0] == 0x1f && magic[1] == 0x8b;
+    unsigned char magic[1024] = { 0 };
+    const ssize_t nm = pread(fd, magic, sizeof(magic), 0);
+    const bool is_gz = nm >= 2 && magic[0] == 0x1f && magic[1] == 0x8b;
+    if (is_gz && nm > 0 && bgzfMemberBytes(magic, (size_t)nm) > 0) {
+        const uint64_t n = readBgzf(up, fd, path, max_records, used_device_parser);
+        inflated_on_device = used_device_parser;
+        return n;
+    }
     gzFile gz = nullptr;
     if (is_gz) {
         gz = gzdopen(fd, "r");
@@ -450,9 +589,9 @@ uint64_t readDataset(Uploader &up, const std::string &f1, const std::string &f2)
     logStream.flush();
     uint64_t n = 0;
     try {
-        bool dev1 = false, dev2 = false;
+        bool dev1 = false, dev2 = false, inf1 = false, inf2 = false;
         if (f2.empty()) {
-            n = readFile(up, f1, UINT64_MAX, dev1);
+            n = readFile(up, f1, UINT64_MAX, dev1, inf1);
             up.takeSegments();
         } else if (!up.active()) {
             sg_host::MatePairStream in(f1, f2);     // --parse-only keeps the reference's alternating order
@@ -464,9 +603,9 @@ uint64_t readDataset(Uploader &up, const std::string &f1, const std::string &f2)
             // records it keeps min(n1, n2 + 1) of file 1 and min(n2, n1) of file 2.  Read ids are ranks in the sorted set,
             // so the upload order is free: file 1, then file 2 capped at n1, then the surplus of file 1 (its last records, in
             // whichever contexts they went to) is dropped.
-            const uint64_t n1 = readFile(up, f1, UINT64_MAX, dev1);
+            const uint64_t n1 = readFile(up, f1, UINT64_MAX, dev1, inf1);
             const std::vector<Segment> file1 = up.takeSegments();
-            const uint64_t n2 = readFile(up, f2, n1, dev2);
+            const uint64_t n2 = readFile(up, f2, n1, dev2, inf2);
             up.takeSegments();
             uint64_t keep1 = n1;
             if (n1 > n2 + 1) {
@@ -475,7 +614,8 @@ uint64_t readDataset(Uploader &up, const std::string &f1, const std::string &f2)
             }
             n = keep1 + n2;
         }
-        logStream << "\tRecords split on the device: " << ((dev1 || dev2) ? "yes" : "no (sequential parser)") << "\n";
+        logStream << "\tRecords split on the device: " << ((dev1 || dev2) ? "yes" : "no (sequential parser)")
+                  << ((inf1 || inf2) ? "; BGZF text inflated on the device" : "") << "\n";
     } catch (const std::runtime_error &e) {
         printError("OPEN_FILE", e.what());
     }
