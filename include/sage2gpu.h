@@ -27,6 +27,7 @@ typedef struct sage2gpu_ctx sage2gpu_ctx;
 enum { SAGE2GPU_OK = 0, SAGE2GPU_ERR_CUDA = 1, SAGE2GPU_ERR_ARG = 2, SAGE2GPU_ERR_STATE = 3, SAGE2GPU_ERR_IO = 4,
        SAGE2GPU_ERR_FORMAT = 5 /* sage2gpu_load_append_text / _bgzf: not the regular 4-line FASTQ / 2-line FASTA layout;
                                   sage2gpu_*bgzf: a BGZF member fails a check;
+                                  sage2gpu_*gzip: gzip data fails a check of zlib's inflate / gzread;
                                   sage2gpu_*saved_reads*: the file breaks the grammar of a saved .reads file */ };
 
 /* Log counters of the reference (readLoader.cpp:164-169,257; hashTable.cpp:86,124;
@@ -114,6 +115,43 @@ int sage2gpu_load_append_bgzf(sage2gpu_ctx *ctx, const uint8_t *prefix, uint64_t
  * above.  *kernel_ms (may be NULL) = the inflate kernel alone. */
 int sage2gpu_inflate_bgzf(sage2gpu_ctx *ctx, const uint8_t *bgzf, uint64_t n_bytes, uint8_t *text, uint64_t text_capacity, uint64_t *text_bytes,
                           int64_t *bad_member, float *kernel_ms);
+/* Where a piece of an ordinary gzip stream (single-member, or members concatenated, as gzip / pigz write them) continues.  All
+ * zeros before the first piece.  A piece hands this to the next one, whichever context decodes it. */
+typedef struct {
+    uint64_t offset;          /* compressed byte offset (in the file) of the byte the next piece starts with */
+    uint64_t member_offset;   /* compressed offset of the current member's header */
+    uint64_t member_bytes;    /* text of the current member so far (its ISIZE is this mod 2^32) */
+    uint32_t bit;             /* the next DEFLATE block starts at this bit (0-7) of that byte */
+    uint32_t in_member;       /* 1: the next piece starts at a block of the current member; 0: at a member header or the end */
+    uint32_t crc;             /* CRC32 of the current member's text so far */
+    uint32_t window_bytes;    /* bytes of the current member's text at the end of window[] (at most 32768) */
+    uint32_t done;            /* the stream has ended: a trailer followed by the end of the file or by bytes that are not a gzip
+                                 header (zlib ignores them) */
+    uint32_t reserved;
+    uint8_t window[32768];    /* the current member's last text, ending at window[32767] */
+} sage2gpu_gzip_state;
+/* The same as sage2gpu_load_append_bgzf for a piece of an ordinary gzip file, inflated on the device (replaces
+ * FastAQReader::getNextRead, fastAQReader.cpp:16-45, over kseq + gzread, whose text this equals byte for byte).  gz[0, n_bytes)
+ * are the compressed bytes from state->offset on; is_final says that they reach the end of the file.  The piece is cut at
+ * DEFLATE block starts found on the device, its ranges inflated at once and stitched; at most max(text_bound, one range of
+ * blocks) bytes of text are inflated, after the host prefix, and split as _load_append_text splits them (prefix, is_final of
+ * the splitter = the stream ended in this piece, *marker, max_records, *consumed, *n_records, rest as for _bgzf).  *state moves
+ * to where the next piece starts and *in_consumed = the compressed bytes it moved past: 0 when the piece holds no complete
+ * block (pass more bytes).  Every member's CRC32 and ISIZE are checked.  Returns SAGE2GPU_ERR_FORMAT with nothing appended and
+ * *state unchanged when the data fails a check (*bad_offset = the compressed offset of the member -- header, CRC, ISIZE,
+ * truncated trailer -- or of the block that broke a DEFLATE rule; sage2gpu_last_error names it and the rule; the context
+ * stays usable) or when the text is irregular (*bad_offset = -1: parse it sequentially).  The buffers may be reused on return. */
+int sage2gpu_load_append_gzip(sage2gpu_ctx *ctx, const uint8_t *prefix, uint64_t prefix_bytes, const uint8_t *gz, uint64_t n_bytes,
+                              int is_final, uint64_t text_bound, sage2gpu_gzip_state *state, int *marker, uint64_t max_records,
+                              uint64_t *consumed, uint64_t *n_records, uint8_t *rest, uint64_t rest_capacity, uint64_t *rest_bytes,
+                              uint64_t *in_consumed, int64_t *bad_offset);
+/* A whole gzip stream gz[0, n_bytes) inflated on the device into text[0, *text_bytes) (host buffers; fails with
+ * SAGE2GPU_ERR_STATE when the text is larger than text_capacity, *text_bytes then being the text inflated so far).  Checks and
+ * *bad_offset as above.  *kernel_ms = the device kernels alone, *ranges = ranges decoded (all passes, false candidates
+ * included), *confirmed = ranges whose text was kept (the confirmed chains of all pieces), *rejected = block-start candidates
+ * found false; each may be NULL. */
+int sage2gpu_inflate_gzip(sage2gpu_ctx *ctx, const uint8_t *gz, uint64_t n_bytes, uint8_t *text, uint64_t text_capacity, uint64_t *text_bytes,
+                          int64_t *bad_offset, float *kernel_ms, uint64_t *ranges, uint64_t *confirmed, uint64_t *rejected);
 /* Reads appended since sage2gpu_load_begin; removal of the appended reads [first, first + count) (the reference
  * stops a two-file data set when the shorter mate file ends, inputReader.cpp:26-49). */
 int sage2gpu_load_count(sage2gpu_ctx *ctx, uint64_t *n_reads);

@@ -20,13 +20,23 @@ LIB_PATH = os.path.join(HERE, "libsage2gpu.so")
 
 class Sage2GpuError(RuntimeError):
     """`code` = the library's return code (include/sage2gpu.h: 5 = SAGE2GPU_ERR_FORMAT), `bad_line` = the line a format error names,
-    `bad_member` = the index of the BGZF member that failed a check (-1: none)."""
+    `bad_member` = the index of the BGZF member that failed a check (-1: none), `bad_offset` = the compressed offset of the gzip
+    member or block that failed a check (-1: none)."""
     code = 0
     bad_line = 0
     bad_member = -1
+    bad_offset = -1
 
 
 ERR_FORMAT = 5
+ERR_STATE = 3
+
+
+class GzipState(C.Structure):
+    """sage2gpu_gzip_state: where a piece of a gzip stream continues (all zeros before the first piece)."""
+    _fields_ = [("offset", C.c_uint64), ("member_offset", C.c_uint64), ("member_bytes", C.c_uint64), ("bit", C.c_uint32),
+                ("in_member", C.c_uint32), ("crc", C.c_uint32), ("window_bytes", C.c_uint32), ("done", C.c_uint32),
+                ("reserved", C.c_uint32), ("window", C.c_uint8 * 32768)]
 
 
 class Counters(C.Structure):
@@ -66,7 +76,8 @@ EXPORTS = ["sage2gpu_create", "sage2gpu_destroy", "sage2gpu_last_error", "sage2g
            "sage2gpu_synth_reads", "sage2gpu_build_hash_table_part", "sage2gpu_load_finish_packed", "sage2gpu_peer_copy",
            "sage2gpu_phase_a_import", "sage2gpu_load_max_length", "sage2gpu_load_finish_slice", "sage2gpu_table_bytes",
            "sage2gpu_load_saved_reads", "sage2gpu_saved_reads_info", "sage2gpu_saved_reads_slice", "sage2gpu_saved_reads_pack",
-           "sage2gpu_saved_reads_finish", "sage2gpu_table_view", "sage2gpu_load_append_bgzf", "sage2gpu_inflate_bgzf"]
+           "sage2gpu_saved_reads_finish", "sage2gpu_table_view", "sage2gpu_load_append_bgzf", "sage2gpu_inflate_bgzf",
+           "sage2gpu_load_append_gzip", "sage2gpu_inflate_gzip"]
 
 _lib = None
 
@@ -100,6 +111,10 @@ def load_library():
         lib.sage2gpu_load_append_bgzf.argtypes = [vp, vp, C.c_uint64, vp, C.c_uint64, C.c_int, C.POINTER(C.c_int), C.c_uint64, u64p, u64p,
                                                   vp, C.c_uint64, u64p, C.POINTER(i64)]
         lib.sage2gpu_inflate_bgzf.argtypes = [vp, vp, C.c_uint64, vp, C.c_uint64, u64p, C.POINTER(i64), C.POINTER(C.c_float)]
+        lib.sage2gpu_load_append_gzip.argtypes = [vp, vp, C.c_uint64, vp, C.c_uint64, C.c_int, C.c_uint64, C.POINTER(GzipState),
+                                                  C.POINTER(C.c_int), C.c_uint64, u64p, u64p, vp, C.c_uint64, u64p, u64p, C.POINTER(i64)]
+        lib.sage2gpu_inflate_gzip.argtypes = [vp, vp, C.c_uint64, vp, C.c_uint64, u64p, C.POINTER(i64), C.POINTER(C.c_float), u64p, u64p,
+                                              u64p]
         lib.sage2gpu_load_count.argtypes = [vp, u64p]
         lib.sage2gpu_load_remove.argtypes = [vp, C.c_uint64, C.c_uint64]
         lib.sage2gpu_load_finish.argtypes = [vp]
@@ -260,6 +275,46 @@ class Sage2Gpu:
         self._check_bgzf(rc, "load_append_bgzf", bad.value)
         return {"marker": mk.value, "consumed": used.value, "n_records": nrec.value,
                 "rest": rest[:min(nrest.value, rest_capacity)].tobytes()}
+
+    def inflate_gzip(self, data: bytes, text_capacity: int = -1):
+        """A whole gzip stream inflated on the device (sage2gpu_inflate_gzip): (text bytes, kernel ms, ranges decoded, ranges
+        confirmed, candidates rejected).  Data that fails a check raises Sage2GpuError with code ERR_FORMAT and `bad_offset` =
+        the compressed offset of the member or block."""
+        src = np.frombuffer(bytes(data) or b"\0", np.uint8)
+        cap = text_capacity if text_capacity >= 0 else 4 * len(data) + (1 << 20)
+        while True:
+            out = np.empty(max(1, cap), np.uint8)
+            n_out, bad, ms, nr, conf, rej = C.c_uint64(), C.c_int64(-1), C.c_float(), C.c_uint64(), C.c_uint64(), C.c_uint64()
+            rc = self._lib.sage2gpu_inflate_gzip(self._h, src.ctypes.data, len(data), out.ctypes.data, cap, C.byref(n_out), C.byref(bad),
+                                                 C.byref(ms), C.byref(nr), C.byref(conf), C.byref(rej))
+            if rc == ERR_STATE and text_capacity < 0 and b"smaller than the text" in (self._lib.sage2gpu_last_error(self._h) or b""):
+                cap *= 4
+                continue
+            self._check_gzip(rc, "inflate_gzip", bad.value)
+            return out[:n_out.value].tobytes(), float(ms.value), nr.value, conf.value, rej.value
+
+    def load_append_gzip(self, prefix: bytes, data: bytes, is_final: bool, state: "GzipState", text_bound: int, marker: int = 0,
+                         max_records: int = (1 << 64) - 1, rest_capacity: int = 1 << 26):
+        """One piece of a gzip stream after the host text `prefix` (sage2gpu_load_append_gzip): `data` = the compressed bytes from
+        state.offset on, `state` moves to where the next piece starts.  Returns a dict with marker, consumed, n_records, rest and
+        in_consumed (compressed bytes the state moved past)."""
+        pre = np.frombuffer(bytes(prefix) or b"\0", np.uint8)
+        src = np.frombuffer(bytes(data) or b"\0", np.uint8)
+        rest = np.empty(max(1, rest_capacity), np.uint8)
+        mk, used, nrec, nrest, nin, bad = C.c_int(marker), C.c_uint64(), C.c_uint64(), C.c_uint64(), C.c_uint64(), C.c_int64(-1)
+        rc = self._lib.sage2gpu_load_append_gzip(self._h, pre.ctypes.data, len(prefix), src.ctypes.data, len(data), int(bool(is_final)),
+                                                 text_bound, C.byref(state), C.byref(mk), max_records, C.byref(used), C.byref(nrec),
+                                                 rest.ctypes.data, rest_capacity, C.byref(nrest), C.byref(nin), C.byref(bad))
+        self._check_gzip(rc, "load_append_gzip", bad.value)
+        return {"marker": mk.value, "consumed": used.value, "n_records": nrec.value,
+                "rest": rest[:min(nrest.value, rest_capacity)].tobytes(), "in_consumed": nin.value}
+
+    def _check_gzip(self, rc: int, what: str, bad_offset: int):
+        try:
+            self._check(rc, what)
+        except Sage2GpuError as e:
+            e.bad_offset = int(bad_offset)
+            raise
 
     def _check_bgzf(self, rc: int, what: str, bad_member: int):
         try:

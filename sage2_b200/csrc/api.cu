@@ -3,6 +3,8 @@
 #include <stdio.h>
 #include <stdlib.h>
 #include <string.h>
+#include <memory>
+#include <stdexcept>
 #include <vector>
 #include "../../include/sage2gpu.h"
 #include "context.h"
@@ -49,6 +51,9 @@ int guarded(sage2gpu_ctx *ctx, Fn fn)
         ctx->c.last_error = e.what();
         return SAGE2GPU_ERR_FORMAT;
     } catch (const sg::BgzfError &e) {
+        ctx->c.last_error = e.what();
+        return SAGE2GPU_ERR_FORMAT;
+    } catch (const sg::GzipError &e) {
         ctx->c.last_error = e.what();
         return SAGE2GPU_ERR_FORMAT;
     } catch (const sg::IoError &e) {
@@ -504,6 +509,87 @@ int sage2gpu_inflate_bgzf(sage2gpu_ctx *ctx, const uint8_t *bgzf, uint64_t n_byt
         }
     });
     return rc;
+}
+
+int sage2gpu_load_append_gzip(sage2gpu_ctx *ctx, const uint8_t *prefix, uint64_t prefix_bytes, const uint8_t *gz, uint64_t n_bytes,
+                              int is_final, uint64_t text_bound, sage2gpu_gzip_state *state, int *marker, uint64_t max_records,
+                              uint64_t *consumed, uint64_t *n_records, uint8_t *rest, uint64_t rest_capacity, uint64_t *rest_bytes,
+                              uint64_t *in_consumed, int64_t *bad_offset)
+{
+    bool regular = true;
+    if (bad_offset) *bad_offset = -1;
+    int rc = guarded(ctx, [&](sg::Context &c) {
+        SG_CHECK(c.up_open, "sage2gpu_load_begin must be called first");
+        SG_CHECK(state && marker && consumed && n_records && rest_bytes && in_consumed && (prefix_bytes == 0 || prefix) && (n_bytes == 0 || gz) &&
+                 (rest_capacity == 0 || rest), "null argument");
+        SG_CUDA(cudaEventSynchronize(c.up_event));
+        *consumed = *n_records = *rest_bytes = *in_consumed = 0;
+        cudaStream_t st = c.stream;
+        sg::ArenaScope arena_scope(c.arena, st);
+        sg::DevBuf<uint8_t> d_text;
+        sage2gpu_gzip_state next = *state;              // *state changes only when the piece is appended
+        try {
+            const sg::GzipPiece g = sg::stage_inflate_gzip_piece(c, gz, n_bytes, is_final != 0, text_bound, &next, prefix, prefix_bytes, d_text);
+            const sg::u64 text_bytes = prefix_bytes + g.text_bytes;
+            sg::u64 used = 0, nrec = 0;
+            regular = sg::stage_parse_device_text(c, d_text.p, text_bytes, next.done != 0, *marker, max_records, used, nrec);
+            if (!regular) return;
+            *consumed = used; *n_records = nrec;
+            *rest_bytes = text_bytes - used;
+            *in_consumed = g.in_consumed;
+            const sg::u64 back = std::min<sg::u64>(*rest_bytes, rest_capacity);
+            if (back) {
+                SG_CUDA(cudaMemcpyAsync(rest, d_text.p + used, back, cudaMemcpyDeviceToHost, st));
+                SG_CUDA(cudaStreamSynchronize(st));
+            }
+            *state = next;
+        } catch (const sg::GzipError &e) {
+            if (bad_offset) *bad_offset = (int64_t)e.offset;
+            throw;
+        }
+    });
+    if (rc == 0 && !regular) { ctx->c.last_error = "text is not in the regular 4-line FASTQ / 2-line FASTA layout"; return SAGE2GPU_ERR_FORMAT; }
+    return rc;
+}
+
+int sage2gpu_inflate_gzip(sage2gpu_ctx *ctx, const uint8_t *gz, uint64_t n_bytes, uint8_t *text, uint64_t text_capacity, uint64_t *text_bytes,
+                          int64_t *bad_offset, float *kernel_ms, uint64_t *ranges, uint64_t *confirmed, uint64_t *rejected)
+{
+    if (bad_offset) *bad_offset = -1;
+    return guarded(ctx, [&](sg::Context &c) {
+        SG_CHECK(text_bytes && (n_bytes == 0 || gz) && (text_capacity == 0 || text), "null argument");
+        // pieces of at most 512 MiB of text; the compressed bytes of a piece follow the ratio seen so far
+        const sg::u64 bound = (sg::u64)512 << 20;
+        sage2gpu_gzip_state *s = (sage2gpu_gzip_state *)calloc(1, sizeof(sage2gpu_gzip_state));
+        SG_CHECK(s, "out of host memory");
+        std::unique_ptr<sage2gpu_gzip_state, void (*)(void *)> hold(s, free);
+        sg::u64 out = 0, nr = 0, conf = 0, rej = 0, feed = (sg::u64)64 << 20;
+        float ms = 0;
+        *text_bytes = 0;
+        try {
+            while (!s->done) {
+                const sg::u64 left = n_bytes - s->offset, take = std::min(left, feed);
+                sg::ArenaScope arena_scope(c.arena, c.stream);
+                sg::DevBuf<uint8_t> d_text;
+                const sg::GzipPiece g = sg::stage_inflate_gzip_piece(c, gz + s->offset, take, take == left, bound, s, nullptr, 0, d_text);
+                ms += g.kernel_ms; nr += g.ranges; conf += g.confirmed; rej += g.rejected;
+                if (out + g.text_bytes > text_capacity) throw std::runtime_error("the text buffer is smaller than the text");
+                if (g.text_bytes) SG_CUDA(cudaMemcpyAsync(text + out, d_text.p, g.text_bytes, cudaMemcpyDeviceToHost, c.stream));
+                SG_CUDA(cudaStreamSynchronize(c.stream));
+                out += g.text_bytes;
+                *text_bytes = out;
+                if (g.in_consumed == 0) { SG_CHECK(take < left, "gzip piece without progress"); feed *= 2; }
+                else feed = std::max<sg::u64>((sg::u64)1 << 20, (sg::u64)((double)bound * g.in_consumed / std::max<sg::u64>(g.text_bytes, 1)));
+            }
+        } catch (const sg::GzipError &e) {
+            if (bad_offset) *bad_offset = (int64_t)e.offset;
+            throw;
+        }
+        if (kernel_ms) *kernel_ms = ms;
+        if (ranges) *ranges = nr;
+        if (confirmed) *confirmed = conf;
+        if (rejected) *rejected = rej;
+    });
 }
 
 int sage2gpu_load_count(sage2gpu_ctx *ctx, uint64_t *n_reads)

@@ -159,7 +159,7 @@ struct BgzfMember {
     u32 crc, out_bytes; // CRC32 and ISIZE of the trailer
 };
 enum BgzfCode : u32 { BGZF_HEADER = 1, BGZF_BSIZE, BGZF_ISIZE_LIMIT, BGZF_BLOCK_TYPE, BGZF_STORED_LEN, BGZF_BAD_CODE_LENGTHS, BGZF_BAD_CODE,
-                      BGZF_DISTANCE, BGZF_OUTPUT_OVERFLOW, BGZF_TRUNCATED, BGZF_TRAILING, BGZF_ISIZE, BGZF_CRC };
+                      BGZF_DISTANCE, BGZF_OUTPUT_OVERFLOW, BGZF_TRUNCATED, BGZF_TRAILING, BGZF_ISIZE, BGZF_CRC, GZIP_HEADER, GZIP_HEADER_CRC };
 const char *bgzf_error_text(u32 code);
 
 // A BGZF member that fails a check: its index in the batch, its byte offset there and the rule (BgzfCode)
@@ -169,6 +169,24 @@ struct BgzfError : public std::runtime_error {
     BgzfError(u64 m, u64 off, u32 c)
         : std::runtime_error("BGZF member " + std::to_string(m) + " (byte " + std::to_string(off) + " of the compressed data): " + bgzf_error_text(c)),
           member(m), offset(off), code(c) {}
+};
+
+// gunzip.cu: gzip data that fails a check: the compressed byte offset (in the file) of the member or the block and the rule
+struct GzipError : public std::runtime_error {
+    u64 offset;
+    u32 code;
+    GzipError(u64 off, u32 c)
+        : std::runtime_error("gzip data at compressed offset " + std::to_string(off) + ": " + bgzf_error_text(c)), offset(off), code(c) {}
+};
+
+// One piece of a single-member (or concatenated) gzip stream inflated on the device (gunzip.cu), continuing from `state`
+// (sage2gpu_gzip_state of include/sage2gpu.h, passed as void to keep the ABI header out of the stages).
+struct GzipPiece {
+    u64 text_bytes = 0;     // text inflated (after the prefix)
+    u64 in_consumed = 0;    // compressed bytes the state moved past
+    u64 ranges = 0, rejected = 0;   // ranges decoded (all passes); block-start candidates passed over as false
+    u64 confirmed = 0;              // ranges of the confirmed chain whose text the piece kept
+    float kernel_ms = 0;
 };
 
 // stages (each throws sg::CudaError)
@@ -188,6 +206,11 @@ void bgzf_scan_members(const uint8_t *buf, u64 n, u64 out_base, std::vector<Bgzf
 // the members inflated from d_in into d_out on the device, CRC32 and ISIZE checked; returns the kernel's milliseconds, throws
 // BgzfError naming the first bad member
 float stage_inflate_members(Context &c, const uint8_t *d_in, const BgzfMember *h_members, u64 n_members, uint8_t *d_out);
+// gunzip.cu: the compressed bytes in[0, n) (from the state's boundary on; `final`: they reach the end of the file) inflated into
+// d_text = prefix[0, prefix_bytes) + at most max(text_bound, one range) bytes of text + 1 spare byte, the state moved to the
+// new boundary; throws GzipError
+GzipPiece stage_inflate_gzip_piece(Context &c, const uint8_t *in, u64 n, bool final, u64 text_bound, void *state, const uint8_t *prefix,
+                                   u64 prefix_bytes, DevBuf<uint8_t> &d_text);
 void stage_remove_uploaded(Context &c, u64 first, u64 count);
 // parse.cu: a saved .reads file (ReadLoader::loadReadsFromFile, readLoader.cpp:289).  Header: the declared number of reads and the
 // byte offset of the body.  Slice: the lines whose first byte lies in [begin, end) of the body, parsed and checked on the device into

@@ -15,9 +15,9 @@
 // mailboxes (low-memory mode); SAGE2GPU_TABLE_LAYOUT=replicated|sharded forces the choice, the log states it.
 //
 // Input: plain FASTA / FASTQ text goes to the GPU in pieces and its records are split there.  BGZF files (htslib's bgzip: gzip
-// members with a BC field) are inflated on the GPU as well, piece by piece of whole members; other gzip files are inflated by
-// host zlib.  A BGZF member that fails a check (CRC32, ISIZE, DEFLATE rules) stops the program with a FORMAT error naming its
-// compressed offset.
+// members with a BC field) are inflated on the GPU as well, piece by piece of whole members, and so are ordinary gzip files
+// (gzip / pigz output), piece by piece of DEFLATE blocks found on the device.  Compressed data that fails a check (CRC32,
+// ISIZE, header or DEFLATE rules, truncation) stops the program with a FORMAT error naming its compressed offset.
 //
 // Restarts: -m 2 and -m 3 load <outputDir><inputPrefix>.reads (ReadLoader::loadReadsFromFile, readLoader.cpp:289) -- parsed
 // and checked on the device, spread over the contexts with --devices -- and do not open the -f / -l inputs in steps 1-3 (the
@@ -273,6 +273,7 @@ public:
         }
     }
     bool active() const { return !ctx_.empty(); }
+    size_t contexts() const { return ctx_.size(); }
     // the context the next piece goes to
     int next() const { return next_; }
     sage2gpu_ctx *ctx(int r) const { return ctx_[r]; }
@@ -292,6 +293,18 @@ public:
         const int r = next_;
         const int rc = sage2gpu_load_append_bgzf(ctx_[r], prefix, np, bgzf, n, final ? 1 : 0, marker, max_records, &consumed, &nrec, rest,
                                                  rest_cap, &rest_bytes, &bad_member);
+        touch(r);
+        if (rc == 0 && nrec) appended(r, nrec);
+        return rc;
+    }
+    // inflate + record splitting of one piece of an ordinary gzip stream on context next(); see sage2gpu_load_append_gzip
+    int appendGzip(const uint8_t *prefix, size_t np, const uint8_t *gz, size_t n, bool final, uint64_t text_bound, sage2gpu_gzip_state *state,
+                   int *marker, uint64_t max_records, uint64_t &consumed, uint64_t &nrec, uint8_t *rest, size_t rest_cap, uint64_t &rest_bytes,
+                   uint64_t &in_consumed, int64_t &bad_offset)
+    {
+        const int r = next_;
+        const int rc = sage2gpu_load_append_gzip(ctx_[r], prefix, np, gz, n, final ? 1 : 0, text_bound, state, marker, max_records, &consumed, &nrec,
+                                                 rest, rest_cap, &rest_bytes, &in_consumed, &bad_offset);
         touch(r);
         if (rc == 0 && nrec) appended(r, nrec);
         return rc;
@@ -521,33 +534,125 @@ uint64_t readBgzf(Uploader &up, int fd, const std::string &path, uint64_t max_re
     return total;
 }
 
+// Text bound of a gzip piece when one context reads the file.  A piece's parallelism is its number of DEFLATE blocks (one warp
+// each): a 32 MB piece of level-6 FASTQ holds some 180, a warp or two per SM of a B200, so one context takes 8 pieces' worth at
+// once (some 1,450 ranges, about 10 warps per SM).  Several contexts keep pieceBytes(), so that the input is spread over them.
+constexpr size_t kGzipSingleContextPieces = 8;
+
+// An ordinary gzip file (one member, or members concatenated): the compressed bytes are read with read(2) into pinned memory
+// and every piece is inflated and split on the device (sage2gpu_load_append_gzip), at most pieceBytes() of text each, or
+// kGzipSingleContextPieces times that with one context.  The
+// piece state (block boundary, the member's last 32 KiB, running CRC and length) and the text a piece leaves over stay on the
+// host and go with the next piece to whichever context takes it.  Irregular text continues on the sequential parser: zlib
+// reopens the file and skips the text the device consumed.
+uint64_t readGzip(Uploader &up, int fd, const std::string &path, uint64_t max_records, bool &used_device_parser)
+{
+    const size_t piece = pieceBytes(), rcap = 2 * piece + ((size_t)1 << 17);
+    const size_t bound = up.contexts() == 1 ? kGzipSingleContextPieces * piece : piece;
+    size_t ccap = bound / 4 + ((size_t)1 << 20);
+    uint8_t *cbuf = (uint8_t *)sage2gpu_host_alloc(ccap), *pre = (uint8_t *)sage2gpu_host_alloc(rcap), *rest = (uint8_t *)sage2gpu_host_alloc(rcap);
+    sage2gpu_gzip_state *gs = (sage2gpu_gzip_state *)calloc(1, sizeof(sage2gpu_gzip_state));
+    if (!cbuf || !pre || !rest || !gs) printError("MEM_ALLOC", "pinned gzip buffers");
+    struct Free {
+        uint8_t **a, **b, **c;
+        sage2gpu_gzip_state *s;
+        ~Free() { sage2gpu_host_free(*a); sage2gpu_host_free(*b); sage2gpu_host_free(*c); free(s); }
+    } release{ &cbuf, &pre, &rest, gs };
+    size_t have = 0, np = 0;               // compressed bytes in cbuf (from gs->offset on); host text in front of the next piece
+    size_t feed = bound / 4 + ((size_t)1 << 16);     // compressed bytes per piece, from the ratio seen so far
+    bool eof = false;
+    int marker = 0;
+    uint64_t total = 0, text_done = 0;     // records; text bytes the device consumed
+    auto fill = [&](size_t want) {
+        if (want > ccap) {
+            uint8_t *b = (uint8_t *)sage2gpu_host_alloc(want);
+            if (!b) printError("MEM_ALLOC", "pinned gzip buffers");
+            memcpy(b, cbuf, have);
+            sage2gpu_host_free(cbuf);
+            cbuf = b;
+            ccap = want;
+        }
+        while (have < want && !eof) {
+            const ssize_t n = read(fd, cbuf + have, want - have);
+            if (n < 0) { close(fd); throw std::runtime_error("cannot read " + path); }
+            if (n == 0) eof = true; else have += (size_t)n;
+        }
+    };
+    auto fallback = [&](const char *why) {
+        logStream << "\tgzip file " << path << ": " << why << " at text offset " << text_done
+                  << "; the rest of the file continues on the sequential parser (host zlib).\n";
+        if (lseek(fd, 0, SEEK_SET) != 0) { close(fd); throw std::runtime_error("cannot read " + path); }
+        gzFile gz = gzdopen(fd, "r");
+        if (!gz) { close(fd); throw std::runtime_error("cannot read " + path); }
+        gzbuffer(gz, 1 << 20);
+        if (gzseek(gz, (z_off_t)(text_done + np), SEEK_SET) < 0) { gzclose(gz); throw std::runtime_error("cannot read " + path); }
+        sg_host::FastAQStream in(gz, pre, np);          // takes the handle
+        const uint64_t got = parseSequential(up, in, max_records - total);
+        up.sync();
+        return total + got;
+    };
+    up.sync();
+    for (;;) {
+        fill(feed);
+        const size_t take = std::min(have, feed);
+        const bool final = eof && take == have;
+        uint64_t consumed = 0, nrec = 0, nrest = 0, nin = 0;
+        int64_t bad = -1;
+        const int r = up.next();
+        const int rc = up.appendGzip(pre, np, cbuf, take, final, bound, gs, &marker, max_records - total, consumed, nrec, rest, rcap, nrest, nin, bad);
+        if (rc == SAGE2GPU_ERR_FORMAT && bad >= 0) {
+            const std::string e = sage2gpu_last_error(up.ctx(r));
+            const size_t colon = e.find(": ");
+            printError("FORMAT", path + ": gzip data at compressed offset " + std::to_string(bad) + ": " +
+                                     (colon == std::string::npos ? e : e.substr(colon + 2)));
+        }
+        if (rc == SAGE2GPU_ERR_FORMAT) return fallback("text not in the regular 4-line FASTQ / 2-line FASTA layout");
+        if (rc != 0) up.fail(r);
+        used_device_parser = true;
+        total += nrec;
+        text_done += consumed;
+        if (total >= max_records) break;
+        if (nrest > rcap) {                // only the start of the unfinished record came back: zlib takes it from its start
+            np = 0;
+            return fallback("a record longer than a piece");
+        }
+        const uint64_t text = consumed + nrest - np;    // inflated by this piece
+        std::swap(pre, rest);
+        np = (size_t)nrest;
+        memmove(cbuf, cbuf + nin, have - nin);
+        have -= (size_t)nin;
+        if (gs->done) break;
+        if (nin == 0) feed *= 2;           // no complete block in the piece
+        else feed = std::max<size_t>((size_t)1 << 16, (size_t)((double)bound * nin / std::max<uint64_t>(text, 1)) + ((size_t)1 << 14));
+        if (consumed == 0 && np > piece) return fallback("a record longer than a piece");
+    }
+    up.sync();
+    close(fd);
+    return total;
+}
+
 // One file: raw text goes to the device in 32 MB pieces and the records are split there
 // (sage2gpu_load_append_text); text that is not in the regular layout is parsed sequentially from that point on.
-// BGZF files are inflated on the device too (readBgzf).
-uint64_t readFile(Uploader &up, const std::string &path, uint64_t max_records, bool &used_device_parser, bool &inflated_on_device)
+// BGZF and other gzip files are inflated on the device too (readBgzf, readGzip); `inflated` names which.
+uint64_t readFile(Uploader &up, const std::string &path, uint64_t max_records, bool &used_device_parser, std::string &inflated)
 {
-    used_device_parser = inflated_on_device = false;
+    used_device_parser = false;
+    inflated.clear();
     if (!up.active()) {                    // --parse-only
         sg_host::FastAQStream in(path);
         return parseSequential(up, in, max_records);
     }
-    // plain files are read with read(2) straight into the pinned buffer; gzip goes through zlib
     const int fd = open(path.c_str(), O_RDONLY);
     if (fd < 0) throw std::runtime_error("cannot open " + path);
     unsigned char magic[1024] = { 0 };
     const ssize_t nm = pread(fd, magic, sizeof(magic), 0);
-    const bool is_gz = nm >= 2 && magic[0] == 0x1f && magic[1] == 0x8b;
-    if (is_gz && nm > 0 && bgzfMemberBytes(magic, (size_t)nm) > 0) {
-        const uint64_t n = readBgzf(up, fd, path, max_records, used_device_parser);
-        inflated_on_device = used_device_parser;
+    if (nm >= 2 && magic[0] == 0x1f && magic[1] == 0x8b) {
+        const bool bgzf = bgzfMemberBytes(magic, (size_t)nm) > 0;
+        const uint64_t n = bgzf ? readBgzf(up, fd, path, max_records, used_device_parser) : readGzip(up, fd, path, max_records, used_device_parser);
+        if (used_device_parser) inflated = bgzf ? "BGZF" : "gzip";
         return n;
     }
-    gzFile gz = nullptr;
-    if (is_gz) {
-        gz = gzdopen(fd, "r");
-        if (!gz) { close(fd); throw std::runtime_error("cannot open " + path); }
-        gzbuffer(gz, 1 << 20);
-    }
+    // plain text is read with read(2) straight into the pinned buffer
     size_t cap = 0, have = 0;
     uint8_t *buf = up.text(cap);
     int marker = 0;                        // the file's record layout ('@' / '>'), found in its first piece; the same for every context
@@ -556,7 +661,7 @@ uint64_t readFile(Uploader &up, const std::string &path, uint64_t max_records, b
     up.sync();                             // the records of this file form segments of their own
     for (;;) {
         while (have < cap && !eof) {
-            const long n = is_gz ? (long)gzread(gz, buf + have, (unsigned)(cap - have)) : (long)read(fd, buf + have, cap - have);
+            const long n = (long)read(fd, buf + have, cap - have);
             if (n <= 0) eof = true; else have += (size_t)n;
         }
         if (have == 0) break;
@@ -564,7 +669,7 @@ uint64_t readFile(Uploader &up, const std::string &path, uint64_t max_records, b
         const int r = up.next();
         const int rc = up.appendText(buf, have, eof, &marker, max_records - total, consumed, nrec);
         if (rc == SAGE2GPU_ERR_FORMAT || (rc == 0 && consumed == 0 && !eof)) {
-            if (!gz) gz = gzdopen(fd, "r");                   // transparent mode, continues at the descriptor's offset
+            gzFile gz = gzdopen(fd, "r");                     // transparent mode, continues at the descriptor's offset
             if (!gz) { close(fd); throw std::runtime_error("cannot read " + path); }
             sg_host::FastAQStream in(gz, buf, have);          // takes the handle; continues behind what the device consumed
             total += parseSequential(up, in, max_records - total);
@@ -578,7 +683,7 @@ uint64_t readFile(Uploader &up, const std::string &path, uint64_t max_records, b
         if (have) memmove(buf, buf + consumed, have);
         if (total >= max_records || (eof && have == 0)) break;
     }
-    if (gz) gzclose(gz); else close(fd);
+    close(fd);
     return total;
 }
 
@@ -589,7 +694,8 @@ uint64_t readDataset(Uploader &up, const std::string &f1, const std::string &f2)
     logStream.flush();
     uint64_t n = 0;
     try {
-        bool dev1 = false, dev2 = false, inf1 = false, inf2 = false;
+        bool dev1 = false, dev2 = false;
+        std::string inf1, inf2;
         if (f2.empty()) {
             n = readFile(up, f1, UINT64_MAX, dev1, inf1);
             up.takeSegments();
@@ -615,7 +721,9 @@ uint64_t readDataset(Uploader &up, const std::string &f1, const std::string &f2)
             n = keep1 + n2;
         }
         logStream << "\tRecords split on the device: " << ((dev1 || dev2) ? "yes" : "no (sequential parser)")
-                  << ((inf1 || inf2) ? "; BGZF text inflated on the device" : "") << "\n";
+                  << (inf1.empty() && inf2.empty() ? "" : "; " + (inf1.empty() ? inf2 : inf2.empty() || inf2 == inf1 ? inf1 : inf1 + " and " + inf2) +
+                                                             " text inflated on the device")
+                  << "\n";
     } catch (const std::runtime_error &e) {
         printError("OPEN_FILE", e.what());
     }
