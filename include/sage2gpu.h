@@ -426,6 +426,22 @@ int sage2gpu_get_edges_packed(sage2gpu_ctx *ctx, uint64_t *out, uint64_t capacit
  * byte for byte, so that `SAGE2 -m 4 -i <prefix>` continues from them. */
 int sage2gpu_write_reads(sage2gpu_ctx *ctx, const char *path);
 int sage2gpu_write_graph3(sage2gpu_ctx *ctx, const char *path);
+/* No reference counterpart: the same reads and edges as one GFA 1.0 file, formatted on the device (for Bandage, gfatools,
+ * vg and other readers of the standard format).  Exactly these bytes, with U = unique reads and ids 1..U as in .reads:
+ *   H<TAB>VN:Z:1.0<LF>
+ *   S<TAB><id><TAB><F><TAB>LN:i:<len><TAB>RC:i:<freq><LF>    one per read in id order; F = the stored (canonical) strand, freq =
+ *                                                           the .reads FREQ (after a restart: the count wrapped modulo 65,536)
+ *   L<TAB><a><TAB><oa><TAB><b><TAB><ob><TAB><n>M<LF>        one per undirected edge, in .graph3 order: the record (a, b, type,
+ *                                                           delta) with a < b (its twin gets no line); n = len(b) - delta
+ * with the orientations of the edge type:
+ *   type 3  fwd b prefix on fwd a suffix   + +
+ *   type 2  rc b prefix on fwd a suffix    + -
+ *   type 0  fwd b suffix on fwd a prefix   - -
+ *   type 1  rc b suffix on fwd a prefix    - +
+ * so that the last n bases of a in orientation oa equal the first n bases of b in orientation ob.  Two reads may share two
+ * L lines of different types.  SAGE2GPU_ERR_STATE (with a message) before the overlap graph is built, or when the context no
+ * longer holds the reads' records, lengths and frequencies; SAGE2GPU_ERR_IO when the file cannot be written. */
+int sage2gpu_write_gfa(sage2gpu_ctx *ctx, const char *path);
 
 #ifdef __cplusplus
 }

@@ -30,6 +30,7 @@ class Sage2GpuError(RuntimeError):
 
 ERR_FORMAT = 5
 ERR_STATE = 3
+ERR_IO = 4
 
 
 class GzipState(C.Structure):
@@ -77,7 +78,7 @@ EXPORTS = ["sage2gpu_create", "sage2gpu_destroy", "sage2gpu_last_error", "sage2g
            "sage2gpu_phase_a_import", "sage2gpu_load_max_length", "sage2gpu_load_finish_slice", "sage2gpu_table_bytes",
            "sage2gpu_load_saved_reads", "sage2gpu_saved_reads_info", "sage2gpu_saved_reads_slice", "sage2gpu_saved_reads_pack",
            "sage2gpu_saved_reads_finish", "sage2gpu_table_view", "sage2gpu_load_append_bgzf", "sage2gpu_inflate_bgzf",
-           "sage2gpu_load_append_gzip", "sage2gpu_inflate_gzip"]
+           "sage2gpu_load_append_gzip", "sage2gpu_inflate_gzip", "sage2gpu_write_gfa"]
 
 _lib = None
 
@@ -161,6 +162,7 @@ def load_library():
         lib.sage2gpu_get_edges_packed.argtypes = [vp, vp, C.c_uint64, u64p]
         lib.sage2gpu_write_reads.argtypes = [vp, C.c_char_p]
         lib.sage2gpu_write_graph3.argtypes = [vp, C.c_char_p]
+        lib.sage2gpu_write_gfa.argtypes = [vp, C.c_char_p]
         lib.sage2gpu_measure_gather.argtypes = [vp, C.c_uint64, C.c_int, C.c_uint64, C.c_int, C.POINTER(C.c_double)]
         lib.sage2gpu_load_reads_partition.argtypes = [vp, vp, vp, i64, C.c_int, C.c_int, C.c_int, C.c_int, u64p]
         lib.sage2gpu_pack_slice.argtypes = [vp, vp, vp, i64, C.c_int, C.c_int, C.c_int, u64p, u64p, u64p]
@@ -649,6 +651,11 @@ class Sage2Gpu:
 
     def write_graph3(self, path: str):
         self._check(self._lib.sage2gpu_write_graph3(self._h, path.encode()), "write_graph3")
+
+    def write_gfa(self, path: str):
+        """The reads and the overlap graph as GFA 1.0 (one S line per read, one L line per edge; include/sage2gpu.h), formatted
+        on the device.  Sage2GpuError with code ERR_STATE before build_overlap_graph, ERR_IO when the file cannot be written."""
+        self._check(self._lib.sage2gpu_write_gfa(self._h, path.encode()), "write_gfa")
 
 
 # ---- mirrors of the reference's step 1-3 classes (main.cpp:37-132) ---------------------------------

@@ -1145,4 +1145,22 @@ int sage2gpu_write_graph3(sage2gpu_ctx *ctx, const char *path)
     return rc;
 }
 
+int sage2gpu_write_gfa(sage2gpu_ctx *ctx, const char *path)
+{
+    int io = 0;
+    int rc = guarded(ctx, [&](sg::Context &c) {
+        // state errors (SAGE2GPU_ERR_STATE), checked before the file is created
+        if (!c.have_graph) throw std::runtime_error("write_gfa: no overlap graph yet (sage2gpu_build_overlap_graph or sage2gpu_finish_graph first)");
+        const bool reads_held = c.have_reads && (c.cnt.unique_reads == 0 || (c.F.p && c.len.p && c.freq.p));
+        if (!reads_held) throw std::runtime_error("write_gfa: this context no longer holds the reads (records, lengths, frequencies)");
+        FILE *f = fopen(path, "wb");
+        if (!f) { io = 1; return; }
+        bool ok = false;
+        try { ok = sg::write_gfa_text(c, f); } catch (...) { fclose(f); throw; }
+        if (fclose(f) != 0 || !ok) io = 1;
+    });
+    if (rc == 0 && io) { ctx->c.last_error = std::string("cannot write ") + path; return SAGE2GPU_ERR_IO; }
+    return rc;
+}
+
 }  // extern "C"

@@ -255,5 +255,7 @@ void stage_digest(Context &c, u64 *reads_digest, u64 *edges_digest);
 // device-side text formatters of the reference's -s files (format.cu); false = short write
 bool write_reads_text(Context &c, FILE *f);
 bool write_graph3_text(Context &c, FILE *f);
+// the reads and the edge list as GFA 1.0 (sage2gpu_write_gfa)
+bool write_gfa_text(Context &c, FILE *f);
 
 }  // namespace sg

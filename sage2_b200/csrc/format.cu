@@ -1,8 +1,9 @@
 // format.cu -- the reference's -s text files formatted on the device (SURVEY.md 8(f) N3).  Restates
 // ReadLoader::saveReadsInFile / operator<<(Read) (inputReader/readLoader.cpp:29-36,270-287) and
 // OverlapGraph::saveOverlapGraphInFile / operator<<(Edge*) (overlapGraph/overlapGraph.cpp:12-20,338-369)
-// byte for byte.  Two passes per batch: line lengths -> exclusive scan -> every line written at its offset;
-// the batch then leaves the device in one copy and the file in one fwrite.
+// byte for byte, and the same graph as GFA 1.0 (no reference counterpart; format in include/sage2gpu.h).  Two passes per
+// batch: line lengths -> exclusive scan -> every line written at its offset; the batch then leaves the device in one copy
+// and the file in one fwrite.
 #include <stdio.h>
 #include "context.h"
 
@@ -84,6 +85,69 @@ __global__ void __launch_bounds__(256) read_fmt_kernel(const u64 *__restrict__ F
     }
 }
 
+// ---- <prefix>.gfa: GFA 1.0 (include/sage2gpu.h, sage2gpu_write_gfa) --------------------------------------------
+// per unique read "S\t<id>\t<F>\tLN:i:<len>\tRC:i:<freq>\n"
+__global__ void __launch_bounds__(256) gfa_seg_len_kernel(const uint16_t *__restrict__ len, const uint16_t *__restrict__ freq, u64 r0, u64 n, u32 *__restrict__ out)
+{
+    for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x) {
+        const u32 l = len[r0 + i];
+        out[i] = (u32)dec_digits((u32)(r0 + i + 1)) + (u32)dec_digits(l) + (u32)dec_digits(freq[r0 + i]) + l + 16u;
+    }
+}
+
+// one warp per read: lanes write the characters of F coalesced, as read_fmt_kernel does
+__global__ void __launch_bounds__(256) gfa_seg_fmt_kernel(const u64 *__restrict__ F, const uint16_t *__restrict__ len, const uint16_t *__restrict__ freq,
+                                                           int SWS, u64 r0, u64 n, const u32 *__restrict__ off, char *__restrict__ out)
+{
+    const int lane = threadIdx.x & 31;
+    const u64 nwarps = (u64)gridDim.x * (blockDim.x >> 5);
+    for (u64 i = (u64)blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5); i < n; i += nwarps) {
+        const u64 r = r0 + i;
+        const u32 l = len[r], id = (u32)(r + 1);
+        char *p = out + off[i];
+        char *s = p + 2 + dec_digits(id) + 1;
+        if (lane == 0) { *p++ = 'S'; *p++ = '\t'; p = put_dec(p, id); *p++ = '\t'; }
+        const u64 *fw = F + r * SWS;
+        for (u32 t = lane; t < l; t += 32) s[t] = "ACGT"[(fw[t >> 5] >> (62 - 2 * (int)(t & 31))) & 3];
+        if (lane == 0) {
+            char *q = put_str(s + l, "\tLN:i:"); q = put_dec(q, l);
+            q = put_str(q, "\tRC:i:"); q = put_dec(q, freq[r]); *q = '\n';
+        }
+    }
+}
+
+// per undirected edge "L\t<a>\t<oa>\t<b>\t<ob>\t<n>M\n", n = len(b) - delta.  Orientations from the edge type (SURVEY 8 A8):
+// 3 = fwd b prefix on fwd a suffix (+ +), 2 = rc b prefix on fwd a suffix (+ -), 0 = fwd b suffix on fwd a prefix (- -),
+// 1 = rc b suffix on fwd a prefix (- +): a is reversed when b extends it to the left, b when its strand differs from a's.
+__device__ __forceinline__ void gfa_link_fields(const u64 *edges, const uint16_t *len, u64 e, u32 &a, u32 &b, u32 &t, u32 &ov)
+{
+    u32 d, dt;
+    edge_fields(edges, len, e, a, b, t, d, dt);
+    ov = (u32)len[b - 1] - d;
+}
+
+__global__ void __launch_bounds__(256) gfa_link_len_kernel(const u64 *__restrict__ edges, const uint16_t *__restrict__ len, u64 e0, u64 n, u32 *__restrict__ out)
+{
+    for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x) {
+        u32 a, b, t, ov;
+        gfa_link_fields(edges, len, e0 + i, a, b, t, ov);
+        out[i] = (u32)(dec_digits(a) + dec_digits(b) + dec_digits(ov)) + 10u;
+    }
+}
+
+__global__ void __launch_bounds__(256) gfa_link_fmt_kernel(const u64 *__restrict__ edges, const uint16_t *__restrict__ len, u64 e0, u64 n,
+                                                            const u32 *__restrict__ off, char *__restrict__ out)
+{
+    for (u64 i = (u64)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (u64)gridDim.x * blockDim.x) {
+        u32 a, b, t, ov;
+        gfa_link_fields(edges, len, e0 + i, a, b, t, ov);
+        char *p = out + off[i];
+        *p++ = 'L'; *p++ = '\t'; p = put_dec(p, a); *p++ = '\t'; *p++ = t >= 2u ? '+' : '-'; *p++ = '\t';
+        p = put_dec(p, b); *p++ = '\t'; *p++ = (t & 1u) ? '+' : '-'; *p++ = '\t';
+        p = put_dec(p, ov); *p++ = 'M'; *p = '\n';
+    }
+}
+
 static unsigned fmt_grid(u64 n)
 {
     unsigned g = grid_for(n, 256, 2);
@@ -147,6 +211,33 @@ bool write_reads_text(Context &c, FILE *f)
             read_fmt_kernel<<<g, 256, 0, st>>>(c.F.p, c.RC.p, c.len.p, c.freq.p, SWS, r0, n, off, out);
             SG_LAUNCHED();
         });
+}
+
+bool write_gfa_text(Context &c, FILE *f)
+{
+    cudaStream_t st = c.stream;
+    if (fputs("H\tVN:Z:1.0\n", f) < 0) return false;
+    // both kinds of line in batches of <= 256 MB of text: one host buffer of that size, offsets far below 2^32
+    const u64 batch_bytes = (u64)1 << 28;
+    const u64 U = c.cnt.unique_reads, E = c.cnt.n_edges;
+    const u64 per_seg = (u64)(c.max_len > 0 ? c.max_len : 1) + 16 + 10 + 4 + 5;      // id, LN and RC values at their widest
+    const u64 per_link = 10 + 10 + 10 + 4;                                            // two ids, an overlap of <= 4 digits
+    const int SWS = c.SWS;
+    const u64 *edges = c.edges.p;
+    const uint16_t *len = c.len.p, *freq = c.freq.p;
+    return write_batches(
+               c, f, U, batch_bytes / per_seg,
+               [&](u64 r0, u64 n, u32 *out) { gfa_seg_len_kernel<<<fmt_grid(n), 256, 0, st>>>(len, freq, r0, n, out); SG_LAUNCHED(); },
+               [&](u64 r0, u64 n, const u32 *off, char *out) {
+                   unsigned g = grid_for(n, 8, 1);
+                   if (g > kSMs * 16u) g = kSMs * 16u;
+                   gfa_seg_fmt_kernel<<<g, 256, 0, st>>>(c.F.p, len, freq, SWS, r0, n, off, out);
+                   SG_LAUNCHED();
+               }) &&
+           write_batches(
+               c, f, E, batch_bytes / per_link,
+               [&](u64 e0, u64 n, u32 *out) { gfa_link_len_kernel<<<fmt_grid(n), 256, 0, st>>>(edges, len, e0, n, out); SG_LAUNCHED(); },
+               [&](u64 e0, u64 n, const u32 *off, char *out) { gfa_link_fmt_kernel<<<fmt_grid(n), 256, 0, st>>>(edges, len, e0, n, off, out); SG_LAUNCHED(); });
 }
 
 }  // namespace sg

@@ -7,7 +7,8 @@
 //
 // Flags are the reference's: -f/--fileInput, -l/--listInput, -k/--minOverlap, -o/--outputDir,
 // -p/--prefix, -i/--inputPrefix, -m/--minStep, -M/--maxStep, -s/--saveAll, -d/--debug, -h/--help.
-// Added: --device N (CUDA ordinal), --reference PATH, --devices LIST (several GPUs in ONE process: one context per listed
+// Added: --device N (CUDA ordinal), --reference PATH, --gfa (the graph of step 3 also as GFA 1.0, <prefix>.gfa, formatted on
+// the device: sage2gpu_write_gfa), --devices LIST (several GPUs in ONE process: one context per listed
 // device; the input is dealt to the contexts piece by piece as it is read and each packs its part; every stage partitioned --
 // reads organised by key range, search by id slice -- and the all-gathers between the stages done as peer copies; no NCCL,
 // no Python; same files out).  The table is replicated on every context (built by key-hash shard, all-gathered) when it fits
@@ -62,7 +63,7 @@ namespace {
 
 struct Options {
     int minStep = 1, maxStep = 7, minOverlap = 0, device = 0;
-    bool saveAll = false, debugging = false, parseOnly = false;
+    bool saveAll = false, debugging = false, parseOnly = false, gfa = false;
     std::vector<int> devices;       // --devices: one context per listed GPU, every stage partitioned, peer copies between them
     std::string fileInput, listInput, outputDir, prefixName = "untitled", inputPrefix, referenceBin;
 };
@@ -106,7 +107,9 @@ void printListOfArgs()
                  "\t-h|--help\n"
                  "ADDED:\n"
                  "\t--device <int>          CUDA device ordinal [0]\n"
-                 "\t--reference <path>      SAGE2 binary that runs steps 4-7 from the files written here\n\n";
+                 "\t--reference <path>      SAGE2 binary that runs steps 4-7 from the files written here\n"
+                 "\t--gfa                   also write the overlap graph of step 3 as GFA 1.0: <outputDir><prefix>.gfa\n"
+                 "\t                        (needs -m <= 3 and -M >= 3)\n\n";
 }
 
 // "0,1,2" or "0-3" (or a mix); a device may be listed twice (two contexts on one GPU)
@@ -133,7 +136,7 @@ void parseArgs(int argc, char **argv, Options &o)
         { "maxStep", required_argument, 0, 'M' },  { "saveAll", no_argument, 0, 's' },
         { "debug", no_argument, 0, 'd' },          { "device", required_argument, 0, 1001 },
         { "reference", required_argument, 0, 1002 }, { "parse-only", no_argument, 0, 1003 },
-        { "devices", required_argument, 0, 1004 }, { 0, 0, 0, 0 } };
+        { "devices", required_argument, 0, 1004 }, { "gfa", no_argument, 0, 1005 }, { 0, 0, 0, 0 } };
     bool fFlag = false, lFlag = false;
     int c, idx = 0;
     while ((c = getopt_long(argc, argv, "hf:l:k:o:p:i:m:M:sd", long_options, &idx)) != -1) {
@@ -158,6 +161,7 @@ void parseArgs(int argc, char **argv, Options &o)
             case 1002: o.referenceBin = optarg; break;
             case 1003: o.parseOnly = true; break;
             case 1004: o.devices = parseDevices(optarg); break;
+            case 1005: o.gfa = true; break;
             case '?': std::cout << "\n"; exit(0);
             default: std::cout << "[ERROR] Wrong command line arguments!\n\n"; exit(0);
         }
@@ -759,6 +763,14 @@ double seconds_since(const std::chrono::steady_clock::time_point &t0)
     return std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count();
 }
 
+// --gfa: <prefix>.gfa from a context that holds the reads and the complete edge list
+void saveGfa(sage2gpu_ctx *ctx, const std::string &base)
+{
+    auto t = std::chrono::steady_clock::now();
+    if (const int rc = sage2gpu_write_gfa(ctx, (base + ".gfa").c_str())) printError(rc == SAGE2GPU_ERR_IO ? "OPEN_FILE" : "CUDA", sage2gpu_last_error(ctx));
+    logStream << "Function saveGfa in " << seconds_since(t) << " sec.\n";
+}
+
 int runReference(const Options &o, int fromStep)
 {
     std::vector<std::string> a = { o.referenceBin };
@@ -1159,6 +1171,10 @@ int runOnSeveralDevices(const Options &o, const std::string &base)
         printError("OPEN_FILE", sage2gpu_last_error(m.ctx[0]));
     // the graph from the LAST context: every context must hold the complete result
     if (sage2gpu_write_graph3(m.ctx[m.G() - 1], (base + ".graph3").c_str()) != 0) printError("OPEN_FILE", sage2gpu_last_error(m.ctx[m.G() - 1]));
+    // the GFA needs the reads and the complete edge list in one context: ctx[0], which wrote .reads.  Both layouts leave them in
+    // every context -- gatherReads gives each the complete reads, finish_graph the complete edges -- and the low-memory mode of
+    // the sharded layout releases only the packed input, the unique runs before the gather, the table and the workspace
+    if (o.gfa) saveGfa(m.ctx[0], base);
     logStream.flush();
     for (sage2gpu_ctx *c : m.ctx) sage2gpu_destroy(c);
     if (o.maxStep <= 3) return 0;
@@ -1180,6 +1196,11 @@ int main(int argc, char **argv)
         printUsage();
         std::cout << "(For more information run ./sage2gpu -h)\n\n";
         exit(0);
+    }
+    if (o.gfa && (o.minStep > 3 || o.maxStep < 3)) {     // the graph of step 3 is what --gfa writes: refused before any work
+        std::cerr << "[ERROR] --gfa writes the overlap graph of step 3: it needs -m <= 3 and -M >= 3 (given -m " << o.minStep << " -M "
+                  << o.maxStep << ")\n";
+        return 1;
     }
     if (!o.outputDir.empty()) {
         const std::string cmd = "mkdir -p '" + o.outputDir + "'";
@@ -1305,6 +1326,7 @@ int main(int argc, char **argv)
         if (sage2gpu_write_graph3(ctx, (base + ".graph3").c_str()) != 0) printError("OPEN_FILE", sage2gpu_last_error(ctx));
         logStream << "Function saveOverlapGraphInFile in " << seconds_since(t) << " sec.\n";
     }
+    if (o.gfa) saveGfa(ctx, base);
     logStream.flush();
     sage2gpu_destroy(ctx);
     if (o.maxStep <= 3) return 0;
